@@ -1,6 +1,6 @@
 """bench.py -- BM25 top-10 queries/sec over a 21M-passage corpus on N B200s (BASELINE.json).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A step = one pass of the hot path over one batch: all n_queries synthetic queries scored
@@ -19,6 +19,8 @@ N>1 the NCCL all-gather of the per-shard lists and the merge.  Prints ONE JSON l
                  plus labelled variants (1 thread = what llama-index runs; threaded C restatement)
   secondary      BASELINE configs 4 and 5 on the same index (N = 1): prober-gated batch, batch x k x round sweep
   --impl reference   times only the CPU path (all host threads), never loads libprobingrag.so, same line shape
+  --dump-outputs DIR the ranked lists of the last timed step as DIR/{scores,doc_ids,query_rows}.npy (see dump_outputs):
+                     the inputs are seeded, so two builds run with the same arguments can be compared list for list
 """
 from __future__ import annotations
 
@@ -37,6 +39,8 @@ import torch
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+if __name__ == "__main__":
+    sys.dont_write_bytecode = True      # the benchmark writes nothing into the tree it runs from (it may be read-only)
 
 from probing_rag_b200 import synth  # noqa: E402
 
@@ -159,6 +163,29 @@ def digest(ids: np.ndarray, scores: np.ndarray) -> str:
     h.update(np.ascontiguousarray(ids, dtype=np.int32).tobytes())
     h.update(np.ascontiguousarray(scores, dtype=np.float32).tobytes())
     return h.hexdigest()
+
+
+DUMP_MAX_BYTES = 64_000_000
+DUMP_SEED = 2024
+
+
+def dump_outputs(out_dir: str, scores: np.ndarray, ids: np.ndarray) -> int:
+    """Write the [B, k] lists a caller of the timed path receives as out_dir/scores.npy (float32), doc_ids.npy (float64:
+    exact for every int32 id) and query_rows.npy (float64: the batch row of each dumped list).  A batch whose lists
+    would exceed DUMP_MAX_BYTES keeps a seeded sample of rows, the same rows for the same batch size.  Returns the
+    number of rows written."""
+    nq, k = scores.shape
+    row_bytes = 4 * k + 8 * k + 8
+    max_rows = (DUMP_MAX_BYTES - 3 * 4096) // row_bytes            # headroom for the three .npy headers
+    rows = np.arange(nq, dtype=np.int64)
+    if nq > max_rows:
+        rows = np.sort(np.random.default_rng(DUMP_SEED).choice(nq, size=max_rows, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "scores.npy"), np.ascontiguousarray(scores[rows], dtype=np.float32))
+    np.save(os.path.join(out_dir, "doc_ids.npy"), np.ascontiguousarray(ids[rows], dtype=np.float64))
+    np.save(os.path.join(out_dir, "query_rows.npy"), rows.astype(np.float64))
+    log(f"[bench] wrote the lists of {len(rows)} of {nq} queries (top-{k}) to {out_dir}")
+    return len(rows)
 
 
 def timed_cpu(fn, host_index, q_indptr, q_terms, k, budget_s, max_queries, n_threads, **kw):
@@ -308,7 +335,11 @@ def main():
     ap.add_argument("--list-rounds", type=int, default=4,
                     help="N > 1, p2p: launches of a call behind which the shards' running lists are all-gathered (union bound)")
     ap.add_argument("--tune", default="", help="comma list key=value for pr_bm25_tuning_t")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the ranked lists of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
 
     import torch.distributed as dist
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -335,12 +366,14 @@ def main():
         from oracle import bm25_oracle as bo
         from oracle import c_oracle as co
         per_step_budget = max(5.0, min(40.0, 120.0 / max(args.steps + args.warmup, 1)))
-        vals, n = [], 0
+        vals, n, last = [], 0, None
         for i in range(args.warmup + args.steps):
-            v, n, _ = timed_cpu(bo.retrieve_batch, host, qi, qt, k, per_step_budget, 512, cores, canonical=False)
+            v, n, last = timed_cpu(bo.retrieve_batch, host, qi, qt, k, per_step_budget, 512, cores, canonical=False)
             if i >= args.warmup:
                 vals.append(v)
         v = float(np.mean(vals))
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, *last)                 # the first n queries of the batch
         base, (s_s, s_d) = cpu_baselines(host, qi, qt, k, 20.0, cores, nq)
         base = dict(base, value=v, sample=f"{n} of {nq} queries per step (first queries of the seeded batch, whole corpus), "
                                            f"NumPy oracle port, thread pool over queries like bm25s n_threads={cores}")
@@ -458,6 +491,8 @@ def main():
         if world > 1:
             dist.destroy_process_group()
         return
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, res_s, res_d)
 
     peaks = {}
     try:

@@ -112,5 +112,6 @@ def make_bm25_golden():
 
 if __name__ == "__main__":
     torch.manual_seed(0)
+    torch.set_num_threads(8)        # test_prober_oracle.GOLDEN_THREADS: the float32 logits depend on the thread count
     make_prober_golden()
     make_bm25_golden()

@@ -7,6 +7,11 @@ import torch
 
 from oracle import prober_oracle as po
 
+# The golden logits are float32 CPU matmuls whose summation order depends on the number of intra-op threads (the
+# BLAS splits the 2048-long reductions differently, ~5e-6 apart).  They were written with this many threads; with it
+# the oracle reproduces them bit for bit whatever the host's core count.
+GOLDEN_THREADS = 8
+
 
 def load_probers():
     probers = []
@@ -23,7 +28,12 @@ def test_oracle_matches_reference_golden(golden_dir):
     assert hashlib.sha256(x.numpy().tobytes()).hexdigest() == str(g["x_digest"])
     for layer, dig in zip(po.PROBE_LAYERS, g["state_digests"]):
         assert po.state_digest(po.make_prober_state(layer)) == str(dig)
-    logits = po.prober_logits(load_probers(), x)
+    n_threads = torch.get_num_threads()
+    torch.set_num_threads(GOLDEN_THREADS)
+    try:
+        logits = po.prober_logits(load_probers(), x)
+    finally:
+        torch.set_num_threads(n_threads)
     assert np.allclose(logits.numpy(), g["logits"], rtol=1e-5, atol=1e-6)
     for j, th in enumerate(g["thetas"]):
         psum, ret = po.gate(torch.from_numpy(g["logits"]), float(th), 0)
