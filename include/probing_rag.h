@@ -245,6 +245,55 @@ int pr_pool_accumulate(float *acc_dev, int32_t n_acc_rows, int32_t n_probers, in
                        const void *act_dev, int32_t act_dtype, int32_t n_rows, int32_t n_tokens,
                        int64_t row_stride, int64_t tok_stride, const int32_t *row_map_dev, pr_stream_t stream);
 
+/* ---- dense flat L2 search ----------------------------------------------------------------
+ * Exact replacement of faiss.IndexFlatL2(d): the index built at /root/reference/make_indexer.py:446-457, loaded at
+ * exp_rag.py:243-248 and searched with k = 5 at exp_rag.py:431-438 and :496 (helpers utils.py:365-380).
+ *   rows     caller-owned f32 [n][d], d a multiple of 64 in [64, PR_FLAT_MAX_D], n <= 2^31 - 1, 16-byte aligned
+ *   result   squared L2 distances f32 [B][k], ascending, ties by row id ascending; row ids i64 [B][k];
+ *            rows short of k (k > n) are padded with (FLT_MAX, -1), the neutral entry of faiss's max-heap
+ * The distance is ||q - x||^2 evaluated in float64 in a fixed order and rounded once to f32 (DESIGN §3), so results
+ * do not depend on the launch plan.  Rows of the index are filtered with a bf16 tensor-core product and a proven
+ * lower bound of the exact distance; only rows that can enter the top-k are evaluated exactly (DESIGN §4.6). */
+#define PR_FLAT_MAX_D 1024
+typedef struct pr_flat pr_flat_t;
+
+/* Launch plan of pr_flat_search; zero fields keep the default. */
+typedef struct pr_flat_tuning {
+    int64_t first_chunk_rows; /* rows of the first filter + refine round (default 2048, rounded up to 128): every one of
+                                 them is a candidate, as no bound is known yet */
+    int32_t growth;           /* each later chunk is this many times the one before (default 4) */
+    int32_t cand_capacity;    /* candidates kept per query and chunk (default 8192); a query that finds more in a chunk
+                                 has that chunk scanned exactly instead (same result, slower) */
+} pr_flat_tuning_t;
+
+/* What the last pr_flat_search on a handle did, for benchmarks. */
+typedef struct pr_flat_stats {
+    int64_t launches;         /* kernel launches enqueued */
+    int64_t chunks;           /* filter + refine rounds */
+    int64_t candidates;       /* (query, row) pairs the filter passed, summed over queries and chunks */
+    int64_t max_candidates;   /* largest count of one query in one chunk */
+    int64_t fallback_queries; /* (query, chunk) pairs whose candidates overflowed and were scanned exactly */
+} pr_flat_stats_t;
+
+/* Handle over caller-owned rows (no copy; the rows must outlive the handle).  Reads the device's SM count; enqueues
+ * nothing. */
+int pr_flat_create(pr_flat_t **out, int device, const float *rows_dev, int64_t n, int32_t d);
+int pr_flat_destroy(pr_flat_t *index);
+/* The bf16 copy of the rows and their norms, built once into caller memory (1024-byte aligned) of
+ * pr_flat_aux_bytes() bytes; the handle keeps the pointer.  pr_flat_build_aux synchronises `stream`. */
+size_t pr_flat_aux_bytes(const pr_flat_t *index);
+int pr_flat_build_aux(pr_flat_t *index, void *aux_dev, size_t aux_bytes, pr_stream_t stream);
+int pr_flat_set_tuning(pr_flat_t *index, const pr_flat_tuning_t *tuning);
+int pr_flat_get_tuning(const pr_flat_t *index, pr_flat_tuning_t *tuning);
+/* Scratch for a batch of n_queries at depth k (1 <= k <= PR_MAX_K) under the current tuning; 0 on bad arguments. */
+size_t pr_flat_workspace_bytes(const pr_flat_t *index, int32_t n_queries, int32_t k);
+/* IndexFlatL2.search(queries, k): queries_dev f32 [n_queries][d] (16-byte aligned), workspace 1024-byte aligned. */
+int pr_flat_search(pr_flat_t *index, int32_t n_queries, const float *queries_dev, int32_t k, float *out_dist_dev,
+                   int64_t *out_ids_dev, void *workspace_dev, size_t workspace_bytes, pr_stream_t stream);
+/* Counters of the last pr_flat_search with this workspace and shape (synchronises `stream`). */
+int pr_flat_last_stats(const pr_flat_t *index, const void *workspace_dev, int32_t n_queries, int32_t k,
+                       pr_flat_stats_t *out, pr_stream_t stream);
+
 #ifdef __cplusplus
 }
 #endif

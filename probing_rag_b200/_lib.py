@@ -39,6 +39,15 @@ class ProberSet(ctypes.Structure):
                 ("w1_hi", c_vp), ("w1_lo", c_vp), ("w2_hi", c_vp), ("w2_lo", c_vp)]
 
 
+class FlatTuning(ctypes.Structure):
+    _fields_ = [("first_chunk_rows", c_i64), ("growth", c_i32), ("cand_capacity", c_i32)]
+
+
+class FlatStats(ctypes.Structure):
+    _fields_ = [("launches", c_i64), ("chunks", c_i64), ("candidates", c_i64), ("max_candidates", c_i64),
+                ("fallback_queries", c_i64)]
+
+
 # every symbol include/probing_rag.h declares: (restype, argtypes)
 SIGNATURES = {
     "pr_version": (ctypes.c_int, []),
@@ -74,6 +83,15 @@ SIGNATURES = {
                                           c_vp, c_vp]),
     "pr_prober_forward": (ctypes.c_int, [ctypes.POINTER(ProberSet), c_i32, c_vp, c_i32, ctypes.c_double, c_i32, c_vp, c_vp,
                                          c_vp, c_vp, c_vp, c_vp, c_sz, c_vp]),
+    "pr_flat_create": (ctypes.c_int, [ctypes.POINTER(c_vp), ctypes.c_int, c_vp, c_i64, c_i32]),
+    "pr_flat_destroy": (ctypes.c_int, [c_vp]),
+    "pr_flat_aux_bytes": (c_sz, [c_vp]),
+    "pr_flat_build_aux": (ctypes.c_int, [c_vp, c_vp, c_sz, c_vp]),
+    "pr_flat_set_tuning": (ctypes.c_int, [c_vp, ctypes.POINTER(FlatTuning)]),
+    "pr_flat_get_tuning": (ctypes.c_int, [c_vp, ctypes.POINTER(FlatTuning)]),
+    "pr_flat_workspace_bytes": (c_sz, [c_vp, c_i32, c_i32]),
+    "pr_flat_search": (ctypes.c_int, [c_vp, c_i32, c_vp, c_i32, c_vp, c_vp, c_vp, c_sz, c_vp]),
+    "pr_flat_last_stats": (ctypes.c_int, [c_vp, c_vp, c_i32, c_i32, ctypes.POINTER(FlatStats), c_vp]),
 }
 
 _lib = None

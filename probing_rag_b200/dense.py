@@ -1,0 +1,244 @@
+"""Exact dense retrieval: a faiss ``IndexFlatL2`` drop-in on the GPU (include/probing_rag.h, "dense flat L2 search").
+
+The reference's dense path (``exp_rag.py`` without ``--is_sparse``) builds ``faiss.IndexFlatL2(768)`` over contriever
+embeddings (/root/reference/make_indexer.py:446-457), loads it with ``faiss.read_index`` (exp_rag.py:243-248) and calls
+``index.search(q, 5)`` (exp_rag.py:431-438, 496; utils.py:365-380).  This module offers the same names:
+
+    index = dense.read_index("wiki_contriever.index")     # or IndexFlatL2(768); index.add(xb)
+    D, I = index.search(q, 5)                              # numpy in -> numpy out, like faiss
+
+``D`` holds float32 squared L2 distances, ascending, ties broken by row id; ``I`` int64 row ids; rows short of k are
+(FLT_MAX, -1).  The distances are exact (float64 evaluation in a fixed order, DESIGN §3), so they can differ from
+faiss's own fp32 BLAS results in the last bits and near-ties may rank differently.  A CUDA tensor batch returns CUDA
+tensors without a host copy.  There is no CPU path: search runs the sm_100a kernels of libprobingrag.so.
+"""
+from __future__ import annotations
+
+import ctypes
+import os
+import struct
+
+import numpy as np
+import torch
+
+from . import _lib
+
+METRIC_L2 = 1
+FOURCC_FLAT_L2 = b"IxF2"
+_HEADER = struct.Struct("<4siqqqBiQ")     # fourcc, d, ntotal, 2 dummies, is_trained, metric_type, float count
+_COPY_BYTES = 256 << 20                  # host <-> device copies of rows go in pieces of this size
+
+
+def _check_d(d) -> int:
+    if not isinstance(d, (int, np.integer)) or d < 64 or d > 1024 or d % 64:
+        raise ValueError(f"d = {d!r} unsupported: a multiple of 64 in [64, 1024]")
+    return int(d)
+
+
+class IndexFlatL2:
+    """faiss.IndexFlatL2 on one GPU: ``d``, ``ntotal``, ``is_trained``, ``metric_type``, ``add``, ``reset``,
+    ``search``.  The float32 rows live on ``device``; a bf16 copy and the row norms (half the rows' size again) are
+    built on the first search after an ``add``."""
+
+    is_trained = True
+    metric_type = METRIC_L2
+
+    def __init__(self, d: int, device="cuda"):
+        self.d = _check_d(d)
+        self.device = torch.device(device)
+        if self.device.type != "cuda":
+            raise ValueError(f"IndexFlatL2 needs a CUDA device, got {self.device}")
+        if self.device.index is None:
+            self.device = torch.device("cuda", torch.cuda.current_device())
+        self._rows = torch.empty((0, self.d), dtype=torch.float32, device=self.device)
+        self._tuning = _lib.FlatTuning()
+        self._h = None
+        self._aux = None
+        self._last = None
+
+    # ------------------------------------------------------------------ faiss interface
+    @property
+    def ntotal(self) -> int:
+        return int(self._rows.shape[0])
+
+    def add(self, x) -> None:
+        """Append float32 rows [n, d] (NumPy array or tensor)."""
+        x = self._as_rows(x, "x")
+        if self.ntotal + x.shape[0] > 2 ** 31 - 1:
+            raise ValueError("an IndexFlatL2 holds at most 2^31 - 1 rows")
+        self._set_rows(torch.cat([self._rows, x.to(self.device)]) if self.ntotal else x.to(self.device).contiguous())
+
+    def reset(self) -> None:
+        self._set_rows(torch.empty((0, self.d), dtype=torch.float32, device=self.device))
+
+    @torch.no_grad()
+    def search(self, x, k: int):
+        """(D, I) of the k nearest rows of every query row of x [B, d] float32."""
+        if isinstance(k, bool) or not isinstance(k, (int, np.integer)) or not 1 <= k <= _lib.PR_MAX_K:
+            raise ValueError(f"k must be an integer in [1, {_lib.PR_MAX_K}], got {k!r}")
+        k = int(k)
+        as_numpy = isinstance(x, np.ndarray)
+        if not as_numpy:
+            if not isinstance(x, torch.Tensor):
+                raise ValueError(f"queries must be a NumPy array or a CUDA tensor, got {type(x).__name__}")
+            if x.device != self.device:
+                raise ValueError(f"queries are on {x.device}, the index on {self.device}")
+        q = self._as_rows(x, "queries").to(self.device).contiguous()
+        B = q.shape[0]
+        D = torch.empty((B, k), dtype=torch.float32, device=self.device)
+        I = torch.empty((B, k), dtype=torch.int64, device=self.device)
+        if B:
+            L = _lib.lib()
+            h = self._handle()
+            nbytes = int(L.pr_flat_workspace_bytes(h, B, k))
+            ws = torch.empty(nbytes + 1024, dtype=torch.uint8, device=self.device)
+            ws_ptr = (ws.data_ptr() + 1023) // 1024 * 1024
+            with torch.cuda.device(self.device):
+                _lib.check(L.pr_flat_search(h, B, q.data_ptr(), k, D.data_ptr(), I.data_ptr(), ws_ptr,
+                                            nbytes, torch.cuda.current_stream(self.device).cuda_stream))
+            self._last = (ws, ws_ptr, B, k)
+        if as_numpy:
+            return D.cpu().numpy(), I.cpu().numpy()
+        return D, I
+
+    # ------------------------------------------------------------------ project extras
+    def set_tuning(self, first_chunk_rows: int = 0, growth: int = 0, cand_capacity: int = 0) -> None:
+        """Launch plan of the search (0 = default); tests force the one-chunk, many-chunk and overflow paths."""
+        self._tuning = _lib.FlatTuning(first_chunk_rows, growth, cand_capacity)
+        if self._h is not None:
+            _lib.check(_lib.lib().pr_flat_set_tuning(self._h, ctypes.byref(self._tuning)))
+
+    def get_tuning(self) -> dict:
+        t = _lib.FlatTuning()
+        _lib.check(_lib.lib().pr_flat_get_tuning(self._handle(), ctypes.byref(t)))
+        return {f: getattr(t, f) for f, _ in _lib.FlatTuning._fields_}
+
+    def last_stats(self) -> dict:
+        """Launches, chunks, candidates (sum and max per query and chunk) and overflow fallbacks of the last search
+        (synchronises the device)."""
+        if self._last is None:
+            raise ValueError("no search has run on this index")
+        _ws, ws_ptr, B, k = self._last
+        s = _lib.FlatStats()
+        with torch.cuda.device(self.device):
+            _lib.check(_lib.lib().pr_flat_last_stats(self._handle(), ws_ptr, B, k, ctypes.byref(s),
+                                                     torch.cuda.current_stream(self.device).cuda_stream))
+        return {f: getattr(s, f) for f, _ in _lib.FlatStats._fields_}
+
+    def rows(self) -> torch.Tensor:
+        """The float32 rows [ntotal, d] on the device (not a copy)."""
+        return self._rows
+
+    # ------------------------------------------------------------------ internals
+    def _as_rows(self, x, what: str) -> torch.Tensor:
+        if isinstance(x, np.ndarray):
+            if x.dtype != np.float32:
+                raise ValueError(f"{what} must be float32, got {x.dtype}")
+            x = torch.from_numpy(np.ascontiguousarray(x))
+        elif not isinstance(x, torch.Tensor):
+            raise ValueError(f"{what} must be a NumPy array or a tensor, got {type(x).__name__}")
+        elif x.dtype != torch.float32:
+            raise ValueError(f"{what} must be float32, got {x.dtype}")
+        if x.dim() != 2 or x.shape[1] != self.d:
+            raise ValueError(f"{what} must be [n, {self.d}], got {tuple(x.shape)}")
+        return x
+
+    def _set_rows(self, rows: torch.Tensor) -> None:
+        self._release()
+        self._rows = rows
+
+    def _release(self) -> None:
+        if self._h is not None:
+            _lib.lib().pr_flat_destroy(self._h)
+        self._h, self._aux, self._last = None, None, None
+
+    def _handle(self):
+        if self._h is None:
+            L = _lib.lib()
+            h = ctypes.c_void_p()
+            n = self.ntotal
+            _lib.check(L.pr_flat_create(ctypes.byref(h), self.device.index, self._rows.data_ptr() if n else None,
+                                        n, self.d))
+            try:
+                _lib.check(L.pr_flat_set_tuning(h, ctypes.byref(self._tuning)))
+                nbytes = int(L.pr_flat_aux_bytes(h))
+                aux = torch.empty(nbytes + 1024, dtype=torch.uint8, device=self.device)
+                aux_ptr = (aux.data_ptr() + 1023) // 1024 * 1024
+                with torch.cuda.device(self.device):
+                    _lib.check(L.pr_flat_build_aux(h, aux_ptr, nbytes,
+                                                   torch.cuda.current_stream(self.device).cuda_stream))
+            except Exception:
+                L.pr_flat_destroy(h)
+                raise
+            self._h, self._aux = h, aux
+        return self._h
+
+    def __del__(self):
+        try:
+            self._release()
+        except Exception:
+            pass
+
+
+# ---------------------------------------------------------------------- persistence (faiss index_write.cpp layout)
+def _read_header(path: str):
+    """(d, ntotal, payload offset) of an IndexFlatL2 file; ValueError for any other index type or metric."""
+    with open(path, "rb") as f:
+        head = f.read(_HEADER.size)
+    if len(head) < 4:
+        raise ValueError(f"{path}: not a faiss index file")
+    if head[:4] != FOURCC_FLAT_L2:
+        raise ValueError(f"{path}: index type {head[:4]!r} is not supported (only IndexFlatL2, fourcc 'IxF2')")
+    if len(head) < _HEADER.size:
+        raise ValueError(f"{path}: truncated header")
+    _, d, ntotal, _, _, _, metric, count = _HEADER.unpack(head)
+    if metric != METRIC_L2:
+        raise ValueError(f"{path}: metric_type {metric} is not supported (only METRIC_L2 = 1)")
+    if ntotal < 0 or count != ntotal * d:
+        raise ValueError(f"{path}: {count} floats stored for ntotal = {ntotal}, d = {d}")
+    if os.path.getsize(path) < _HEADER.size + 4 * count:
+        raise ValueError(f"{path}: truncated payload")
+    return d, ntotal, _HEADER.size
+
+
+def read_rows(path: str) -> np.ndarray:
+    """The rows of an IndexFlatL2 file as a read-only memory map [ntotal, d] (nothing is read yet)."""
+    d, ntotal, off = _read_header(path)
+    if ntotal == 0:
+        return np.zeros((0, d), dtype=np.float32)
+    return np.memmap(path, dtype="<f4", mode="r", offset=off, shape=(ntotal, d))
+
+
+def read_index(path: str, device="cuda") -> IndexFlatL2:
+    """faiss.read_index for IndexFlatL2 files: the payload is memory-mapped and copied to the device in pieces, so a
+    64 GB index is never held in host RAM (not even once)."""
+    rows_mm = read_rows(path)
+    index = IndexFlatL2(rows_mm.shape[1], device)
+    n, d = rows_mm.shape
+    rows = torch.empty((n, d), dtype=torch.float32, device=index.device)
+    step = max(1, _COPY_BYTES // (4 * d))
+    for a in range(0, n, step):
+        rows[a:a + step].copy_(torch.from_numpy(np.array(rows_mm[a:a + step], dtype=np.float32)))
+    index._set_rows(rows)
+    return index
+
+
+def write_rows(path: str, rows, d: int) -> None:
+    """Write float32 rows [n, d] (NumPy array, or a tensor copied to the host piece by piece) as an IndexFlatL2
+    file readable by faiss.read_index."""
+    n = int(rows.shape[0])
+    with open(path, "wb") as f:
+        f.write(_HEADER.pack(FOURCC_FLAT_L2, d, n, 1 << 20, 1 << 20, 1, METRIC_L2, n * d))
+        step = max(1, _COPY_BYTES // (4 * d))
+        for a in range(0, n, step):
+            piece = rows[a:a + step]
+            if isinstance(piece, torch.Tensor):
+                piece = piece.cpu().numpy()
+            f.write(np.ascontiguousarray(piece, dtype="<f4").tobytes())
+
+
+def write_index(index: IndexFlatL2, path: str) -> None:
+    """faiss.write_index for an IndexFlatL2."""
+    if not isinstance(index, IndexFlatL2):
+        raise ValueError(f"write_index writes IndexFlatL2 only, got {type(index).__name__}")
+    write_rows(path, index.rows(), index.d)

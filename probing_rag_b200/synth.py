@@ -159,3 +159,41 @@ def make_hidden_states(n: int, seed: int, n_probers: int = 6, d_model: int = D_M
     x = rng.standard_normal((n, n_probers, d_model), dtype=np.float32)
     s = np.exp(rng.uniform(np.log(10.0), np.log(300.0), size=(n, 1, 1))).astype(np.float32)
     return torch.from_numpy(x * s)
+
+
+# ----------------------------------------------------------------------------- dense embeddings (faiss IndexFlatL2 path)
+EMB_SEED = 2468
+EMB_BLOCK = 1 << 20
+EMB_CLUSTERS = 4096
+EMB_CENTROID_NORM = 1.5      # contriever-like: unnormalised mean-pooled embeddings of norm ~1.5
+EMB_NOISE_NORM = 0.6
+EMB_QUERY_NOISE_NORM = 0.3
+
+
+def dense_rows(n: int, d: int, device="cuda", kind: str = "clustered", seed: int = EMB_SEED) -> torch.Tensor:
+    """f32 [n, d] embeddings generated on `device` in blocks of EMB_BLOCK rows, each block from its own seeded
+    generator (the 21M x 768 corpus never exists on the host).  "clustered": one of EMB_CLUSTERS random centroids
+    plus isotropic noise; "isotropic": N(0, 1/d) per dimension, the worst case of any filter (distances concentrate)."""
+    if kind not in ("clustered", "isotropic"):
+        raise ValueError(kind)
+    out = torch.empty((n, d), dtype=torch.float32, device=device)
+    g = _block_generator(device, seed, 1 << 20)
+    cent = torch.randn((EMB_CLUSTERS, d), generator=g, device=device) * (EMB_CENTROID_NORM / d ** 0.5)
+    for blk in range((n + EMB_BLOCK - 1) // EMB_BLOCK):
+        a, b = blk * EMB_BLOCK, min(n, (blk + 1) * EMB_BLOCK)
+        g = _block_generator(device, seed, blk)
+        noise = torch.randn((b - a, d), generator=g, device=device)
+        if kind == "isotropic":
+            out[a:b] = noise * d ** -0.5
+        else:
+            c = torch.randint(0, EMB_CLUSTERS, (b - a,), generator=g, device=device)
+            out[a:b] = cent[c] + noise * (EMB_NOISE_NORM / d ** 0.5)
+    return out
+
+
+def dense_queries(rows: torch.Tensor, n_queries: int, seed: int = EMB_SEED + 1) -> torch.Tensor:
+    """f32 [n_queries, d]: perturbed copies of random rows (a question near its passage)."""
+    g = _block_generator(rows.device, seed, 0)
+    d = rows.shape[1]
+    idx = torch.randint(0, rows.shape[0], (n_queries,), generator=g, device=rows.device)
+    return rows[idx] + torch.randn((n_queries, d), generator=g, device=rows.device) * (EMB_QUERY_NOISE_NORM / d ** 0.5)
