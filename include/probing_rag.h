@@ -294,6 +294,19 @@ int pr_flat_search(pr_flat_t *index, int32_t n_queries, const float *queries_dev
 int pr_flat_last_stats(const pr_flat_t *index, const void *workspace_dev, int32_t n_queries, int32_t k,
                        pr_flat_stats_t *out, pr_stream_t stream);
 
+/* Merge n_lists ranked dense lists per query into one, in the order pr_flat_search produces (the step after the
+ * all-gather of a row-range sharded search, dense.ShardedIndexFlatL2).
+ *   dist_dev f32 [n_lists][n_queries][k], ids_dev i64 [n_lists][n_queries][k]: each list sorted as pr_flat_search
+ *   outputs it; entries with id < 0 are padding and are ignored whatever their distance.
+ *   id_base  host array of n_lists non-negative offsets added to every real id of list l (local row -> global row).
+ *   -> out_dist_dev f32 [n_queries][k], out_ids_dev i64 [n_queries][k], short rows padded (FLT_MAX, -1).
+ * Order: (uint32 bit pattern of the distance, global id) ascending. That is the key order of pr_flat_search's
+ * ranked lists, so a sharded search equals the single index bit for bit.  Enqueues one kernel on `stream` on the
+ * current device; no sync, no allocation. */
+#define PR_FLAT_MAX_LISTS 32
+int pr_flat_merge(int32_t n_queries, int32_t k, int32_t n_lists, const float *dist_dev, const int64_t *ids_dev,
+                  const int64_t *id_base, float *out_dist_dev, int64_t *out_ids_dev, pr_stream_t stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -5,7 +5,7 @@ the prober gate, exact dense (faiss IndexFlatL2) search, as hand-written sm_100a
 Python host side that mirrors the reference's retriever / prober interfaces
 (/root/reference/exp_rag.py:236-242, 381-415, 426-428; utils.py:29-57, 282-330).
 """
-from .dense import IndexFlatL2, read_index, write_index          # noqa: F401
+from .dense import IndexFlatL2, ShardedIndexFlatL2, read_index, write_index   # noqa: F401
 from .index import BM25Index, merge_topk                       # noqa: F401
 from .retriever import (BM25Retriever, Document, NodeWithScore,   # noqa: F401
                         SimpleDocumentStore, TextNode)

@@ -15,6 +15,7 @@ PR_OK, PR_EINVAL, PR_ECUDA, PR_ERANGE, PR_EWORKSPACE, PR_EUNSUPPORTED = 0, -1, -
 PR_MAX_K = 128
 PR_PROBER_MAX = 8
 PR_MAX_PEERS = 15
+PR_FLAT_MAX_LISTS = 32
 
 c_i32, c_i64, c_f32, c_vp, c_sz = ctypes.c_int32, ctypes.c_int64, ctypes.c_float, ctypes.c_void_p, ctypes.c_size_t
 
@@ -92,6 +93,7 @@ SIGNATURES = {
     "pr_flat_workspace_bytes": (c_sz, [c_vp, c_i32, c_i32]),
     "pr_flat_search": (ctypes.c_int, [c_vp, c_i32, c_vp, c_i32, c_vp, c_vp, c_vp, c_sz, c_vp]),
     "pr_flat_last_stats": (ctypes.c_int, [c_vp, c_vp, c_i32, c_i32, ctypes.POINTER(FlatStats), c_vp]),
+    "pr_flat_merge": (ctypes.c_int, [c_i32, c_i32, c_i32, c_vp, c_vp, ctypes.POINTER(c_i64), c_vp, c_vp, c_vp]),
 }
 
 _lib = None

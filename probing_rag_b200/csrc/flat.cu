@@ -19,6 +19,7 @@
 //                                    when the list overflowed), merged into the running top-k; theta[q] = its k-th
 //                                    distance, a valid upper bound of the final k-th distance
 //   output   flat_output_kernel      running lists -> (distance, id) with (FLT_MAX, -1) padding
+//   merge    flat_merge_kernel       pr_flat_merge: the lists of row-range shards -> one list in the same order
 //
 // The rows are cut into chunks of growing size; filter and refine alternate per chunk on the caller's stream, so
 // every chunk filters with the bound the earlier ones established ("bounds raised between launches", as BM25 does).
@@ -368,6 +369,80 @@ __global__ void flat_output_kernel(int64_t total, const uint64_t *__restrict__ t
     }
 }
 
+// ------------------------------------------------------------------------------------ merge of shard lists
+// One warp per query.  The query's n_lists lists are first staged in shared memory; lane l then holds the head of
+// list l (entries with id < 0 skipped) and each of the k rounds takes the warp-wide minimum of (distance bits,
+// global id, lane) and advances the winner's list.  A head past the end of its list carries hi = 2^32, above every
+// real distance's bits, so padding ranks after FLT_MAX and +inf; once the minimum is padding, so is the rest.
+struct MergeArgs {
+    int n_queries, k, n_lists, warps;
+    const float *dist;
+    const int64_t *ids;
+    float *out_dist;
+    int64_t *out_ids;
+    int64_t base[PR_FLAT_MAX_LISTS];
+};
+
+constexpr int kMergeSmemBudget = 48 * 1024;    // the default limit: 32 lists x k = 128 fit one warp
+constexpr int kMergeMaxWarps = 8;
+
+__global__ void __launch_bounds__(kMergeMaxWarps * 32) flat_merge_kernel(const MergeArgs g)
+{
+    extern __shared__ __align__(16) unsigned char merge_smem[];
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int q = blockIdx.x * g.warps + warp;
+    if (q >= g.n_queries) return;
+    const int k = g.k, L = g.n_lists;
+    int64_t *s_id = reinterpret_cast<int64_t *>(merge_smem) + (size_t)warp * L * k;
+    float *s_d = reinterpret_cast<float *>(reinterpret_cast<int64_t *>(merge_smem) + (size_t)g.warps * L * k) +
+                 (size_t)warp * L * k;
+    for (int l = 0; l < L; ++l) {
+        const size_t src = ((size_t)l * g.n_queries + q) * k;
+        for (int i = lane; i < k; i += 32) {
+            s_d[l * k + i] = __ldg(g.dist + src + i);
+            s_id[l * k + i] = __ldg(g.ids + src + i);
+        }
+    }
+    __syncwarp();
+    const bool mine = lane < L;
+    const int64_t base = mine ? g.base[lane] : 0;
+    int pos = 0;
+    if (mine)
+        while (pos < k && s_id[lane * k + pos] < 0) ++pos;
+    float *od = g.out_dist + (size_t)q * k;
+    int64_t *oi = g.out_ids + (size_t)q * k;
+    for (int r = 0; r < k; ++r) {
+        const bool live = mine && pos < k;
+        uint64_t hi = live ? (uint64_t)__float_as_uint(s_d[lane * k + pos]) : (1ull << 32);
+        int64_t gid = live ? s_id[lane * k + pos] + base : INT64_MAX;
+        int who = lane;
+#pragma unroll
+        for (int o = 16; o; o >>= 1) {
+            const uint64_t h2 = __shfl_xor_sync(PR_FULL_MASK, hi, o);
+            const int64_t g2 = __shfl_xor_sync(PR_FULL_MASK, gid, o);
+            const int w2 = __shfl_xor_sync(PR_FULL_MASK, who, o);
+            if (h2 < hi || (h2 == hi && (g2 < gid || (g2 == gid && w2 < who)))) {
+                hi = h2;
+                gid = g2;
+                who = w2;
+            }
+        }
+        if (hi >> 32) {                       // every list is exhausted: pad the rest of the row
+            for (int i = r + lane; i < k; i += 32) {
+                od[i] = FLT_MAX;
+                oi[i] = -1;
+            }
+            break;
+        }
+        if (lane == who) {
+            od[r] = __uint_as_float((uint32_t)hi);
+            oi[r] = gid;
+            ++pos;
+            while (pos < k && s_id[lane * k + pos] < 0) ++pos;
+        }
+    }
+}
+
 // ------------------------------------------------------------------------------------ host
 struct FlatLayout {
     int nq, n_qb, b_pad;
@@ -645,5 +720,45 @@ extern "C" int pr_flat_last_stats(const pr_flat_t *h, const void *workspace_dev,
     out->candidates = (int64_t)s[0];
     out->max_candidates = (int64_t)s[1];
     out->fallback_queries = (int64_t)s[2];
+    return PR_OK;
+}
+
+extern "C" int pr_flat_merge(int32_t n_queries, int32_t k, int32_t n_lists, const float *dist_dev, const int64_t *ids_dev,
+                             const int64_t *id_base, float *out_dist_dev, int64_t *out_ids_dev, pr_stream_t stream)
+{
+    if (n_queries < 0 || !id_base ||
+        (n_queries > 0 && (!dist_dev || !ids_dev || !out_dist_dev || !out_ids_dev))) {
+        pr_set_error("pr_flat_merge: bad argument (null pointer or negative batch)");
+        return PR_EINVAL;
+    }
+    if (n_lists < 1 || n_lists > PR_FLAT_MAX_LISTS) {
+        pr_set_error("pr_flat_merge: n_lists must be in [1, %d], got %d", PR_FLAT_MAX_LISTS, n_lists);
+        return PR_EINVAL;
+    }
+    if (k < 1 || k > PR_MAX_K) {
+        pr_set_error("pr_flat_merge: k must be in [1, %d], got %d", PR_MAX_K, k);
+        return PR_EINVAL;
+    }
+    MergeArgs a;
+    for (int l = 0; l < n_lists; ++l) {
+        if (id_base[l] < 0) {
+            pr_set_error("pr_flat_merge: id_base[%d] = %lld is negative", l, (long long)id_base[l]);
+            return PR_EINVAL;
+        }
+        a.base[l] = id_base[l];
+    }
+    if (n_queries == 0) return PR_OK;
+    const size_t per_warp = (size_t)n_lists * k * (sizeof(float) + sizeof(int64_t));
+    a.n_queries = n_queries;
+    a.k = k;
+    a.n_lists = n_lists;
+    a.warps = (int)std::max<size_t>(1, std::min<size_t>(kMergeMaxWarps, kMergeSmemBudget / per_warp));
+    a.dist = dist_dev;
+    a.ids = ids_dev;
+    a.out_dist = out_dist_dev;
+    a.out_ids = out_ids_dev;
+    const unsigned grid = (unsigned)((n_queries + a.warps - 1) / a.warps);
+    flat_merge_kernel<<<grid, a.warps * 32, a.warps * per_warp, (cudaStream_t)stream>>>(a);
+    PR_CUDA_CHECK(cudaGetLastError());
     return PR_OK;
 }

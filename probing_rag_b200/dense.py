@@ -7,6 +7,9 @@ embeddings (/root/reference/make_indexer.py:446-457), loads it with ``faiss.read
     index = dense.read_index("wiki_contriever.index")     # or IndexFlatL2(768); index.add(xb)
     D, I = index.search(q, 5)                              # numpy in -> numpy out, like faiss
 
+Under torchrun (one process per GPU), ``dense.read_index(path, sharded=True)`` gives each rank a contiguous row range
+of the file and returns a ``ShardedIndexFlatL2``; its ``search`` returns, on every rank, the same lists as one index.
+
 ``D`` holds float32 squared L2 distances, ascending, ties broken by row id; ``I`` int64 row ids; rows short of k are
 (FLT_MAX, -1).  The distances are exact (float64 evaluation in a fixed order, DESIGN §3), so they can differ from
 faiss's own fp32 BLAS results in the last bits and near-ties may rank differently.  A CUDA tensor batch returns CUDA
@@ -20,6 +23,7 @@ import struct
 
 import numpy as np
 import torch
+import torch.distributed as dist
 
 from . import _lib
 
@@ -33,6 +37,26 @@ def _check_d(d) -> int:
     if not isinstance(d, (int, np.integer)) or d < 64 or d > 1024 or d % 64:
         raise ValueError(f"d = {d!r} unsupported: a multiple of 64 in [64, 1024]")
     return int(d)
+
+
+def _check_k(k) -> int:
+    if isinstance(k, bool) or not isinstance(k, (int, np.integer)) or not 1 <= k <= _lib.PR_MAX_K:
+        raise ValueError(f"k must be an integer in [1, {_lib.PR_MAX_K}], got {k!r}")
+    return int(k)
+
+
+def _as_rows(x, d: int, what: str) -> torch.Tensor:
+    if isinstance(x, np.ndarray):
+        if x.dtype != np.float32:
+            raise ValueError(f"{what} must be float32, got {x.dtype}")
+        x = torch.from_numpy(np.ascontiguousarray(x))
+    elif not isinstance(x, torch.Tensor):
+        raise ValueError(f"{what} must be a NumPy array or a tensor, got {type(x).__name__}")
+    elif x.dtype != torch.float32:
+        raise ValueError(f"{what} must be float32, got {x.dtype}")
+    if x.dim() != 2 or x.shape[1] != d:
+        raise ValueError(f"{what} must be [n, {d}], got {tuple(x.shape)}")
+    return x
 
 
 class IndexFlatL2:
@@ -74,9 +98,7 @@ class IndexFlatL2:
     @torch.no_grad()
     def search(self, x, k: int):
         """(D, I) of the k nearest rows of every query row of x [B, d] float32."""
-        if isinstance(k, bool) or not isinstance(k, (int, np.integer)) or not 1 <= k <= _lib.PR_MAX_K:
-            raise ValueError(f"k must be an integer in [1, {_lib.PR_MAX_K}], got {k!r}")
-        k = int(k)
+        k = _check_k(k)
         as_numpy = isinstance(x, np.ndarray)
         if not as_numpy:
             if not isinstance(x, torch.Tensor):
@@ -131,17 +153,7 @@ class IndexFlatL2:
 
     # ------------------------------------------------------------------ internals
     def _as_rows(self, x, what: str) -> torch.Tensor:
-        if isinstance(x, np.ndarray):
-            if x.dtype != np.float32:
-                raise ValueError(f"{what} must be float32, got {x.dtype}")
-            x = torch.from_numpy(np.ascontiguousarray(x))
-        elif not isinstance(x, torch.Tensor):
-            raise ValueError(f"{what} must be a NumPy array or a tensor, got {type(x).__name__}")
-        elif x.dtype != torch.float32:
-            raise ValueError(f"{what} must be float32, got {x.dtype}")
-        if x.dim() != 2 or x.shape[1] != self.d:
-            raise ValueError(f"{what} must be [n, {self.d}], got {tuple(x.shape)}")
-        return x
+        return _as_rows(x, self.d, what)
 
     def _set_rows(self, rows: torch.Tensor) -> None:
         self._release()
@@ -180,6 +192,119 @@ class IndexFlatL2:
             pass
 
 
+# ---------------------------------------------------------------------- row-range shards over the GPUs of one box
+def merge_lists(dist_lists: torch.Tensor, id_lists: torch.Tensor, bases) -> tuple[torch.Tensor, torch.Tensor]:
+    """pr_flat_merge: ranked lists f32 / i64 [L, B, k] on one device, list l's ids offset by bases[l] -> the merged
+    (D [B, k], I [B, k]) in (distance bits, global id) order, short rows (FLT_MAX, -1)."""
+    L_, B, k = dist_lists.shape
+    if tuple(id_lists.shape) != (L_, B, k) or len(bases) != L_:
+        raise ValueError(f"lists {tuple(dist_lists.shape)} / {tuple(id_lists.shape)} with {len(bases)} bases")
+    if dist_lists.dtype != torch.float32 or id_lists.dtype != torch.int64 or not dist_lists.is_cuda \
+            or id_lists.device != dist_lists.device:
+        raise ValueError("merge_lists takes float32 distances and int64 ids on one CUDA device")
+    dev = dist_lists.device
+    D = torch.empty((B, k), dtype=torch.float32, device=dev)
+    I = torch.empty((B, k), dtype=torch.int64, device=dev)
+    if B:
+        base = (ctypes.c_int64 * L_)(*[int(b) for b in bases])
+        dl, il = dist_lists.contiguous(), id_lists.contiguous()
+        with torch.cuda.device(dev):
+            _lib.check(_lib.lib().pr_flat_merge(B, k, L_, dl.data_ptr(), il.data_ptr(), base, D.data_ptr(),
+                                                I.data_ptr(), torch.cuda.current_stream(dev).cuda_stream))
+    return D, I
+
+
+class ShardedIndexFlatL2:
+    """One rank's share of a row-range sharded IndexFlatL2: ``shard`` holds the global rows
+    [row_base, row_base + shard.ntotal).  One process per GPU (torchrun); every rank passes the same batch to
+    ``search`` and gets the same global (D, I), equal bit for bit to one IndexFlatL2 over all rows:
+
+        local search     pr_flat_search over this rank's rows                 [B, k] local ids
+        all-gather       sharding.gather_lists                               [G, B, k], rank-major
+        merge            pr_flat_merge with every rank's row_base              global ids, (distance, id) order
+
+    Each row is evaluated on exactly one rank, by the same exact distance as the single index, and the merge uses the
+    single index's key order, so ties (equal distances, even across shard boundaries) rank by global row id.
+    ``local_search(q, k) -> (D, I)`` and ``merge(D [G,B,k], I [G,B,k], bases) -> (D, I)`` can be injected (the host
+    logic is then testable on CPU with an oracle standing in); with them, ``shard`` only needs ``d`` and ``ntotal``.
+    Not supported: appending rows (``add``), writing the sharded index, one process driving several GPUs, multi-node."""
+
+    is_trained = True
+    metric_type = METRIC_L2
+
+    def __init__(self, shard, row_base: int, group=None, local_search=None, merge=None):
+        from . import sharding
+        self.shard, self.group = shard, group
+        self.d = int(shard.d)
+        self._local, self._merge = local_search, merge
+        self._gath = {}
+        self.device = getattr(shard, "device", torch.device("cpu"))
+        world = sharding._world(group)
+        if world > _lib.PR_FLAT_MAX_LISTS:
+            raise ValueError(f"at most {_lib.PR_FLAT_MAX_LISTS} ranks can share a dense index, got {world}")
+        mine = torch.tensor([int(row_base), int(shard.ntotal), self.d], dtype=torch.int64, device=self.device)
+        if world > 1:
+            every = torch.empty((world, 3), dtype=torch.int64, device=self.device)
+            dist.all_gather_into_tensor(every.view(-1), mine, group=group)
+            every = every.cpu().tolist()
+        else:
+            every = [mine.cpu().tolist()]
+        expect = 0
+        for r, (base, n, d) in enumerate(every):
+            if base != expect or n < 0:
+                raise ValueError(f"rank {r} holds rows [{base}, {base + n}), expected them to start at {expect}: "
+                                 f"the ranks' row ranges must be contiguous, in rank order, from 0 "
+                                 f"(ranges {[(b, b + m) for b, m, _ in every]})")
+            if d != self.d:
+                raise ValueError(f"rank {r} has d = {d}, this rank d = {self.d}")
+            expect += n
+        self.bases = [b for b, _, _ in every]
+        self.row_base = int(row_base)
+        self.ntotal = expect
+
+    # ------------------------------------------------------------------ faiss interface
+    def add(self, x) -> None:
+        raise ValueError("a sharded index is read-only: appending rows would break the contiguous row ranges")
+
+    def reset(self) -> None:
+        raise ValueError("a sharded index is read-only: build a new one instead of resetting it")
+
+    @torch.no_grad()
+    def search(self, x, k: int):
+        """(D, I) of the k nearest rows among ALL ranks' rows for every query of x [B, d] float32 (the same batch on
+        every rank); NumPy in -> NumPy out, a CUDA tensor in -> CUDA tensors out."""
+        from . import sharding
+        k = _check_k(k)
+        as_numpy = isinstance(x, np.ndarray)
+        q = _as_rows(x, self.d, "queries")
+        if self._local is not None:
+            Dl, Il = self._local(q, k)
+        else:
+            if not as_numpy and q.device != self.device:
+                raise ValueError(f"queries are on {q.device}, the index on {self.device}")
+            Dl, Il = self.shard.search(q.to(self.device), k)
+        B = q.shape[0]
+        if B:
+            key = (B, k)
+            gd, gi = self._gath[key] = sharding.gather_lists(Dl, Il, self.group, self._gath.get(key))
+            if len(self._gath) > 16:
+                self._gath = {key: (gd, gi)}
+            D, I = (self._merge or merge_lists)(gd, gi, self.bases)
+        else:
+            D, I = Dl, Il
+        if as_numpy:
+            return D.cpu().numpy(), I.cpu().numpy()
+        return D, I
+
+    # ------------------------------------------------------------------ project extras (this rank's shard)
+    def set_tuning(self, first_chunk_rows: int = 0, growth: int = 0, cand_capacity: int = 0) -> None:
+        self.shard.set_tuning(first_chunk_rows, growth, cand_capacity)
+
+    def last_stats(self) -> dict:
+        """Counters of this rank's local search in the last call (IndexFlatL2.last_stats)."""
+        return self.shard.last_stats()
+
+
 # ---------------------------------------------------------------------- persistence (faiss index_write.cpp layout)
 def _read_header(path: str):
     """(d, ntotal, payload offset) of an IndexFlatL2 file; ValueError for any other index type or metric."""
@@ -209,10 +334,25 @@ def read_rows(path: str) -> np.ndarray:
     return np.memmap(path, dtype="<f4", mode="r", offset=off, shape=(ntotal, d))
 
 
-def read_index(path: str, device="cuda") -> IndexFlatL2:
-    """faiss.read_index for IndexFlatL2 files: the payload is memory-mapped and copied to the device in pieces, so a
-    64 GB index is never held in host RAM (not even once)."""
+def read_shard_rows(path: str, group=None):
+    """(row_base, rows): this rank's row range sharding.shard_range(ntotal, rank, world) of an IndexFlatL2 file, as a
+    read-only memory map (nothing is read yet)."""
+    from . import sharding
     rows_mm = read_rows(path)
+    rank = dist.get_rank(group) if sharding._world(group) > 1 else 0
+    lo, hi = sharding.shard_range(rows_mm.shape[0], rank, sharding._world(group))
+    return lo, rows_mm[lo:hi]
+
+
+def read_index(path: str, device="cuda", sharded: bool = False, group=None):
+    """faiss.read_index for IndexFlatL2 files: the payload is memory-mapped and copied to the device in pieces, so a
+    64 GB index is never held in host RAM (not even once).  sharded=True (one process per GPU, torch.distributed
+    initialised, every rank of `group` calling): each rank copies only its row range (read_shard_rows) and gets a
+    ShardedIndexFlatL2 whose search covers the whole file."""
+    if sharded:
+        row_base, rows_mm = read_shard_rows(path, group)
+    else:
+        row_base, rows_mm = 0, read_rows(path)
     index = IndexFlatL2(rows_mm.shape[1], device)
     n, d = rows_mm.shape
     rows = torch.empty((n, d), dtype=torch.float32, device=index.device)
@@ -220,7 +360,7 @@ def read_index(path: str, device="cuda") -> IndexFlatL2:
     for a in range(0, n, step):
         rows[a:a + step].copy_(torch.from_numpy(np.array(rows_mm[a:a + step], dtype=np.float32)))
     index._set_rows(rows)
-    return index
+    return ShardedIndexFlatL2(index, row_base, group) if sharded else index
 
 
 def write_rows(path: str, rows, d: int) -> None:

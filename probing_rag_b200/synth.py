@@ -170,24 +170,32 @@ EMB_NOISE_NORM = 0.6
 EMB_QUERY_NOISE_NORM = 0.3
 
 
-def dense_rows(n: int, d: int, device="cuda", kind: str = "clustered", seed: int = EMB_SEED) -> torch.Tensor:
+def dense_rows(n: int, d: int, device="cuda", kind: str = "clustered", seed: int = EMB_SEED, row_lo: int = 0,
+               row_hi: int | None = None) -> torch.Tensor:
     """f32 [n, d] embeddings generated on `device` in blocks of EMB_BLOCK rows, each block from its own seeded
     generator (the 21M x 768 corpus never exists on the host).  "clustered": one of EMB_CLUSTERS random centroids
-    plus isotropic noise; "isotropic": N(0, 1/d) per dimension, the worst case of any filter (distances concentrate)."""
+    plus isotropic noise; "isotropic": N(0, 1/d) per dimension, the worst case of any filter (distances concentrate).
+    row_lo / row_hi: exactly dense_rows(n, d)[row_lo:row_hi], generating only the blocks that overlap the range
+    (whole blocks: a block's generator cannot be sought into) -- a row-range shard builds just its own rows."""
     if kind not in ("clustered", "isotropic"):
         raise ValueError(kind)
-    out = torch.empty((n, d), dtype=torch.float32, device=device)
+    row_hi = n if row_hi is None else row_hi
+    if not 0 <= row_lo <= row_hi <= n:
+        raise ValueError(f"row range [{row_lo}, {row_hi}) outside [0, {n})")
+    out = torch.empty((row_hi - row_lo, d), dtype=torch.float32, device=device)
     g = _block_generator(device, seed, 1 << 20)
     cent = torch.randn((EMB_CLUSTERS, d), generator=g, device=device) * (EMB_CENTROID_NORM / d ** 0.5)
-    for blk in range((n + EMB_BLOCK - 1) // EMB_BLOCK):
+    for blk in range(row_lo // EMB_BLOCK, (row_hi + EMB_BLOCK - 1) // EMB_BLOCK):
         a, b = blk * EMB_BLOCK, min(n, (blk + 1) * EMB_BLOCK)
         g = _block_generator(device, seed, blk)
         noise = torch.randn((b - a, d), generator=g, device=device)
         if kind == "isotropic":
-            out[a:b] = noise * d ** -0.5
+            block = noise * d ** -0.5
         else:
             c = torch.randint(0, EMB_CLUSTERS, (b - a,), generator=g, device=device)
-            out[a:b] = cent[c] + noise * (EMB_NOISE_NORM / d ** 0.5)
+            block = cent[c] + noise * (EMB_NOISE_NORM / d ** 0.5)
+        s, e = max(a, row_lo), min(b, row_hi)
+        out[s - row_lo:e - row_lo] = block[s - a:e - a]
     return out
 
 
@@ -197,3 +205,21 @@ def dense_queries(rows: torch.Tensor, n_queries: int, seed: int = EMB_SEED + 1) 
     d = rows.shape[1]
     idx = torch.randint(0, rows.shape[0], (n_queries,), generator=g, device=rows.device)
     return rows[idx] + torch.randn((n_queries, d), generator=g, device=rows.device) * (EMB_QUERY_NOISE_NORM / d ** 0.5)
+
+
+def dense_queries_of(n: int, d: int, n_queries: int, device="cuda", kind: str = "clustered", row_seed: int = EMB_SEED,
+                     seed: int = EMB_SEED + 1) -> torch.Tensor:
+    """Exactly dense_queries(dense_rows(n, d, device, kind, row_seed), n_queries, seed) without the rows: the same
+    randint and randn draws, and only the blocks that hold the sampled rows are regenerated (every rank of a sharded
+    index builds the same query batch from the shape alone)."""
+    g = _block_generator(device, seed, 0)
+    idx = torch.randint(0, n, (n_queries,), generator=g, device=device)
+    noise = torch.randn((n_queries, d), generator=g, device=device)
+    picked = torch.empty((n_queries, d), dtype=torch.float32, device=device)
+    blocks = idx // EMB_BLOCK
+    for blk in torch.unique(blocks).tolist():
+        a = blk * EMB_BLOCK
+        rows = dense_rows(n, d, device, kind, row_seed, row_lo=a, row_hi=min(n, a + EMB_BLOCK))
+        sel = torch.nonzero(blocks == blk).flatten()
+        picked[sel] = rows[idx[sel] - a]
+    return picked + noise * (EMB_QUERY_NOISE_NORM / d ** 0.5)
