@@ -194,8 +194,10 @@ int pr_topk_merge(int32_t n_queries, int32_t k, int32_t n_lists, const float *sc
 
 /* A set of n_probers ImprovedProbe MLPs, packed per prober and kept in caller-owned device memory
  * (probing_rag_b200/prober.py packs a list of state_dicts; utils.py:29-57 names in the comments).  The input LayerNorm
- * is folded around fc1 -- fc1(LN(x)) = rstd * (W' x - mean * rowsum(W')) + (W beta + b1) with W' = W diag(gamma) -- so
- * the tensor cores multiply the raw hidden states and the kernel's epilogue applies the row statistics:
+ * is folded around fc1 -- fc1(LN(x)) = rstd * (W' (x - s) - (mean - s) * rowsum(W')) + (W beta + b1) with
+ * W' = W diag(gamma) and s a per-row shift (the mean of the row's first 64 features, so that the bf16 split error does
+ * not grow with a common offset) -- so the tensor cores multiply the shifted hidden states and the kernel's epilogue
+ * applies the row statistics:
  *   w1_hi / w1_lo   fc1.weight * layer_norm_input.weight[None, :], split for bf16x3 accumulation
  *                   (hi = bf16(w), lo = bf16(w - hi), row-major [out, in] like nn.Linear.weight)
  *   w1_rowsum       its row sums
@@ -237,10 +239,14 @@ int pr_prober_forward(const pr_prober_set_t *probers, int32_t n_rows, const void
  * the prober input matrix:
  *   acc_dev float[n_acc_rows, n_probers, d_model]  +=  sum_t act[r, t, :]   into [row, slot, :]
  *   act_dev [n_rows, n_tokens, d_model] of act_dtype (0 = f32, 1 = bf16, 2 = f16), element strides
- *   row_stride / tok_stride (feature stride 1); row_map_dev int32[n_rows] maps activation row r to an
- *   accumulator row (negative = skip), NULL = identity.
- * The caller skips the prefill call of a generation (the reference drops cache[name][0]).  fp32
- * accumulation in token order.  Pointers and strides must allow 4-element vector access. */
+ *   row_stride / tok_stride (feature stride 1, tok_stride 0 allowed); row_map_dev int32[n_rows] maps
+ *   activation row r to an accumulator row, NULL = identity.  Negative entries and entries >= n_acc_rows
+ *   skip the row.  The other entries must be distinct: each row is added with a plain (non-atomic)
+ *   read-modify-write, so two rows into one accumulator row race and the result is undefined.  The
+ *   function cannot check a device array; HiddenStatePooler.add (pooling.py) checks it and raises.
+ * The caller skips the prefill call of a generation (the reference drops cache[name][0]).  Exact
+ * arithmetic: per activation row the tokens are summed in fp32 in token order starting from 0, and that
+ * sum is added to the accumulator once.  Pointers and strides must allow 4-element vector access. */
 int pr_pool_accumulate(float *acc_dev, int32_t n_acc_rows, int32_t n_probers, int32_t slot, int32_t d_model,
                        const void *act_dev, int32_t act_dtype, int32_t n_rows, int32_t n_tokens,
                        int64_t row_stride, int64_t tok_stride, const int32_t *row_map_dev, pr_stream_t stream);

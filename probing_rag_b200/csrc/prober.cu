@@ -116,11 +116,12 @@ constexpr size_t kGemmSmemBytes =
 
 // EPI 1 (fc1): the input LayerNorm is folded AROUND the GEMM and the A operand never exists in global memory.
 //     fc1(LN(x)) = rstd * (W' x - mean * rowsum(W')) + (W beta + b1),   W' = W diag(gamma)
-// so the tensor cores multiply the RAW hidden states by W' (packed once per checkpoint, prober.py) and the epilogue
+// so the tensor cores multiply the hidden states (raw but for a per-row shift) by W' (packed once per checkpoint, prober.py) and the epilogue
 // applies rstd, the mean term and the shifted bias per row.  The 8 epilogue warps -- idle while the MMAs run -- stream
 // X[128 rows, 64 features] k-block by k-block (each element of X is read from HBM exactly once, one k-block ahead of
-// the MMAs), split it into (hi, lo) bf16 straight into the stage in the 128-byte-swizzled K-major layout the tensor
-// core reads, and accumulate every row's sum and sum of squares (shifted by the row's first feature) on the way: by
+// the MMAs), subtract a per-row shift s (the mean of the row's first k-block), split x - s into (hi, lo) bf16 straight
+// into the stage in the 128-byte-swizzled K-major layout the tensor core reads, and accumulate every row's sum and sum
+// of squares of x - s on the way: by
 // the time the accumulator is complete so are mean and rstd.  This replaces a separate LayerNorm kernel that read X
 // and wrote + re-read 2 x 403 MB of split operand (0.32 of 1.05 ms at 16,384 rows) and needs no statistics pre-pass.
 // XT = dtype of X (f32 / bf16 / f16).   EPI 2 (fc2) loads A with TMA.
@@ -142,7 +143,7 @@ prober_gemm_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __grid_co
     uint64_t *acc_bar = empty_bar + kStages;                                // accumulator complete
     uint32_t *tmem_slot = reinterpret_cast<uint32_t *>(acc_bar + 1);
     float *s_red = reinterpret_cast<float *>(reinterpret_cast<unsigned char *>(full_bar) + 256);  // [4][kEpiThreads] row partials
-    float *s_mean = s_red + 4 * kEpiThreads;                                // [kBM] input LayerNorm statistics (EPI 1)
+    float *s_mean = s_red + 4 * kEpiThreads;                                // [kBM] input LayerNorm mean - s, rstd (EPI 1)
     float *s_rstd = s_mean + kBM;
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -251,9 +252,16 @@ prober_gemm_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __grid_co
                 xrow[i] = reinterpret_cast<const XT *>(g.X) + ((size_t)(live ? row0 + r : 0) * g.n_probers + p) * g.K;
                 dst[i] = (uint32_t)(r * 128 + (((c4 >> 1) ^ (r & 7)) << 4) + ((c4 & 1) << 3));
                 cur[i] = load_x4<XT>(xrow[i], c4);
-                // statistics are accumulated around the row's first feature: no E[x^2] - mean^2 cancellation for rows
-                // with a large common offset
-                shift[i] = __shfl_sync(PR_FULL_MASK, cur[i].x, lane & 16);
+                // Per-row shift s = mean of the row's first 64 features (the 16 lanes of the row hold them; the xor
+                // butterfly leaves the same value in all 16).  The tensor cores multiply the split of x - s, not of x:
+                //     W'x - mean * rowsum(W') = W'(x - s) - (mean - s) * rowsum(W')   for any s,
+                // and the bf16 split error of x - s is relative to |x - s|, about sigma, where that of x is relative
+                // to |x|: with a common offset c the error after scaling by rstd grew like |c| / sigma.  The row
+                // statistics are accumulated around the same s (no E[x^2] - mean^2 cancellation either).
+                float s4 = (cur[i].x + cur[i].y) + (cur[i].z + cur[i].w);
+#pragma unroll
+                for (int o = 8; o; o >>= 1) s4 += __shfl_xor_sync(PR_FULL_MASK, s4, o);
+                shift[i] = s4 * (1.f / kBK);
                 sum[i] = 0.f;
                 sq[i] = 0.f;
             }
@@ -273,8 +281,8 @@ prober_gemm_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __grid_co
                     __nv_bfloat16 hh[4], ll[4];
 #pragma unroll
                     for (int k = 0; k < 4; ++k) {
-                        split_bf16(x[k], hh[k], ll[k]);
                         const float d = x[k] - shift[i];
+                        split_bf16(d, hh[k], ll[k]);
                         sum[i] += d;
                         sq[i] = fmaf(d, d, sq[i]);
                     }
@@ -301,8 +309,8 @@ prober_gemm_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __grid_co
                     b += __shfl_xor_sync(PR_FULL_MASK, b, o);
                 }
                 if (c4 == 0) {
-                    const float inv_k = 1.f / (float)g.K, m = a * inv_k;
-                    s_mean[rbase + 2 * i + rsub] = shift[i] + m;
+                    const float inv_k = 1.f / (float)g.K, m = a * inv_k;   // m = mean - s
+                    s_mean[rbase + 2 * i + rsub] = m;
                     s_rstd[rbase + 2 * i + rsub] = rsqrtf(fmaxf(b * inv_k - m * m, 0.f) + kLnEps);   // biased variance
                 }
             }
@@ -325,7 +333,7 @@ prober_gemm_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __grid_co
             float csum = 0.f;
 #pragma unroll
             for (int j = 0; j < 32; ++j) {
-                // EPI 1: fc1(LN(x))_j = rstd * acc_j - (mean * rstd) * rowsum(W')_j + (W beta + b1)_j
+                // EPI 1: fc1(LN(x))_j = rstd * acc_j - ((mean - s) * rstd) * rowsum(W')_j + (W beta + b1)_j, acc = W'(x - s)
                 const float pre = EPI == 1 ? fmaf(__uint_as_float(r[j]), in_rstd, fmaf(-in_mean_rstd, s_w3[c0 + j], s_bias[c0 + j]))
                                            : __uint_as_float(r[j]) + s_bias[c0 + j];
                 const float a = silu(pre);

@@ -50,7 +50,10 @@ class HiddenStatePooler:
         return self._calls[self._slot[layer]]
 
     def add(self, layer, activations: torch.Tensor, row_map: torch.Tensor | None = None) -> None:
-        """Add sum_t activations[r, t, :] to X[row, slot(layer), :] (row = row_map[r] or r)."""
+        """Add sum_t activations[r, t, :] to X[row, slot(layer), :] (row = row_map[r] or r).  A negative row_map
+        entry skips the row; the others must be distinct and below n_rows, else ValueError (two activation rows
+        into one accumulator row would race in the kernel).  The check reads row_map on the host: a row_map on
+        the device costs a synchronisation."""
         slot = self._slot[layer]
         a = activations.detach()
         if a.dim() == 2:
@@ -65,9 +68,13 @@ class HiddenStatePooler:
             a = a.contiguous()
         rm = None
         if row_map is not None:
-            rm = row_map.to(self.device, torch.int32).contiguous()
+            rm = row_map.to("cpu", torch.int64).flatten()
             if rm.numel() != a.shape[0]:
                 raise ValueError("row_map needs one entry per activation row")
+            live = rm[rm >= 0]
+            if live.numel() and (int(live.max()) >= self.n_rows or live.unique().numel() != live.numel()):
+                raise ValueError(f"row_map: non-negative entries must be distinct and below {self.n_rows}")
+            rm = rm.to(self.device, torch.int32)
         elif a.shape[0] > self.n_rows:
             raise ValueError(f"{a.shape[0]} activation rows for {self.n_rows} accumulator rows")
         with torch.cuda.device(self.device):
