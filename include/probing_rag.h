@@ -251,7 +251,7 @@ int pr_pool_accumulate(float *acc_dev, int32_t n_acc_rows, int32_t n_probers, in
                        const void *act_dev, int32_t act_dtype, int32_t n_rows, int32_t n_tokens,
                        int64_t row_stride, int64_t tok_stride, const int32_t *row_map_dev, pr_stream_t stream);
 
-/* ---- dense flat L2 search ----------------------------------------------------------------
+/* ---- dense flat L2 and inner-product search ------------------------------------------------
  * Exact replacement of faiss.IndexFlatL2(d): the index built at /root/reference/make_indexer.py:446-457, loaded at
  * exp_rag.py:243-248 and searched with k = 5 at exp_rag.py:431-438 and :496 (helpers utils.py:365-380).
  *   rows     caller-owned f32 [n][d], d a multiple of 64 in [64, PR_FLAT_MAX_D], n <= 2^31 - 1, 16-byte aligned
@@ -262,6 +262,17 @@ int pr_pool_accumulate(float *acc_dev, int32_t n_acc_rows, int32_t n_probers, in
  * lower bound of the exact distance; only rows that can enter the top-k are evaluated exactly (DESIGN §4.6). */
 #define PR_FLAT_MAX_D 1024
 typedef struct pr_flat pr_flat_t;
+
+/* faiss's metric numbering.  PR_METRIC_INNER_PRODUCT replaces faiss.IndexFlatIP(d), the index Contriever's and DPR's
+ * own indexing code builds:
+ *   result   scores q.x f32 [B][k], descending, ties by row id ascending; NaN scores rank after -inf, among
+ *            themselves by id (and come back as the NaN with bit pattern 0xFFFFFFFF); row ids i64 [B][k]; rows short of
+ *            k are padded with (-FLT_MAX, -1), the neutral entry of faiss's min-heap.  A real row whose score is
+ *            -FLT_MAX or -inf still ranks before the padding.
+ * The score is q.x evaluated in float64 in a fixed order and rounded once to f32, never -0 (DESIGN §3); rows are
+ * filtered with the same bf16 tensor-core product and a proven upper bound of the exact score (DESIGN §4.6). */
+#define PR_METRIC_INNER_PRODUCT 0
+#define PR_METRIC_L2 1
 
 /* Launch plan of pr_flat_search; zero fields keep the default. */
 typedef struct pr_flat_tuning {
@@ -282,8 +293,10 @@ typedef struct pr_flat_stats {
 } pr_flat_stats_t;
 
 /* Handle over caller-owned rows (no copy; the rows must outlive the handle).  Reads the device's SM count; enqueues
- * nothing. */
+ * nothing.  pr_flat_create is pr_flat_create_metric(..., PR_METRIC_L2); any other metric than the two above returns
+ * PR_EUNSUPPORTED.  Every other pr_flat_* function serves the handle's metric. */
 int pr_flat_create(pr_flat_t **out, int device, const float *rows_dev, int64_t n, int32_t d);
+int pr_flat_create_metric(pr_flat_t **out, int device, const float *rows_dev, int64_t n, int32_t d, int metric);
 int pr_flat_destroy(pr_flat_t *index);
 /* The bf16 copy of the rows and their norms, built once into caller memory (1024-byte aligned) of
  * pr_flat_aux_bytes() bytes; the handle keeps the pointer.  pr_flat_build_aux synchronises `stream`. */
@@ -293,7 +306,7 @@ int pr_flat_set_tuning(pr_flat_t *index, const pr_flat_tuning_t *tuning);
 int pr_flat_get_tuning(const pr_flat_t *index, pr_flat_tuning_t *tuning);
 /* Scratch for a batch of n_queries at depth k (1 <= k <= PR_MAX_K) under the current tuning; 0 on bad arguments. */
 size_t pr_flat_workspace_bytes(const pr_flat_t *index, int32_t n_queries, int32_t k);
-/* IndexFlatL2.search(queries, k): queries_dev f32 [n_queries][d] (16-byte aligned), workspace 1024-byte aligned. */
+/* IndexFlatL2.search / IndexFlatIP.search(queries, k): queries_dev f32 [n_queries][d] (16-byte aligned), workspace 1024-byte aligned. */
 int pr_flat_search(pr_flat_t *index, int32_t n_queries, const float *queries_dev, int32_t k, float *out_dist_dev,
                    int64_t *out_ids_dev, void *workspace_dev, size_t workspace_bytes, pr_stream_t stream);
 /* Counters of the last pr_flat_search with this workspace and shape (synchronises `stream`). */
@@ -312,6 +325,13 @@ int pr_flat_last_stats(const pr_flat_t *index, const void *workspace_dev, int32_
 #define PR_FLAT_MAX_LISTS 32
 int pr_flat_merge(int32_t n_queries, int32_t k, int32_t n_lists, const float *dist_dev, const int64_t *ids_dev,
                   const int64_t *id_base, float *out_dist_dev, int64_t *out_ids_dev, pr_stream_t stream);
+/* pr_flat_merge for lists of either metric (pr_flat_merge is its PR_METRIC_L2 case).  PR_METRIC_INNER_PRODUCT: the same
+ * rules, in the inner-product order above: (key of the score, global id) ascending, where the key ascends as the score
+ * descends and puts NaN after -inf -- the key of pr_flat_search's inner-product lists; padding ranks after every real
+ * entry (-FLT_MAX, -inf and NaN included) and short rows are padded (-FLT_MAX, -1).  Another metric: PR_EUNSUPPORTED. */
+int pr_flat_merge_metric(int32_t n_queries, int32_t k, int32_t n_lists, const float *dist_dev, const int64_t *ids_dev,
+                         const int64_t *id_base, float *out_dist_dev, int64_t *out_ids_dev, pr_stream_t stream,
+                         int metric);
 
 #ifdef __cplusplus
 }

@@ -16,6 +16,7 @@ PR_MAX_K = 128
 PR_PROBER_MAX = 8
 PR_MAX_PEERS = 15
 PR_FLAT_MAX_LISTS = 32
+PR_METRIC_INNER_PRODUCT, PR_METRIC_L2 = 0, 1
 
 c_i32, c_i64, c_f32, c_vp, c_sz = ctypes.c_int32, ctypes.c_int64, ctypes.c_float, ctypes.c_void_p, ctypes.c_size_t
 
@@ -85,6 +86,7 @@ SIGNATURES = {
     "pr_prober_forward": (ctypes.c_int, [ctypes.POINTER(ProberSet), c_i32, c_vp, c_i32, ctypes.c_double, c_i32, c_vp, c_vp,
                                          c_vp, c_vp, c_vp, c_vp, c_sz, c_vp]),
     "pr_flat_create": (ctypes.c_int, [ctypes.POINTER(c_vp), ctypes.c_int, c_vp, c_i64, c_i32]),
+    "pr_flat_create_metric": (ctypes.c_int, [ctypes.POINTER(c_vp), ctypes.c_int, c_vp, c_i64, c_i32, ctypes.c_int]),
     "pr_flat_destroy": (ctypes.c_int, [c_vp]),
     "pr_flat_aux_bytes": (c_sz, [c_vp]),
     "pr_flat_build_aux": (ctypes.c_int, [c_vp, c_vp, c_sz, c_vp]),
@@ -94,6 +96,8 @@ SIGNATURES = {
     "pr_flat_search": (ctypes.c_int, [c_vp, c_i32, c_vp, c_i32, c_vp, c_vp, c_vp, c_sz, c_vp]),
     "pr_flat_last_stats": (ctypes.c_int, [c_vp, c_vp, c_i32, c_i32, ctypes.POINTER(FlatStats), c_vp]),
     "pr_flat_merge": (ctypes.c_int, [c_i32, c_i32, c_i32, c_vp, c_vp, ctypes.POINTER(c_i64), c_vp, c_vp, c_vp]),
+    "pr_flat_merge_metric": (ctypes.c_int, [c_i32, c_i32, c_i32, c_vp, c_vp, ctypes.POINTER(c_i64), c_vp, c_vp, c_vp,
+                                            ctypes.c_int]),
 }
 
 _lib = None

@@ -1,10 +1,11 @@
-// Exact flat L2 search (faiss IndexFlatL2 drop-in) on B200 tensor cores (sm_100a).
+// Exact flat L2 and inner-product search (faiss IndexFlatL2 / IndexFlatIP drop-ins) on B200 tensor cores (sm_100a).
 //
 // Replaces faiss.IndexFlatL2(768).search(q, k), the brute-force CPU scan the reference's dense path runs
 // (/root/reference/exp_rag.py:243-248, 431-438, 496; utils.py:365-380; index built at make_indexer.py:446-457).
 //
-// The result is EXACT: distances are evaluated in float64 in a fixed order (DESIGN §3) and the ranked list is the
-// canonical (distance asc, id asc) order.  The tensor cores only decide which rows need that evaluation:
+// The result is EXACT: distances (scores) are evaluated in float64 in a fixed order (DESIGN §3) and the ranked list is
+// the canonical (distance asc, id asc) order, or (score desc, id asc) for inner products.  The tensor cores only decide
+// which rows need that evaluation:
 //
 //   prep     flat_prep_kernel        bf16 copy (RNE) of every row, ||x||^2 and ||x|| in f32 (aux buffer, once per index;
 //                                    the same kernel prepares the query batch per call)
@@ -15,10 +16,14 @@
 //                                      warps 4-7 epilogue: lower bound ||q||^2 + ||x||^2 - 2 q.x - margin(q, x) of the
 //                                              exact distance; (query, row) pairs whose bound does not exceed the
 //                                              query's running bound theta[q] go to a per-query candidate list
+//            flat_ip_filter_kernel   the same GEMM; epilogue: upper bound q.x + margin(q, x) of the exact score, pairs
+//                                    whose bound is not below theta[q] are candidates
 //   refine   flat_refine_kernel      one CTA per query: exact distances of the candidates (or of the whole chunk
 //                                    when the list overflowed), merged into the running top-k; theta[q] = its k-th
 //                                    distance, a valid upper bound of the final k-th distance
-//   output   flat_output_kernel      running lists -> (distance, id) with (FLT_MAX, -1) padding
+//            flat_ip_refine_kernel   the same with exact inner products; theta[q] = the k-th score, a lower bound of
+//                                    the final k-th score
+//   output   flat_output_kernel      running lists -> (distance, id) with (FLT_MAX, -1) padding, (-FLT_MAX, -1) for IP
 //   merge    flat_merge_kernel       pr_flat_merge: the lists of row-range shards -> one list in the same order
 //
 // The rows are cut into chunks of growing size; filter and refine alternate per chunk on the caller's stream, so
@@ -40,6 +45,7 @@ struct pr_flat {
     const float *rows;
     const __nv_bfloat16 *rows_bf;   // aux: bf16 copy [n][d]
     const float *norm2, *norm;      // aux: ||x||^2, ||x|| (f32)
+    int metric;                     // PR_METRIC_L2 or PR_METRIC_INNER_PRODUCT
     pr_flat_tuning_t tun;
     int64_t last_launches, last_chunks;
 };
@@ -60,6 +66,16 @@ constexpr int32_t kDefaultGrowth = 4;
 constexpr int32_t kDefaultCapacity = 8192;
 
 inline size_t up(size_t x, size_t a) { return (x + a - 1) / a * a; }
+
+// Key of an inner-product score's bits: ascends as the score descends (+inf first, -inf last), with every NaN mapped
+// to 0xFFFFFFFF, above -inf.  ip_bits inverts it (a NaN comes back as the NaN 0xFFFFFFFF).
+__device__ __forceinline__ uint32_t ip_key(uint32_t bits)
+{
+    if ((bits & 0x7FFFFFFFu) > 0x7F800000u) return 0xFFFFFFFFu;
+    return (bits & 0x80000000u) ? bits : bits ^ 0x7FFFFFFFu;
+}
+
+__device__ __forceinline__ uint32_t ip_bits(uint32_t key) { return (key & 0x80000000u) ? key : key ^ 0x7FFFFFFFu; }
 
 __device__ __forceinline__ void tmem_ld32_nowait(uint32_t taddr, uint32_t (&r)[32])
 {
@@ -99,13 +115,14 @@ __global__ void flat_prep_kernel(const float *__restrict__ x, int64_t n, int64_t
     }
 }
 
-__global__ void flat_init_kernel(int n_queries, int k, float *__restrict__ theta, int32_t *__restrict__ count,
-                                 uint64_t *__restrict__ topk, unsigned long long *__restrict__ stats)
+__global__ void flat_init_kernel(int n_queries, int k, float theta0, float *__restrict__ theta,
+                                 int32_t *__restrict__ count, uint64_t *__restrict__ topk,
+                                 unsigned long long *__restrict__ stats)
 {
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i < (int64_t)n_queries * k) topk[i] = kEmptyKey;
     if (i < n_queries) {
-        theta[i] = INFINITY;
+        theta[i] = theta0;
         count[i] = 0;
     }
     if (i < 4) stats[i] = 0;
@@ -119,7 +136,7 @@ struct FilterArgs {
     int n_stages;
     uint32_t idesc;
     uint32_t tmem_cols;
-    float c1, c2, c3;               // margin(q, x) = c1 |q| |x| + c2 (|q|^2 + |x|^2) + c3 (1 + |q| + |x|)
+    float c1, c2, c3;               // margin(q, x) = c1 |q| |x| + c2 (|q|^2 + |x|^2) + c3 (1 + |q| + |x|) (IP: c2 = 0)
     const float *norm2, *norm;      // rows
     const float *qn2, *qn;          // queries
     const float *theta;
@@ -128,9 +145,9 @@ struct FilterArgs {
     int cap;
 };
 
-__global__ void __launch_bounds__(kFilterThreads, 1)
-flat_filter_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_constant__ CUtensorMap map_q,
-                   const FilterArgs g)
+// The GEMM and its pipeline are shared; M (PR_METRIC_*) selects only the epilogue's bound and comparison.
+template <int M>
+__device__ __forceinline__ void flat_filter(const CUtensorMap &map_x, const CUtensorMap &map_q, const FilterArgs &g)
 {
     extern __shared__ unsigned char smem_dyn[];
     unsigned char *smem = reinterpret_cast<unsigned char *>(((uintptr_t)smem_dyn + 1023) & ~(uintptr_t)1023);
@@ -213,7 +230,8 @@ flat_filter_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_const
             const int64_t row = g.row_begin + (t / g.n_qb) * kRowsPerTile + quad * 32 + lane;
             const int q0 = (int)(t % g.n_qb) * g.nq;
             const bool live = row < g.row_end;
-            const float nx2 = live ? __ldg(g.norm2 + row) : 0.f, nx = live ? __ldg(g.norm + row) : 0.f;
+            const float nx2 = (M == PR_METRIC_L2 && live) ? __ldg(g.norm2 + row) : 0.f;
+            const float nx = live ? __ldg(g.norm + row) : 0.f;
             mbar_wait(&tfull_bar[a], (it >> 1) & 1u);
             tc_fence_after();
             const uint32_t taddr = tmem_base + a * (uint32_t)g.nq + ((uint32_t)(quad * 32) << 16);
@@ -225,11 +243,18 @@ flat_filter_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_const
                 for (int j = 0; j < 32; ++j) {
                     const int q = q0 + c0 + j;
                     if (q >= g.n_queries) continue;   // (warp-uniform)
-                    const float qn2 = __ldg(g.qn2 + q), qn = __ldg(g.qn + q), th = __ldg(g.theta + q);
-                    const float s2 = qn2 + nx2;
-                    const float margin = fmaf(g.c1 * qn, nx, fmaf(g.c2, s2, g.c3 * (1.f + qn + nx)));
-                    const float bound = fmaf(-2.f, __uint_as_float(r[j]), s2) - margin;
-                    const bool take = live && !(bound > th);   // (a NaN bound is a candidate)
+                    bool take;
+                    if constexpr (M == PR_METRIC_L2) {
+                        const float qn2 = __ldg(g.qn2 + q), qn = __ldg(g.qn + q), th = __ldg(g.theta + q);
+                        const float s2 = qn2 + nx2;
+                        const float margin = fmaf(g.c1 * qn, nx, fmaf(g.c2, s2, g.c3 * (1.f + qn + nx)));
+                        const float bound = fmaf(-2.f, __uint_as_float(r[j]), s2) - margin;
+                        take = live && !(bound > th);          // (a NaN bound is a candidate)
+                    } else {
+                        const float qn = __ldg(g.qn + q), th = __ldg(g.theta + q);
+                        const float bound = __uint_as_float(r[j]) + fmaf(g.c1 * qn, nx, g.c3 * (1.f + qn + nx));
+                        take = live && !(bound < th);          // (a NaN bound is a candidate)
+                    }
                     const unsigned m = __ballot_sync(PR_FULL_MASK, take);
                     if (m) {
                         int base = 0;
@@ -254,6 +279,20 @@ flat_filter_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_const
     }
 }
 
+__global__ void __launch_bounds__(kFilterThreads, 1)
+flat_filter_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_constant__ CUtensorMap map_q,
+                   const FilterArgs g)
+{
+    flat_filter<PR_METRIC_L2>(map_x, map_q, g);
+}
+
+__global__ void __launch_bounds__(kFilterThreads, 1)
+flat_ip_filter_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_constant__ CUtensorMap map_q,
+                      const FilterArgs g)
+{
+    flat_filter<PR_METRIC_INNER_PRODUCT>(map_x, map_q, g);
+}
+
 // ------------------------------------------------------------------------------------ refine
 // The exact distance (DESIGN §3): lane l sums (q_j - x_j)^2 over j = l, l+32, ... in increasing j, every difference,
 // square and add a separately rounded f64 operation (no contraction), then an xor butterfly over the 32 lanes
@@ -268,6 +307,19 @@ __device__ __forceinline__ float exact_dist(const float *__restrict__ sq, const 
 #pragma unroll
     for (int o = 16; o; o >>= 1) s = __dadd_rn(s, __shfl_xor_sync(PR_FULL_MASK, s, o));
     return __double2float_rn(s);
+}
+
+// The exact inner product (DESIGN §3): lane l starts at +0.0 and adds q_j x_j over j = l, l+32, ... in increasing j
+// (the product of two floats is exact in f64; __dmul_rn keeps it from contracting into an FMA), then the same butterfly
+// and one rounding to f32.  A negative sum that underflows f32 would round to -0; adding +0 makes it +0, so a score is
+// never -0.
+__device__ __forceinline__ float exact_ip(const float *__restrict__ sq, const float *__restrict__ x, int d, int lane)
+{
+    double s = 0.0;
+    for (int j = lane; j < d; j += 32) s = __dadd_rn(s, __dmul_rn((double)sq[j], (double)__ldg(x + j)));
+#pragma unroll
+    for (int o = 16; o; o >>= 1) s = __dadd_rn(s, __shfl_xor_sync(PR_FULL_MASK, s, o));
+    return __fadd_rn(__double2float_rn(s), 0.f);
 }
 
 // ascending bitonic sort of keys[0, n), n a power of two, by the whole block
@@ -297,13 +349,13 @@ struct RefineArgs {
     int64_t row_begin, row_end;
     int32_t *count;
     const int32_t *cand;
-    uint64_t *topk;                 // [B][k] keys (f32 distance bits << 32 | row), ascending
+    uint64_t *topk;                 // [B][k] keys (f32 distance bits, or ip_key of the score, << 32 | row), ascending
     float *theta;
     unsigned long long *stats;      // candidates, max candidates, fallback queries
 };
 
-__global__ void __launch_bounds__(kRefineThreads)
-flat_refine_kernel(const RefineArgs g)
+template <int M>
+__device__ __forceinline__ void flat_refine(const RefineArgs &g)
 {
     __shared__ uint64_t s_keys[kRefineKeys];
     __shared__ float s_q[PR_FLAT_MAX_D];
@@ -330,8 +382,12 @@ flat_refine_kernel(const RefineArgs g)
         const int64_t end = min(n_items, base + round);
         for (int64_t i = base + warp; i < end; i += n_warps) {
             const int64_t row = overflow ? g.row_begin + i : (int64_t)g.cand[(size_t)q * g.cap + i];
-            const float dist = exact_dist(s_q, g.rows + row * g.d, g.d, lane);
-            const uint64_t key = ((uint64_t)__float_as_uint(dist) << 32) | (uint64_t)row;
+            uint32_t hi;
+            if constexpr (M == PR_METRIC_L2)
+                hi = __float_as_uint(exact_dist(s_q, g.rows + row * g.d, g.d, lane));
+            else
+                hi = ip_key(__float_as_uint(exact_ip(s_q, g.rows + row * g.d, g.d, lane)));
+            const uint64_t key = ((uint64_t)hi << 32) | (uint64_t)row;
             if (lane == 0 && key < kth) s_keys[g.k + atomicAdd(&s_new, 1)] = key;
         }
         __syncthreads();
@@ -349,33 +405,46 @@ flat_refine_kernel(const RefineArgs g)
     }
     for (int i = threadIdx.x; i < g.k; i += blockDim.x) g.topk[(size_t)q * g.k + i] = s_keys[i];
     if (threadIdx.x == 0) {
-        g.theta[q] = kth == kEmptyKey ? INFINITY : __uint_as_float((uint32_t)(kth >> 32));
+        if constexpr (M == PR_METRIC_L2)
+            g.theta[q] = kth == kEmptyKey ? INFINITY : __uint_as_float((uint32_t)(kth >> 32));
+        else
+            g.theta[q] = kth == kEmptyKey ? -INFINITY : __uint_as_float(ip_bits((uint32_t)(kth >> 32)));
         g.count[q] = 0;
     }
 }
 
+__global__ void __launch_bounds__(kRefineThreads) flat_refine_kernel(const RefineArgs g) { flat_refine<PR_METRIC_L2>(g); }
+
+__global__ void __launch_bounds__(kRefineThreads) flat_ip_refine_kernel(const RefineArgs g)
+{
+    flat_refine<PR_METRIC_INNER_PRODUCT>(g);
+}
+
 __global__ void flat_output_kernel(int64_t total, const uint64_t *__restrict__ topk, float *__restrict__ dist,
-                                   int64_t *__restrict__ ids)
+                                   int64_t *__restrict__ ids, int metric)
 {
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= total) return;
     const uint64_t key = topk[i];
+    const bool ip = metric == PR_METRIC_INNER_PRODUCT;
     if (key == kEmptyKey) {
-        dist[i] = FLT_MAX;
+        dist[i] = ip ? -FLT_MAX : FLT_MAX;
         ids[i] = -1;
     } else {
-        dist[i] = __uint_as_float((uint32_t)(key >> 32));
+        const uint32_t hi = (uint32_t)(key >> 32);
+        dist[i] = __uint_as_float(ip ? ip_bits(hi) : hi);
         ids[i] = (int64_t)(uint32_t)key;
     }
 }
 
 // ------------------------------------------------------------------------------------ merge of shard lists
 // One warp per query.  The query's n_lists lists are first staged in shared memory; lane l then holds the head of
-// list l (entries with id < 0 skipped) and each of the k rounds takes the warp-wide minimum of (distance bits,
-// global id, lane) and advances the winner's list.  A head past the end of its list carries hi = 2^32, above every
-// real distance's bits, so padding ranks after FLT_MAX and +inf; once the minimum is padding, so is the rest.
+// list l (entries with id < 0 skipped) and each of the k rounds takes the warp-wide minimum of (key, global id, lane)
+// and advances the winner's list.  The key is the refine's: the distance bits (L2) or ip_key of the score (IP).  A head
+// past the end of its list carries hi = 2^32, above every real key, so padding ranks after FLT_MAX and +inf (L2) or
+// -FLT_MAX, -inf and NaN (IP); once the minimum is padding, so is the rest.
 struct MergeArgs {
-    int n_queries, k, n_lists, warps;
+    int n_queries, k, n_lists, warps, metric;
     const float *dist;
     const int64_t *ids;
     float *out_dist;
@@ -404,6 +473,7 @@ __global__ void __launch_bounds__(kMergeMaxWarps * 32) flat_merge_kernel(const M
         }
     }
     __syncwarp();
+    const bool ip = g.metric == PR_METRIC_INNER_PRODUCT;
     const bool mine = lane < L;
     const int64_t base = mine ? g.base[lane] : 0;
     int pos = 0;
@@ -413,7 +483,8 @@ __global__ void __launch_bounds__(kMergeMaxWarps * 32) flat_merge_kernel(const M
     int64_t *oi = g.out_ids + (size_t)q * k;
     for (int r = 0; r < k; ++r) {
         const bool live = mine && pos < k;
-        uint64_t hi = live ? (uint64_t)__float_as_uint(s_d[lane * k + pos]) : (1ull << 32);
+        const uint32_t bits = live ? __float_as_uint(s_d[lane * k + pos]) : 0u;
+        uint64_t hi = live ? (uint64_t)(ip ? ip_key(bits) : bits) : (1ull << 32);
         int64_t gid = live ? s_id[lane * k + pos] + base : INT64_MAX;
         int who = lane;
 #pragma unroll
@@ -429,13 +500,13 @@ __global__ void __launch_bounds__(kMergeMaxWarps * 32) flat_merge_kernel(const M
         }
         if (hi >> 32) {                       // every list is exhausted: pad the rest of the row
             for (int i = r + lane; i < k; i += 32) {
-                od[i] = FLT_MAX;
+                od[i] = ip ? -FLT_MAX : FLT_MAX;
                 oi[i] = -1;
             }
             break;
         }
         if (lane == who) {
-            od[r] = __uint_as_float((uint32_t)hi);
+            od[r] = __uint_as_float(ip ? ip_bits((uint32_t)hi) : (uint32_t)hi);
             oi[r] = gid;
             ++pos;
             while (pos < k && s_id[lane * k + pos] < 0) ++pos;
@@ -493,25 +564,43 @@ float margin_c1(int K)
     return std::nextafter((float)c, INFINITY);
 }
 
+// The same for the inner-product bound q.x + margin (derivation: DESIGN §4.6): the bf16 rounding, 2u + u^2, and the
+// assumed fp32 accumulation, K 2^-22 (1 + u)^2, without the factor 2; (K + 5) 2^-53 for the f64 sum of the exact score
+// and 2^-22 for its f32 rounding and that of the bound's last add; 2^-10 of head room covers the f32 rounding of |q|,
+// |x| and of the margin's own evaluation.
+float margin_c1ip(int K)
+{
+    const double u = std::ldexp(1.0, -8);
+    const double c = ((2.0 * u + u * u) + K * std::ldexp(1.0, -22) * (1.0 + u) * (1.0 + u) +
+                      (K + 5) * std::ldexp(1.0, -53) + std::ldexp(1.0, -22)) * (1.0 + std::ldexp(1.0, -10));
+    return std::nextafter((float)c, INFINITY);
+}
+
 }  // namespace
 
-extern "C" int pr_flat_create(pr_flat_t **out, int device, const float *rows_dev, int64_t n, int32_t d)
+extern "C" int pr_flat_create_metric(pr_flat_t **out, int device, const float *rows_dev, int64_t n, int32_t d,
+                                     int metric)
 {
+    const char *fn = metric == PR_METRIC_L2 ? "pr_flat_create" : "pr_flat_create_metric";
     if (!out || (n > 0 && !rows_dev) || n < 0) {
-        pr_set_error("pr_flat_create: bad argument (null pointer or negative row count)");
+        pr_set_error("%s: bad argument (null pointer or negative row count)", fn);
         return PR_EINVAL;
     }
     *out = nullptr;
+    if (metric != PR_METRIC_L2 && metric != PR_METRIC_INNER_PRODUCT) {
+        pr_set_error("%s: metric %d unsupported (PR_METRIC_INNER_PRODUCT = 0 or PR_METRIC_L2 = 1)", fn, metric);
+        return PR_EUNSUPPORTED;
+    }
     if (d < 64 || d > PR_FLAT_MAX_D || d % 64 != 0) {
-        pr_set_error("pr_flat_create: d = %d unsupported (a multiple of 64 in [64, %d])", d, PR_FLAT_MAX_D);
+        pr_set_error("%s: d = %d unsupported (a multiple of 64 in [64, %d])", fn, d, PR_FLAT_MAX_D);
         return PR_EUNSUPPORTED;
     }
     if (n > INT32_MAX) {
-        pr_set_error("pr_flat_create: %lld rows, at most 2^31 - 1 per index", (long long)n);
+        pr_set_error("%s: %lld rows, at most 2^31 - 1 per index", fn, (long long)n);
         return PR_EUNSUPPORTED;
     }
     if ((uintptr_t)rows_dev & 15) {
-        pr_set_error("pr_flat_create: rows_dev must be 16-byte aligned");
+        pr_set_error("%s: rows_dev must be 16-byte aligned", fn);
         return PR_EINVAL;
     }
     PR_CUDA_CHECK(cudaSetDevice(device));
@@ -523,8 +612,14 @@ extern "C" int pr_flat_create(pr_flat_t **out, int device, const float *rows_dev
     h->n = n;
     h->d = d;
     h->rows = rows_dev;
+    h->metric = metric;
     *out = h;
     return PR_OK;
+}
+
+extern "C" int pr_flat_create(pr_flat_t **out, int device, const float *rows_dev, int64_t n, int32_t d)
+{
+    return pr_flat_create_metric(out, device, rows_dev, n, d, PR_METRIC_L2);
 }
 
 extern "C" int pr_flat_destroy(pr_flat_t *h)
@@ -632,7 +727,9 @@ extern "C" int pr_flat_search(pr_flat_t *h, int32_t n_queries, const float *quer
     unsigned long long *stats = (unsigned long long *)(ws + l.stats);
     const int64_t total = (int64_t)n_queries * k;
 
-    flat_init_kernel<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(n_queries, k, theta, count, topk, stats);
+    const bool ip = h->metric == PR_METRIC_INNER_PRODUCT;
+    flat_init_kernel<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(n_queries, k, ip ? -INFINITY : INFINITY, theta,
+                                                                     count, topk, stats);
     int64_t launches = 1;
     if (h->n > 0) {
         flat_prep_kernel<<<(unsigned)((l.b_pad + 7) / 8), 256, 0, st>>>(queries_dev, n_queries, l.b_pad, h->d, q_bf, qn2, qn);
@@ -651,8 +748,8 @@ extern "C" int pr_flat_search(pr_flat_t *h, int32_t n_queries, const float *quer
         fa.idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(l.nq >> 3) << 17) | ((uint32_t)(kRowsPerTile >> 4) << 24);
         fa.tmem_cols = 32;
         while (fa.tmem_cols < (uint32_t)(2 * l.nq)) fa.tmem_cols <<= 1;
-        fa.c1 = margin_c1(h->d);
-        fa.c2 = std::ldexp(1.f, -17);
+        fa.c1 = ip ? margin_c1ip(h->d) : margin_c1(h->d);
+        fa.c2 = ip ? 0.f : std::ldexp(1.f, -17);
         fa.c3 = std::ldexp(1.f, -100);
         fa.norm2 = h->norm2;
         fa.norm = h->norm;
@@ -663,11 +760,12 @@ extern "C" int pr_flat_search(pr_flat_t *h, int32_t n_queries, const float *quer
         fa.cand = cand;
         fa.cap = tun.cand_capacity;
         const size_t smem = 1024 + (size_t)fa.n_stages * stage_bytes + (2 * kMaxStages + 4) * 8 + 16;
-        static bool attr_done = false;   // (idempotent; a race only repeats the call)
-        if (!attr_done) {
-            PR_CUDA_CHECK(cudaFuncSetAttribute((const void *)flat_filter_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+        const void *filter = ip ? (const void *)flat_ip_filter_kernel : (const void *)flat_filter_kernel;
+        static bool attr_done[2] = {false, false};   // (idempotent; a race only repeats the call)
+        if (!attr_done[ip]) {
+            PR_CUDA_CHECK(cudaFuncSetAttribute(filter, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                                1024 + kStageBudget + (2 * kMaxStages + 4) * 8 + 16));
-            attr_done = true;
+            attr_done[ip] = true;
         }
         RefineArgs ra;
         ra.rows = h->rows;
@@ -687,8 +785,13 @@ extern "C" int pr_flat_search(pr_flat_t *h, int32_t n_queries, const float *quer
             fa.row_end = ra.row_end = end;
             const int64_t tiles = (end - begin + kRowsPerTile - 1) / kRowsPerTile * l.n_qb;
             const unsigned grid = (unsigned)std::min<int64_t>(tiles, h->n_sm);
-            flat_filter_kernel<<<grid, kFilterThreads, smem, st>>>(map_x, map_q, fa);
-            flat_refine_kernel<<<n_queries, kRefineThreads, 0, st>>>(ra);
+            if (ip) {
+                flat_ip_filter_kernel<<<grid, kFilterThreads, smem, st>>>(map_x, map_q, fa);
+                flat_ip_refine_kernel<<<n_queries, kRefineThreads, 0, st>>>(ra);
+            } else {
+                flat_filter_kernel<<<grid, kFilterThreads, smem, st>>>(map_x, map_q, fa);
+                flat_refine_kernel<<<n_queries, kRefineThreads, 0, st>>>(ra);
+            }
             PR_CUDA_CHECK(cudaGetLastError());
             launches += 2;
             ++h->last_chunks;
@@ -696,7 +799,8 @@ extern "C" int pr_flat_search(pr_flat_t *h, int32_t n_queries, const float *quer
             chunk = std::min<int64_t>(chunk * tun.growth, (int64_t)1 << 40);
         }
     }
-    flat_output_kernel<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(total, topk, out_dist_dev, out_ids_dev);
+    flat_output_kernel<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(total, topk, out_dist_dev, out_ids_dev,
+                                                                       h->metric);
     PR_CUDA_CHECK(cudaGetLastError());
     h->last_launches = launches + 1;
     return PR_OK;
@@ -723,26 +827,32 @@ extern "C" int pr_flat_last_stats(const pr_flat_t *h, const void *workspace_dev,
     return PR_OK;
 }
 
-extern "C" int pr_flat_merge(int32_t n_queries, int32_t k, int32_t n_lists, const float *dist_dev, const int64_t *ids_dev,
-                             const int64_t *id_base, float *out_dist_dev, int64_t *out_ids_dev, pr_stream_t stream)
+extern "C" int pr_flat_merge_metric(int32_t n_queries, int32_t k, int32_t n_lists, const float *dist_dev,
+                                    const int64_t *ids_dev, const int64_t *id_base, float *out_dist_dev,
+                                    int64_t *out_ids_dev, pr_stream_t stream, int metric)
 {
+    const char *fn = metric == PR_METRIC_L2 ? "pr_flat_merge" : "pr_flat_merge_metric";
     if (n_queries < 0 || !id_base ||
         (n_queries > 0 && (!dist_dev || !ids_dev || !out_dist_dev || !out_ids_dev))) {
-        pr_set_error("pr_flat_merge: bad argument (null pointer or negative batch)");
+        pr_set_error("%s: bad argument (null pointer or negative batch)", fn);
         return PR_EINVAL;
     }
+    if (metric != PR_METRIC_L2 && metric != PR_METRIC_INNER_PRODUCT) {
+        pr_set_error("%s: metric %d unsupported (PR_METRIC_INNER_PRODUCT = 0 or PR_METRIC_L2 = 1)", fn, metric);
+        return PR_EUNSUPPORTED;
+    }
     if (n_lists < 1 || n_lists > PR_FLAT_MAX_LISTS) {
-        pr_set_error("pr_flat_merge: n_lists must be in [1, %d], got %d", PR_FLAT_MAX_LISTS, n_lists);
+        pr_set_error("%s: n_lists must be in [1, %d], got %d", fn, PR_FLAT_MAX_LISTS, n_lists);
         return PR_EINVAL;
     }
     if (k < 1 || k > PR_MAX_K) {
-        pr_set_error("pr_flat_merge: k must be in [1, %d], got %d", PR_MAX_K, k);
+        pr_set_error("%s: k must be in [1, %d], got %d", fn, PR_MAX_K, k);
         return PR_EINVAL;
     }
     MergeArgs a;
     for (int l = 0; l < n_lists; ++l) {
         if (id_base[l] < 0) {
-            pr_set_error("pr_flat_merge: id_base[%d] = %lld is negative", l, (long long)id_base[l]);
+            pr_set_error("%s: id_base[%d] = %lld is negative", fn, l, (long long)id_base[l]);
             return PR_EINVAL;
         }
         a.base[l] = id_base[l];
@@ -752,6 +862,7 @@ extern "C" int pr_flat_merge(int32_t n_queries, int32_t k, int32_t n_lists, cons
     a.n_queries = n_queries;
     a.k = k;
     a.n_lists = n_lists;
+    a.metric = metric;
     a.warps = (int)std::max<size_t>(1, std::min<size_t>(kMergeMaxWarps, kMergeSmemBudget / per_warp));
     a.dist = dist_dev;
     a.ids = ids_dev;
@@ -761,4 +872,11 @@ extern "C" int pr_flat_merge(int32_t n_queries, int32_t k, int32_t n_lists, cons
     flat_merge_kernel<<<grid, a.warps * 32, a.warps * per_warp, (cudaStream_t)stream>>>(a);
     PR_CUDA_CHECK(cudaGetLastError());
     return PR_OK;
+}
+
+extern "C" int pr_flat_merge(int32_t n_queries, int32_t k, int32_t n_lists, const float *dist_dev, const int64_t *ids_dev,
+                             const int64_t *id_base, float *out_dist_dev, int64_t *out_ids_dev, pr_stream_t stream)
+{
+    return pr_flat_merge_metric(n_queries, k, n_lists, dist_dev, ids_dev, id_base, out_dist_dev, out_ids_dev, stream,
+                                PR_METRIC_L2);
 }

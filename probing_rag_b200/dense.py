@@ -1,4 +1,5 @@
-"""Exact dense retrieval: a faiss ``IndexFlatL2`` drop-in on the GPU (include/probing_rag.h, "dense flat L2 search").
+"""Exact dense retrieval: faiss ``IndexFlatL2`` and ``IndexFlatIP`` drop-ins on the GPU (include/probing_rag.h, "dense
+flat L2 and inner-product search").
 
 The reference's dense path (``exp_rag.py`` without ``--is_sparse``) builds ``faiss.IndexFlatL2(768)`` over contriever
 embeddings (/root/reference/make_indexer.py:446-457), loads it with ``faiss.read_index`` (exp_rag.py:243-248) and calls
@@ -11,7 +12,9 @@ Under torchrun (one process per GPU), ``dense.read_index(path, sharded=True)`` g
 of the file and returns a ``ShardedIndexFlatL2``; its ``search`` returns, on every rank, the same lists as one index.
 
 ``D`` holds float32 squared L2 distances, ascending, ties broken by row id; ``I`` int64 row ids; rows short of k are
-(FLT_MAX, -1).  The distances are exact (float64 evaluation in a fixed order, DESIGN §3), so they can differ from
+(FLT_MAX, -1).  ``IndexFlatIP`` (Contriever's and DPR's own indexes, fourcc 'IxFI') returns inner products q.x instead,
+descending, ties by row id, NaN after -inf, rows short of k padded (-FLT_MAX, -1); ``read_index`` returns whichever class
+the file holds.  The distances are exact (float64 evaluation in a fixed order, DESIGN §3), so they can differ from
 faiss's own fp32 BLAS results in the last bits and near-ties may rank differently.  A CUDA tensor batch returns CUDA
 tensors without a host copy.  There is no CPU path: search runs the sm_100a kernels of libprobingrag.so.
 """
@@ -27,8 +30,10 @@ import torch.distributed as dist
 
 from . import _lib
 
-METRIC_L2 = 1
-FOURCC_FLAT_L2 = b"IxF2"
+METRIC_INNER_PRODUCT, METRIC_L2 = _lib.PR_METRIC_INNER_PRODUCT, _lib.PR_METRIC_L2     # faiss's numbering
+FOURCC_FLAT_L2, FOURCC_FLAT_IP = b"IxF2", b"IxFI"
+_FOURCC = {METRIC_L2: FOURCC_FLAT_L2, METRIC_INNER_PRODUCT: FOURCC_FLAT_IP}
+_NAME = {METRIC_L2: "IndexFlatL2", METRIC_INNER_PRODUCT: "IndexFlatIP"}
 _HEADER = struct.Struct("<4siqqqBiQ")     # fourcc, d, ntotal, 2 dummies, is_trained, metric_type, float count
 _COPY_BYTES = 256 << 20                  # host <-> device copies of rows go in pieces of this size
 
@@ -59,19 +64,17 @@ def _as_rows(x, d: int, what: str) -> torch.Tensor:
     return x
 
 
-class IndexFlatL2:
-    """faiss.IndexFlatL2 on one GPU: ``d``, ``ntotal``, ``is_trained``, ``metric_type``, ``add``, ``reset``,
-    ``search``.  The float32 rows live on ``device``; a bf16 copy and the row norms (half the rows' size again) are
-    built on the first search after an ``add``."""
+class _IndexFlat:
+    """A flat index of one metric (the subclass's ``metric_type``) on one GPU."""
 
     is_trained = True
-    metric_type = METRIC_L2
+    metric_type: int
 
     def __init__(self, d: int, device="cuda"):
         self.d = _check_d(d)
         self.device = torch.device(device)
         if self.device.type != "cuda":
-            raise ValueError(f"IndexFlatL2 needs a CUDA device, got {self.device}")
+            raise ValueError(f"{type(self).__name__} needs a CUDA device, got {self.device}")
         if self.device.index is None:
             self.device = torch.device("cuda", torch.cuda.current_device())
         self._rows = torch.empty((0, self.d), dtype=torch.float32, device=self.device)
@@ -89,7 +92,7 @@ class IndexFlatL2:
         """Append float32 rows [n, d] (NumPy array or tensor)."""
         x = self._as_rows(x, "x")
         if self.ntotal + x.shape[0] > 2 ** 31 - 1:
-            raise ValueError("an IndexFlatL2 holds at most 2^31 - 1 rows")
+            raise ValueError(f"an {type(self).__name__} holds at most 2^31 - 1 rows")
         self._set_rows(torch.cat([self._rows, x.to(self.device)]) if self.ntotal else x.to(self.device).contiguous())
 
     def reset(self) -> None:
@@ -97,7 +100,8 @@ class IndexFlatL2:
 
     @torch.no_grad()
     def search(self, x, k: int):
-        """(D, I) of the k nearest rows of every query row of x [B, d] float32."""
+        """(D, I) of the k nearest rows (L2) or the k largest inner products (IP) of every query row of x [B, d]
+        float32."""
         k = _check_k(k)
         as_numpy = isinstance(x, np.ndarray)
         if not as_numpy:
@@ -169,8 +173,8 @@ class IndexFlatL2:
             L = _lib.lib()
             h = ctypes.c_void_p()
             n = self.ntotal
-            _lib.check(L.pr_flat_create(ctypes.byref(h), self.device.index, self._rows.data_ptr() if n else None,
-                                        n, self.d))
+            _lib.check(L.pr_flat_create_metric(ctypes.byref(h), self.device.index,
+                                               self._rows.data_ptr() if n else None, n, self.d, self.metric_type))
             try:
                 _lib.check(L.pr_flat_set_tuning(h, ctypes.byref(self._tuning)))
                 nbytes = int(L.pr_flat_aux_bytes(h))
@@ -192,10 +196,27 @@ class IndexFlatL2:
             pass
 
 
+class IndexFlatL2(_IndexFlat):
+    """faiss.IndexFlatL2 on one GPU: ``d``, ``ntotal``, ``is_trained``, ``metric_type``, ``add``, ``reset``,
+    ``search``.  The float32 rows live on ``device``; a bf16 copy and the row norms (half the rows' size again) are
+    built on the first search after an ``add``."""
+
+    metric_type = METRIC_L2
+
+
+class IndexFlatIP(_IndexFlat):
+    """faiss.IndexFlatIP on one GPU, with the surface of IndexFlatL2.  ``search`` returns exact inner products q.x,
+    descending, ties by row id, NaN after -inf; rows short of k are (-FLT_MAX, -1)."""
+
+    metric_type = METRIC_INNER_PRODUCT
+
+
 # ---------------------------------------------------------------------- row-range shards over the GPUs of one box
-def merge_lists(dist_lists: torch.Tensor, id_lists: torch.Tensor, bases) -> tuple[torch.Tensor, torch.Tensor]:
-    """pr_flat_merge: ranked lists f32 / i64 [L, B, k] on one device, list l's ids offset by bases[l] -> the merged
-    (D [B, k], I [B, k]) in (distance bits, global id) order, short rows (FLT_MAX, -1)."""
+def merge_lists(dist_lists: torch.Tensor, id_lists: torch.Tensor, bases,
+                metric: int = METRIC_L2) -> tuple[torch.Tensor, torch.Tensor]:
+    """pr_flat_merge_metric: ranked lists f32 / i64 [L, B, k] on one device, list l's ids offset by bases[l] -> the
+    merged (D [B, k], I [B, k]) in the order of the metric's search: (distance bits, global id), short rows
+    (FLT_MAX, -1); METRIC_INNER_PRODUCT: (score descending with NaN last, global id), short rows (-FLT_MAX, -1)."""
     L_, B, k = dist_lists.shape
     if tuple(id_lists.shape) != (L_, B, k) or len(bases) != L_:
         raise ValueError(f"lists {tuple(dist_lists.shape)} / {tuple(id_lists.shape)} with {len(bases)} bases")
@@ -209,31 +230,37 @@ def merge_lists(dist_lists: torch.Tensor, id_lists: torch.Tensor, bases) -> tupl
         base = (ctypes.c_int64 * L_)(*[int(b) for b in bases])
         dl, il = dist_lists.contiguous(), id_lists.contiguous()
         with torch.cuda.device(dev):
-            _lib.check(_lib.lib().pr_flat_merge(B, k, L_, dl.data_ptr(), il.data_ptr(), base, D.data_ptr(),
-                                                I.data_ptr(), torch.cuda.current_stream(dev).cuda_stream))
+            _lib.check(_lib.lib().pr_flat_merge_metric(B, k, L_, dl.data_ptr(), il.data_ptr(), base, D.data_ptr(),
+                                                       I.data_ptr(), torch.cuda.current_stream(dev).cuda_stream,
+                                                       metric))
     return D, I
 
 
-class ShardedIndexFlatL2:
-    """One rank's share of a row-range sharded IndexFlatL2: ``shard`` holds the global rows
-    [row_base, row_base + shard.ntotal).  One process per GPU (torchrun); every rank passes the same batch to
-    ``search`` and gets the same global (D, I), equal bit for bit to one IndexFlatL2 over all rows:
+class _ShardedIndexFlat:
+    """One rank's share of a row-range sharded flat index: ``shard`` (an index of the class's metric) holds the global
+    rows [row_base, row_base + shard.ntotal).  One process per GPU (torchrun); every rank passes the same batch to
+    ``search`` and gets the same global (D, I), equal bit for bit to one index over all rows:
 
         local search     pr_flat_search over this rank's rows                 [B, k] local ids
         all-gather       sharding.gather_lists                               [G, B, k], rank-major
-        merge            pr_flat_merge with every rank's row_base              global ids, (distance, id) order
+        merge            pr_flat_merge_metric with every rank's row_base       global ids, the single index's order
 
-    Each row is evaluated on exactly one rank, by the same exact distance as the single index, and the merge uses the
-    single index's key order, so ties (equal distances, even across shard boundaries) rank by global row id.
+    Each row is evaluated on exactly one rank, by the same exact distance or score as the single index, and the merge
+    uses the single index's key order, so ties (equal values, even across shard boundaries) rank by global row id.
     ``local_search(q, k) -> (D, I)`` and ``merge(D [G,B,k], I [G,B,k], bases) -> (D, I)`` can be injected (the host
     logic is then testable on CPU with an oracle standing in); with them, ``shard`` only needs ``d`` and ``ntotal``.
+    A shard whose ``metric_type`` is the other metric raises ValueError.
     Not supported: appending rows (``add``), writing the sharded index, one process driving several GPUs, multi-node."""
 
     is_trained = True
-    metric_type = METRIC_L2
+    metric_type: int
 
     def __init__(self, shard, row_base: int, group=None, local_search=None, merge=None):
         from . import sharding
+        m = getattr(shard, "metric_type", self.metric_type)
+        if m != self.metric_type:
+            raise ValueError(f"{type(self).__name__} needs shards of metric {self.metric_type} "
+                             f"({_NAME[self.metric_type]}), got a shard of metric {m}")
         self.shard, self.group = shard, group
         self.d = int(shard.d)
         self._local, self._merge = local_search, merge
@@ -289,7 +316,8 @@ class ShardedIndexFlatL2:
             gd, gi = self._gath[key] = sharding.gather_lists(Dl, Il, self.group, self._gath.get(key))
             if len(self._gath) > 16:
                 self._gath = {key: (gd, gi)}
-            D, I = (self._merge or merge_lists)(gd, gi, self.bases)
+            D, I = self._merge(gd, gi, self.bases) if self._merge else \
+                merge_lists(gd, gi, self.bases, self.metric_type)
         else:
             D, I = Dl, Il
         if as_numpy:
@@ -305,20 +333,49 @@ class ShardedIndexFlatL2:
         return self.shard.last_stats()
 
 
+class ShardedIndexFlatL2(_ShardedIndexFlat):
+    """Row-range shards of an IndexFlatL2 (see _ShardedIndexFlat): (distance asc, global id) order."""
+    metric_type = METRIC_L2
+
+
+class ShardedIndexFlatIP(_ShardedIndexFlat):
+    """Row-range shards of an IndexFlatIP (see _ShardedIndexFlat): (score desc with NaN last, global id) order."""
+    metric_type = METRIC_INNER_PRODUCT
+
+
 # ---------------------------------------------------------------------- persistence (faiss index_write.cpp layout)
-def _read_header(path: str):
-    """(d, ntotal, payload offset) of an IndexFlatL2 file; ValueError for any other index type or metric."""
+def _fourcc(path: str) -> bytes:
     with open(path, "rb") as f:
-        head = f.read(_HEADER.size)
+        head = f.read(4)
     if len(head) < 4:
         raise ValueError(f"{path}: not a faiss index file")
-    if head[:4] != FOURCC_FLAT_L2:
-        raise ValueError(f"{path}: index type {head[:4]!r} is not supported (only IndexFlatL2, fourcc 'IxF2')")
+    return head
+
+
+def _metric_of(path: str) -> int:
+    """The metric of a flat index file from its fourcc; ValueError for any other index type."""
+    head = _fourcc(path)
+    for metric, fourcc in _FOURCC.items():
+        if head == fourcc:
+            return metric
+    raise ValueError(f"{path}: index type {head!r} is not supported (only IndexFlatL2, fourcc 'IxF2', and "
+                     f"IndexFlatIP, fourcc 'IxFI')")
+
+
+def _read_header(path: str, metric: int = METRIC_L2):
+    """(d, ntotal, payload offset) of a flat index file of `metric`; ValueError for any other index type or metric."""
+    fourcc = _FOURCC[metric]
+    head = _fourcc(path)
+    if head != fourcc:
+        raise ValueError(f"{path}: index type {head!r} is not supported here (only {_NAME[metric]}, "
+                         f"fourcc {fourcc.decode()!r})")
+    with open(path, "rb") as f:
+        head = f.read(_HEADER.size)
     if len(head) < _HEADER.size:
         raise ValueError(f"{path}: truncated header")
-    _, d, ntotal, _, _, _, metric, count = _HEADER.unpack(head)
-    if metric != METRIC_L2:
-        raise ValueError(f"{path}: metric_type {metric} is not supported (only METRIC_L2 = 1)")
+    _, d, ntotal, _, _, _, m, count = _HEADER.unpack(head)
+    if m != metric:
+        raise ValueError(f"{path}: metric_type {m} is not supported in an {_NAME[metric]} file (only {metric})")
     if ntotal < 0 or count != ntotal * d:
         raise ValueError(f"{path}: {count} floats stored for ntotal = {ntotal}, d = {d}")
     if os.path.getsize(path) < _HEADER.size + 4 * count:
@@ -326,49 +383,55 @@ def _read_header(path: str):
     return d, ntotal, _HEADER.size
 
 
-def read_rows(path: str) -> np.ndarray:
-    """The rows of an IndexFlatL2 file as a read-only memory map [ntotal, d] (nothing is read yet)."""
-    d, ntotal, off = _read_header(path)
+def read_rows(path: str, metric: int = METRIC_L2) -> np.ndarray:
+    """The rows of an IndexFlatL2 file (an IndexFlatIP file with metric=METRIC_INNER_PRODUCT) as a read-only memory
+    map [ntotal, d] (nothing is read yet)."""
+    d, ntotal, off = _read_header(path, metric)
     if ntotal == 0:
         return np.zeros((0, d), dtype=np.float32)
     return np.memmap(path, dtype="<f4", mode="r", offset=off, shape=(ntotal, d))
 
 
-def read_shard_rows(path: str, group=None):
-    """(row_base, rows): this rank's row range sharding.shard_range(ntotal, rank, world) of an IndexFlatL2 file, as a
-    read-only memory map (nothing is read yet)."""
+def read_shard_rows(path: str, group=None, metric: int = METRIC_L2):
+    """(row_base, rows): this rank's row range sharding.shard_range(ntotal, rank, world) of a flat index file of
+    `metric`, as a read-only memory map (nothing is read yet)."""
     from . import sharding
-    rows_mm = read_rows(path)
+    rows_mm = read_rows(path, metric)
     rank = dist.get_rank(group) if sharding._world(group) > 1 else 0
     lo, hi = sharding.shard_range(rows_mm.shape[0], rank, sharding._world(group))
     return lo, rows_mm[lo:hi]
 
 
 def read_index(path: str, device="cuda", sharded: bool = False, group=None):
-    """faiss.read_index for IndexFlatL2 files: the payload is memory-mapped and copied to the device in pieces, so a
-    64 GB index is never held in host RAM (not even once).  sharded=True (one process per GPU, torch.distributed
-    initialised, every rank of `group` calling): each rank copies only its row range (read_shard_rows) and gets a
-    ShardedIndexFlatL2 whose search covers the whole file."""
+    """faiss.read_index for IndexFlatL2 and IndexFlatIP files (the fourcc picks the class): the payload is
+    memory-mapped and copied to the device in pieces, so a 64 GB index is never held in host RAM (not even once).
+    sharded=True (one process per GPU, torch.distributed initialised, every rank of `group` calling): each rank copies
+    only its row range (read_shard_rows) and gets a ShardedIndexFlatL2 / ShardedIndexFlatIP whose search covers the
+    whole file."""
+    metric = _metric_of(path)
     if sharded:
-        row_base, rows_mm = read_shard_rows(path, group)
+        row_base, rows_mm = read_shard_rows(path, group, metric)
     else:
-        row_base, rows_mm = 0, read_rows(path)
-    index = IndexFlatL2(rows_mm.shape[1], device)
+        row_base, rows_mm = 0, read_rows(path, metric)
+    cls, sharded_cls = (IndexFlatL2, ShardedIndexFlatL2) if metric == METRIC_L2 else (IndexFlatIP, ShardedIndexFlatIP)
+    index = cls(rows_mm.shape[1], device)
     n, d = rows_mm.shape
     rows = torch.empty((n, d), dtype=torch.float32, device=index.device)
     step = max(1, _COPY_BYTES // (4 * d))
     for a in range(0, n, step):
         rows[a:a + step].copy_(torch.from_numpy(np.array(rows_mm[a:a + step], dtype=np.float32)))
     index._set_rows(rows)
-    return ShardedIndexFlatL2(index, row_base, group) if sharded else index
+    return sharded_cls(index, row_base, group) if sharded else index
 
 
-def write_rows(path: str, rows, d: int) -> None:
-    """Write float32 rows [n, d] (NumPy array, or a tensor copied to the host piece by piece) as an IndexFlatL2
-    file readable by faiss.read_index."""
+def write_rows(path: str, rows, d: int, metric: int = METRIC_L2) -> None:
+    """Write float32 rows [n, d] (NumPy array, or a tensor copied to the host piece by piece) as an IndexFlatL2 file
+    (metric=METRIC_INNER_PRODUCT: an IndexFlatIP file) readable by faiss.read_index."""
+    if metric not in _FOURCC:
+        raise ValueError(f"metric {metric!r} unsupported (METRIC_L2 = 1 or METRIC_INNER_PRODUCT = 0)")
     n = int(rows.shape[0])
     with open(path, "wb") as f:
-        f.write(_HEADER.pack(FOURCC_FLAT_L2, d, n, 1 << 20, 1 << 20, 1, METRIC_L2, n * d))
+        f.write(_HEADER.pack(_FOURCC[metric], d, n, 1 << 20, 1 << 20, 1, metric, n * d))
         step = max(1, _COPY_BYTES // (4 * d))
         for a in range(0, n, step):
             piece = rows[a:a + step]
@@ -377,8 +440,8 @@ def write_rows(path: str, rows, d: int) -> None:
             f.write(np.ascontiguousarray(piece, dtype="<f4").tobytes())
 
 
-def write_index(index: IndexFlatL2, path: str) -> None:
-    """faiss.write_index for an IndexFlatL2."""
-    if not isinstance(index, IndexFlatL2):
-        raise ValueError(f"write_index writes IndexFlatL2 only, got {type(index).__name__}")
-    write_rows(path, index.rows(), index.d)
+def write_index(index, path: str) -> None:
+    """faiss.write_index for an IndexFlatL2 or an IndexFlatIP."""
+    if not isinstance(index, _IndexFlat):
+        raise ValueError(f"write_index writes IndexFlatL2 and IndexFlatIP only, got {type(index).__name__}")
+    write_rows(path, index.rows(), index.d, index.metric_type)
