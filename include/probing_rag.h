@@ -182,7 +182,10 @@ int64_t pr_bm25_last_launches(const pr_index_t *index);
 /* k-way merge of per-shard ranked lists (the step after the NCCL all-gather, SURVEY 8e):
  *   scores_dev float[n_lists, n_queries, k], ids_dev int32[n_lists, n_queries, k]
  *   -> out_scores_dev float[n_queries, k], out_ids_dev int32[n_queries, k].
- * Entries with id < 0 are ignored. */
+ * Each input list is in the canonical order (score descending, id ascending), scores >= +0, and may end in padding
+ * (score < 0, id -1), which is ignored.  The inputs must hold at least k valid entries per query over all lists,
+ * which doc-range shards guarantee (each fills its zero-score tail, and together they hold >= k documents): the
+ * merge fills no zero-score tail of its own, so a query with fewer valid entries ends in (-inf, -1). */
 int pr_topk_merge(int32_t n_queries, int32_t k, int32_t n_lists, const float *scores_dev,
                   const int32_t *ids_dev, float *out_scores_dev, int32_t *out_ids_dev,
                   pr_stream_t stream);
