@@ -77,6 +77,14 @@ __device__ __forceinline__ uint32_t ip_key(uint32_t bits)
 
 __device__ __forceinline__ uint32_t ip_bits(uint32_t key) { return (key & 0x80000000u) ? key : key ^ 0x7FFFFFFFu; }
 
+// Key of a squared L2 distance's bits: the bits themselves (a distance is +0, positive or +inf), with every NaN, of
+// either sign and any payload, mapped to 0x7FFFFFFF, above +inf.  The key is also the distance returned, so a NaN
+// distance comes back as the NaN 0x7FFFFFFF.
+__device__ __forceinline__ uint32_t l2_key(uint32_t bits)
+{
+    return (bits & 0x7FFFFFFFu) > 0x7F800000u ? 0x7FFFFFFFu : bits;
+}
+
 __device__ __forceinline__ void tmem_ld32_nowait(uint32_t taddr, uint32_t (&r)[32])
 {
     asm volatile(
@@ -349,7 +357,7 @@ struct RefineArgs {
     int64_t row_begin, row_end;
     int32_t *count;
     const int32_t *cand;
-    uint64_t *topk;                 // [B][k] keys (f32 distance bits, or ip_key of the score, << 32 | row), ascending
+    uint64_t *topk;                 // [B][k] keys (l2_key of the distance or ip_key of the score, << 32 | row), ascending
     float *theta;
     unsigned long long *stats;      // candidates, max candidates, fallback queries
 };
@@ -384,7 +392,7 @@ __device__ __forceinline__ void flat_refine(const RefineArgs &g)
             const int64_t row = overflow ? g.row_begin + i : (int64_t)g.cand[(size_t)q * g.cap + i];
             uint32_t hi;
             if constexpr (M == PR_METRIC_L2)
-                hi = __float_as_uint(exact_dist(s_q, g.rows + row * g.d, g.d, lane));
+                hi = l2_key(__float_as_uint(exact_dist(s_q, g.rows + row * g.d, g.d, lane)));
             else
                 hi = ip_key(__float_as_uint(exact_ip(s_q, g.rows + row * g.d, g.d, lane)));
             const uint64_t key = ((uint64_t)hi << 32) | (uint64_t)row;
@@ -440,7 +448,7 @@ __global__ void flat_output_kernel(int64_t total, const uint64_t *__restrict__ t
 // ------------------------------------------------------------------------------------ merge of shard lists
 // One warp per query.  The query's n_lists lists are first staged in shared memory; lane l then holds the head of
 // list l (entries with id < 0 skipped) and each of the k rounds takes the warp-wide minimum of (key, global id, lane)
-// and advances the winner's list.  The key is the refine's: the distance bits (L2) or ip_key of the score (IP).  A head
+// and advances the winner's list.  The key is the refine's: l2_key of the distance or ip_key of the score.  A head
 // past the end of its list carries hi = 2^32, above every real key, so padding ranks after FLT_MAX and +inf (L2) or
 // -FLT_MAX, -inf and NaN (IP); once the minimum is padding, so is the rest.
 struct MergeArgs {
@@ -484,7 +492,7 @@ __global__ void __launch_bounds__(kMergeMaxWarps * 32) flat_merge_kernel(const M
     for (int r = 0; r < k; ++r) {
         const bool live = mine && pos < k;
         const uint32_t bits = live ? __float_as_uint(s_d[lane * k + pos]) : 0u;
-        uint64_t hi = live ? (uint64_t)(ip ? ip_key(bits) : bits) : (1ull << 32);
+        uint64_t hi = live ? (uint64_t)(ip ? ip_key(bits) : l2_key(bits)) : (1ull << 32);
         int64_t gid = live ? s_id[lane * k + pos] + base : INT64_MAX;
         int who = lane;
 #pragma unroll
@@ -761,12 +769,10 @@ extern "C" int pr_flat_search(pr_flat_t *h, int32_t n_queries, const float *quer
         fa.cap = tun.cand_capacity;
         const size_t smem = 1024 + (size_t)fa.n_stages * stage_bytes + (2 * kMaxStages + 4) * 8 + 16;
         const void *filter = ip ? (const void *)flat_ip_filter_kernel : (const void *)flat_filter_kernel;
-        static bool attr_done[2] = {false, false};   // (idempotent; a race only repeats the call)
-        if (!attr_done[ip]) {
-            PR_CUDA_CHECK(cudaFuncSetAttribute(filter, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                               1024 + kStageBudget + (2 * kMaxStages + 4) * 8 + 16));
-            attr_done[ip] = true;
-        }
+        // A function attribute holds for the current device only: set it on every call (host-only and cheap), so that
+        // an index on a second GPU of the process launches as the first one did.
+        PR_CUDA_CHECK(cudaFuncSetAttribute(filter, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                           1024 + kStageBudget + (2 * kMaxStages + 4) * 8 + 16));
         RefineArgs ra;
         ra.rows = h->rows;
         ra.queries = queries_dev;

@@ -589,15 +589,10 @@ extern "C" int pr_prober_forward(const pr_prober_set_t *ps, int32_t n_rows, cons
     const gemm_fn_t fc1 = x_dtype == 0 ? prober_gemm_kernel<1, float>
                           : x_dtype == 1 ? prober_gemm_kernel<1, __nv_bfloat16> : prober_gemm_kernel<1, __half>;
     const gemm_fn_t fc2 = prober_gemm_kernel<2, float>;
-    static bool attr_done[4] = {false, false, false, false};  // (idempotent; a race only repeats the call)
-    if (!attr_done[x_dtype]) {
-        PR_CUDA_CHECK(cudaFuncSetAttribute((const void *)fc1, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kGemmSmemBytes));
-        attr_done[x_dtype] = true;
-    }
-    if (!attr_done[3]) {
-        PR_CUDA_CHECK(cudaFuncSetAttribute((const void *)fc2, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kGemmSmemBytes));
-        attr_done[3] = true;
-    }
+    // A function attribute holds for the current device only: set it on every call (host-only and cheap), so that a
+    // gate on a second GPU of the process launches as the first one did.
+    PR_CUDA_CHECK(cudaFuncSetAttribute((const void *)fc1, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kGemmSmemBytes));
+    PR_CUDA_CHECK(cudaFuncSetAttribute((const void *)fc2, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kGemmSmemBytes));
     GemmArgs g;
     g.n_rows = n_rows;
     g.rows_pad = l.rows_pad;

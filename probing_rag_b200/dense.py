@@ -89,11 +89,15 @@ class _IndexFlat:
         return int(self._rows.shape[0])
 
     def add(self, x) -> None:
-        """Append float32 rows [n, d] (NumPy array or tensor)."""
+        """Append float32 rows [n, d] (NumPy array or tensor).  The rows are copied, as faiss copies them: changing
+        or reusing x afterwards leaves the index as it was."""
         x = self._as_rows(x, "x")
         if self.ntotal + x.shape[0] > 2 ** 31 - 1:
             raise ValueError(f"an {type(self).__name__} holds at most 2^31 - 1 rows")
-        self._set_rows(torch.cat([self._rows, x.to(self.device)]) if self.ntotal else x.to(self.device).contiguous())
+        if self.ntotal:
+            self._set_rows(torch.cat([self._rows, x.to(self.device)]))
+        else:       # a contiguous float32 tensor already on the device would otherwise be stored as it is
+            self._set_rows(x.to(self.device, memory_format=torch.contiguous_format, copy=True))
 
     def reset(self) -> None:
         self._set_rows(torch.empty((0, self.d), dtype=torch.float32, device=self.device))

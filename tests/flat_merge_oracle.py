@@ -1,8 +1,9 @@
 """CPU restatement of pr_flat_merge (csrc/flat.cu) -- TEST INFRASTRUCTURE ONLY.
 
   merge_canonical   per query, every entry of the L lists with id >= 0, its id offset by its list's base, ranked by
-                    (uint32 bit pattern of the distance, global id) ascending -- the key order of the single index's
-                    lists -- and cut to k; short rows padded (FLT_MAX, -1).  Entries equal in both keys keep list order.
+                    (uint32 bit pattern of the distance, every NaN as 0x7FFFFFFF; global id) ascending -- the key
+                    order of the single index's lists -- and cut to k; short rows padded (FLT_MAX, -1); a NaN comes
+                    back as 0x7FFFFFFF.  Entries equal in both keys keep list order.
 """
 from __future__ import annotations
 
@@ -18,7 +19,9 @@ def merge_canonical(D: np.ndarray, I: np.ndarray, bases, k: int):
     I = np.asarray(I, dtype=np.int64)
     L, B, kk = D.shape
     valid = I >= 0
-    hi = np.where(valid, D.view(np.uint32).astype(np.uint64), _EMPTY)
+    bits = D.view(np.uint32).astype(np.uint64)
+    bits = np.where((bits & np.uint64(0x7FFFFFFF)) > np.uint64(0x7F800000), np.uint64(0x7FFFFFFF), bits)
+    hi = np.where(valid, bits, _EMPTY)
     gid = np.where(valid, I + np.asarray(bases, dtype=np.int64)[:, None, None], np.iinfo(np.int64).max)
     hi = hi.transpose(1, 0, 2).reshape(B, L * kk)          # per query, list-major: equal keys keep list order
     gid = gid.transpose(1, 0, 2).reshape(B, L * kk)

@@ -21,10 +21,12 @@ FMAX = float(np.finfo(np.float32).max)
 # ---------------------------------------------------------------------------------------------- pr_flat_merge
 def _lists(rng, L, B, k, short="some", empty_list=False):
     """[L, B, k] ranked lists as pr_flat_search writes them: distances from a small set (exact ties within and
-    across lists, real FLT_MAX and +inf), distinct local ids per list, (distance bits, id) ascending, padded tails
-    whose distance is arbitrary."""
-    values = np.array([0.0, 0.25, 0.5, 1.0, 1.0 + 2 ** -23, 3.0, FMAX, np.inf], np.float32)
+    across lists, real FLT_MAX, +inf and NaN), distinct local ids per list, (distance bits, id) ascending with NaN
+    as 0x7FFFFFFF after +inf, padded tails whose distance is arbitrary.  A NaN is then given one of several bit
+    patterns (either sign, other payloads): the merge ranks and returns every NaN as 0x7FFFFFFF."""
+    values = np.array([0.0, 0.25, 0.5, 1.0, 1.0 + 2 ** -23, 3.0, FMAX, np.inf, np.nan], np.float32)
     dist_ = rng.choice(values, size=(L, B, k)).astype(np.float32)
+    dist_[np.isnan(dist_)] = np.uint32(0x7FFFFFFF).view(np.float32)
     ids = np.argsort(rng.random((L, B, 3 * k)), axis=-1)[:, :, :k].astype(np.int64)
     m = rng.integers(0, k + 1, size=(L, B)) if short == "some" else \
         (rng.integers(0, k, size=(L, B)) if short == "all" else np.full((L, B), k))
@@ -37,7 +39,10 @@ def _lists(rng, L, B, k, short="some", empty_list=False):
     pad = key == np.iinfo(np.uint64).max
     dist_ = (key >> np.uint64(32)).astype(np.uint32).view(np.float32)
     ids = (key & np.uint64(0xFFFFFFFF)).astype(np.int64)
-    dist_[pad] = rng.choice(np.array([FMAX, 0.0, 2.0], np.float32), size=int(pad.sum()))
+    nan = np.isnan(dist_)
+    dist_[nan] = rng.choice(np.array([0x7FFFFFFF, 0x7FC00000, 0xFFC00000, 0x7FC0BEEF, 0xFFFFFFFF], np.uint32),
+                            size=int(nan.sum())).view(np.float32)
+    dist_[pad] = rng.choice(np.array([FMAX, 0.0, 2.0, np.nan], np.float32), size=int(pad.sum()))
     ids[pad] = -1
     return dist_, ids
 
@@ -69,6 +74,10 @@ def _split(n, parts):
     return [r[0], (r[0][1], r[0][1])] + r[1:]
 
 
+def _same_bits(a, b):
+    return torch.equal(a.view(torch.int32), b.view(torch.int32))
+
+
 def _check_shards(rows, Q, k):
     single = IndexFlatL2(rows.shape[1])
     single.add(rows)
@@ -83,10 +92,10 @@ def _check_shards(rows, Q, k):
             Dl.append(d)
             Il.append(i)
         D, I = dense.merge_lists(torch.stack(Dl), torch.stack(Il), [lo for lo, _ in ranges])
-        assert torch.equal(I, Is) and torch.equal(D, Ds), f"{parts} shards differ from the single index"
+        assert torch.equal(I, Is) and _same_bits(D, Ds), f"{parts} shards differ from the single index"
     sx = ShardedIndexFlatL2(single, 0)                   # world 1 (no process group): the full path
     D, I = sx.search(Q, k)
-    assert sx.ntotal == rows.shape[0] and torch.equal(I, Is) and torch.equal(D, Ds)
+    assert sx.ntotal == rows.shape[0] and torch.equal(I, Is) and _same_bits(D, Ds)
     return Ds, Is
 
 
@@ -106,6 +115,23 @@ def test_simulated_shards_isotropic_and_ties():
     D, I = _check_shards(X, Q, 64)
     Dr, Ir = fo.search_canonical_torch(Q, X, 64)
     assert np.array_equal(I.cpu().numpy(), Ir) and np.array_equal(D.cpu().numpy(), Dr)
+
+
+def test_simulated_shards_nan_and_infinite_distances():
+    """NaN rows of several bit patterns and +-inf rows across every cut: the merge ranks NaN after +inf, by id, as the
+    single index does, and both return the NaN 0x7FFFFFFF."""
+    g = torch.Generator(device="cuda").manual_seed(7)
+    X = torch.randn((150, 128), generator=g, device="cuda")        # 30 NaN rows: every top-128 reaches them
+    nans = torch.tensor([0x7FC00000, 0xFFC00000, 0x7FC0BEEF, 0xFFFFFFFF], dtype=torch.int64).to(torch.int32)
+    X[3::5, 0] = nans.view(torch.float32).cuda().repeat(8)[:30]
+    X[[1, 75, 149], 1] = float("inf")
+    X[[2, 76], 2] = -float("inf")
+    Q = torch.randn((6, 128), generator=g, device="cuda")
+    Q[5, 0] = float("nan")
+    D, I = _check_shards(X, Q, 128)
+    bits = D.cpu().numpy().view(np.uint32)
+    assert np.all(bits[np.isnan(D.cpu().numpy())] == 0x7FFFFFFF) and np.isnan(D[0, -1].item())
+    assert torch.equal(I[5], torch.arange(128, device="cuda"))      # a NaN query: every distance NaN, id order
 
 
 # ---------------------------------------------------------------------------------------------- NCCL, one process per GPU
