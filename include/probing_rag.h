@@ -316,6 +316,22 @@ int pr_flat_search(pr_flat_t *index, int32_t n_queries, const float *queries_dev
 int pr_flat_last_stats(const pr_flat_t *index, const void *workspace_dev, int32_t n_queries, int32_t k,
                        pr_flat_stats_t *out, pr_stream_t stream);
 
+/* IndexFlatL2.range_search / IndexFlatIP.range_search(queries, radius) for the handle's metric (DESIGN §3):
+ *   L2  row r is a result of query q iff its exact distance D(q, r) < radius;  IP  iff its exact score S(q, r) > radius.
+ *   The values are those pr_flat_search returns; NaN values are never results, and a NaN radius gives none.
+ * Results are placed by the caller: query q's hits, in ascending row id, are written to dist_dev / ids_dev at
+ * [lims_in_dev[q], lims_in_dev[q + 1]) (i64 [n_queries + 1], on the device), and count_dev i64 [n_queries] receives
+ * each query's full number of hits, including those past the segment's end, which are not written.  Call it once with
+ * segments of a fixed staging size; if some count exceeds it, call it again with lims_in_dev = the exclusive prefix sum
+ * of the counts: the second call evaluates the same rows and writes every hit.  Results do not depend on the launch plan.
+ * A (query, chunk) with more candidates than min(cand_capacity, 8192) is scanned exactly, in row order.
+ * queries_dev 16-byte aligned, workspace_dev 1024-byte aligned, lims_in_dev, count_dev, ids_dev 8-byte aligned.
+ * Enqueues on `stream`, no sync.  pr_flat_last_stats(index, workspace, n_queries, 1, ...) reads its counters. */
+size_t pr_flat_range_workspace_bytes(const pr_flat_t *index, int32_t n_queries);
+int pr_flat_range_search(pr_flat_t *index, int32_t n_queries, const float *queries_dev, float radius,
+                         const int64_t *lims_in_dev, int64_t *count_dev, float *dist_dev, int64_t *ids_dev,
+                         void *workspace_dev, size_t workspace_bytes, pr_stream_t stream);
+
 /* Merge n_lists ranked dense lists per query into one, in the order pr_flat_search produces (the step after the
  * all-gather of a row-range sharded search, dense.ShardedIndexFlatL2).
  *   dist_dev f32 [n_lists][n_queries][k], ids_dev i64 [n_lists][n_queries][k]: each list sorted as pr_flat_search

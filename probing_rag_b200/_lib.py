@@ -95,6 +95,8 @@ SIGNATURES = {
     "pr_flat_workspace_bytes": (c_sz, [c_vp, c_i32, c_i32]),
     "pr_flat_search": (ctypes.c_int, [c_vp, c_i32, c_vp, c_i32, c_vp, c_vp, c_vp, c_sz, c_vp]),
     "pr_flat_last_stats": (ctypes.c_int, [c_vp, c_vp, c_i32, c_i32, ctypes.POINTER(FlatStats), c_vp]),
+    "pr_flat_range_workspace_bytes": (c_sz, [c_vp, c_i32]),
+    "pr_flat_range_search": (ctypes.c_int, [c_vp, c_i32, c_vp, c_f32, c_vp, c_vp, c_vp, c_vp, c_vp, c_sz, c_vp]),
     "pr_flat_merge": (ctypes.c_int, [c_i32, c_i32, c_i32, c_vp, c_vp, ctypes.POINTER(c_i64), c_vp, c_vp, c_vp]),
     "pr_flat_merge_metric": (ctypes.c_int, [c_i32, c_i32, c_i32, c_vp, c_vp, ctypes.POINTER(c_i64), c_vp, c_vp, c_vp,
                                             ctypes.c_int]),

@@ -24,6 +24,8 @@
 //            flat_ip_refine_kernel   the same with exact inner products; theta[q] = the k-th score, a lower bound of
 //                                    the final k-th score
 //   output   flat_output_kernel      running lists -> (distance, id) with (FLT_MAX, -1) padding, (-FLT_MAX, -1) for IP
+//   range    pr_flat_range_search: the same filter with theta[q] = radius throughout, then the range refine of
+//            flat_range.cu per chunk (each query's candidates in row order, hits appended to the query's segment)
 //   merge    flat_merge_kernel       pr_flat_merge: the lists of row-range shards -> one list in the same order
 //
 // The rows are cut into chunks of growing size; filter and refine alternate per chunk on the caller's stream, so
@@ -35,6 +37,7 @@
 #include <cuda_bf16.h>
 
 #include "common.cuh"
+#include "flat_exact.cuh"
 #include "tcgen05.cuh"
 
 struct pr_flat {
@@ -302,55 +305,6 @@ flat_ip_filter_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_co
 }
 
 // ------------------------------------------------------------------------------------ refine
-// The exact distance (DESIGN §3): lane l sums (q_j - x_j)^2 over j = l, l+32, ... in increasing j, every difference,
-// square and add a separately rounded f64 operation (no contraction), then an xor butterfly over the 32 lanes
-// (offsets 16, 8, 4, 2, 1), rounded once to f32.  Every lane ends with the same value.
-__device__ __forceinline__ float exact_dist(const float *__restrict__ sq, const float *__restrict__ x, int d, int lane)
-{
-    double s = 0.0;
-    for (int j = lane; j < d; j += 32) {
-        const double df = __dsub_rn((double)sq[j], (double)__ldg(x + j));
-        s = __dadd_rn(s, __dmul_rn(df, df));
-    }
-#pragma unroll
-    for (int o = 16; o; o >>= 1) s = __dadd_rn(s, __shfl_xor_sync(PR_FULL_MASK, s, o));
-    return __double2float_rn(s);
-}
-
-// The exact inner product (DESIGN §3): lane l starts at +0.0 and adds q_j x_j over j = l, l+32, ... in increasing j
-// (the product of two floats is exact in f64; __dmul_rn keeps it from contracting into an FMA), then the same butterfly
-// and one rounding to f32.  A negative sum that underflows f32 would round to -0; adding +0 makes it +0, so a score is
-// never -0.
-__device__ __forceinline__ float exact_ip(const float *__restrict__ sq, const float *__restrict__ x, int d, int lane)
-{
-    double s = 0.0;
-    for (int j = lane; j < d; j += 32) s = __dadd_rn(s, __dmul_rn((double)sq[j], (double)__ldg(x + j)));
-#pragma unroll
-    for (int o = 16; o; o >>= 1) s = __dadd_rn(s, __shfl_xor_sync(PR_FULL_MASK, s, o));
-    return __fadd_rn(__double2float_rn(s), 0.f);
-}
-
-// ascending bitonic sort of keys[0, n), n a power of two, by the whole block
-__device__ void block_bitonic_sort(uint64_t *keys, int n)
-{
-    for (int size = 2; size <= n; size <<= 1) {
-        for (int stride = size >> 1; stride > 0; stride >>= 1) {
-            __syncthreads();
-            for (int i = threadIdx.x; i < n / 2; i += blockDim.x) {
-                const int lo = 2 * i - (i & (stride - 1));
-                const int hi = lo + stride;
-                const bool asc = (lo & size) == 0;
-                const uint64_t a = keys[lo], b = keys[hi];
-                if ((a > b) == asc) {
-                    keys[lo] = b;
-                    keys[hi] = a;
-                }
-            }
-        }
-    }
-    __syncthreads();
-}
-
 struct RefineArgs {
     const float *rows, *queries;
     int d, k, cap;
@@ -830,6 +784,128 @@ extern "C" int pr_flat_last_stats(const pr_flat_t *h, const void *workspace_dev,
     out->candidates = (int64_t)s[0];
     out->max_candidates = (int64_t)s[1];
     out->fallback_queries = (int64_t)s[2];
+    return PR_OK;
+}
+
+// The workspace of a search at k = 1, so that pr_flat_last_stats(..., k = 1) reads the range search's counters.
+extern "C" size_t pr_flat_range_workspace_bytes(const pr_flat_t *h, int32_t n_queries)
+{
+    if (!h || n_queries < 1) return 0;
+    return flat_layout(h->d, n_queries, 1, effective_tuning(h).cand_capacity).total;
+}
+
+extern "C" int pr_flat_range_search(pr_flat_t *h, int32_t n_queries, const float *queries_dev, float radius,
+                                    const int64_t *lims_in_dev, int64_t *count_dev, float *dist_dev, int64_t *ids_dev,
+                                    void *workspace_dev, size_t workspace_bytes, pr_stream_t stream)
+{
+    if (!h || n_queries < 0 || (n_queries > 0 && (!queries_dev || !lims_in_dev || !count_dev || !dist_dev || !ids_dev ||
+                                                  !workspace_dev))) {
+        pr_set_error("pr_flat_range_search: bad argument (null pointer or negative batch)");
+        return PR_EINVAL;
+    }
+    if (h->n > 0 && !h->rows_bf) {
+        pr_set_error("pr_flat_range_search: pr_flat_build_aux has not been called on this handle");
+        return PR_EINVAL;
+    }
+    if (((uintptr_t)queries_dev & 15) || ((uintptr_t)workspace_dev & 1023) || ((uintptr_t)lims_in_dev & 7) ||
+        ((uintptr_t)count_dev & 7) || ((uintptr_t)dist_dev & 3) || ((uintptr_t)ids_dev & 7)) {
+        pr_set_error("pr_flat_range_search: queries_dev must be 16-byte aligned, workspace_dev 1024-byte aligned, "
+                     "lims_in_dev, count_dev and ids_dev 8-byte aligned, dist_dev 4-byte aligned");
+        return PR_EINVAL;
+    }
+    h->last_launches = 0;
+    h->last_chunks = 0;
+    if (n_queries == 0) return PR_OK;
+    const pr_flat_tuning_t tun = effective_tuning(h);
+    const FlatLayout l = flat_layout(h->d, n_queries, 1, tun.cand_capacity);
+    if (workspace_bytes < l.total) {
+        pr_set_error("pr_flat_range_search: workspace of %zu bytes, need %zu", workspace_bytes, l.total);
+        return PR_EWORKSPACE;
+    }
+    PR_CUDA_CHECK(cudaSetDevice(h->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    unsigned char *ws = (unsigned char *)workspace_dev;
+    PR_CUDA_CHECK(cudaMemsetAsync(count_dev, 0, (size_t)n_queries * sizeof(int64_t), st));
+    if (std::isnan(radius)) {                  // no results; the counters read zero
+        PR_CUDA_CHECK(cudaMemsetAsync(ws + l.stats, 0, 4 * 8, st));
+        return PR_OK;
+    }
+    __nv_bfloat16 *q_bf = (__nv_bfloat16 *)(ws + l.q_bf);
+    float *qn2 = (float *)(ws + l.qn2), *qn = (float *)(ws + l.qn), *theta = (float *)(ws + l.theta);
+    int32_t *count = (int32_t *)(ws + l.count), *cand = (int32_t *)(ws + l.cand);
+    unsigned long long *stats = (unsigned long long *)(ws + l.stats);
+
+    const bool ip = h->metric == PR_METRIC_INNER_PRODUCT;
+    flat_init_kernel<<<(unsigned)((n_queries + 255) / 256), 256, 0, st>>>(n_queries, 1, radius, theta, count,
+                                                                         (uint64_t *)(ws + l.topk), stats);
+    PR_CUDA_CHECK(cudaGetLastError());
+    int64_t launches = 1;
+    if (h->n > 0) {
+        flat_prep_kernel<<<(unsigned)((l.b_pad + 7) / 8), 256, 0, st>>>(queries_dev, n_queries, l.b_pad, h->d, q_bf, qn2, qn);
+        ++launches;
+        CUtensorMap map_x, map_q;
+        int rc;
+        if ((rc = make_map(&map_x, h->rows_bf, (uint64_t)h->n, (uint64_t)h->d, kRowsPerTile)) != PR_OK) return rc;
+        if ((rc = make_map(&map_q, q_bf, (uint64_t)l.b_pad, (uint64_t)h->d, (uint32_t)l.nq)) != PR_OK) return rc;
+        const int cap = std::min<int>(tun.cand_capacity, kFlatRangeMaxCap);
+        const int stage_bytes = kDocTileBytes + l.nq * kBK * 2;
+        FilterArgs fa;
+        fa.n_queries = n_queries;
+        fa.nq = l.nq;
+        fa.n_qb = l.n_qb;
+        fa.K = h->d;
+        fa.n_stages = std::min(kMaxStages, kStageBudget / stage_bytes);
+        fa.idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(l.nq >> 3) << 17) | ((uint32_t)(kRowsPerTile >> 4) << 24);
+        fa.tmem_cols = 32;
+        while (fa.tmem_cols < (uint32_t)(2 * l.nq)) fa.tmem_cols <<= 1;
+        fa.c1 = ip ? margin_c1ip(h->d) : margin_c1(h->d);
+        fa.c2 = ip ? 0.f : std::ldexp(1.f, -17);
+        fa.c3 = std::ldexp(1.f, -100);
+        fa.norm2 = h->norm2;
+        fa.norm = h->norm;
+        fa.qn2 = qn2;
+        fa.qn = qn;
+        fa.theta = theta;
+        fa.count = count;
+        fa.cand = cand;
+        fa.cap = cap;
+        const size_t smem = 1024 + (size_t)fa.n_stages * stage_bytes + (2 * kMaxStages + 4) * 8 + 16;
+        const void *filter = ip ? (const void *)flat_ip_filter_kernel : (const void *)flat_filter_kernel;
+        PR_CUDA_CHECK(cudaFuncSetAttribute(filter, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                           1024 + kStageBudget + (2 * kMaxStages + 4) * 8 + 16));
+        FlatRangeArgs ra;
+        ra.rows = h->rows;
+        ra.queries = queries_dev;
+        ra.d = h->d;
+        ra.cap = cap;
+        ra.radius = radius;
+        ra.count = count;
+        ra.cand = cand;
+        ra.lims = lims_in_dev;
+        ra.hits = count_dev;
+        ra.dist = dist_dev;
+        ra.ids = ids_dev;
+        ra.stats = stats;
+        int64_t chunk = (tun.first_chunk_rows + kRowsPerTile - 1) / kRowsPerTile * kRowsPerTile;
+        for (int64_t begin = 0; begin < h->n;) {
+            const int64_t end = std::min(h->n, begin + chunk);
+            fa.row_begin = ra.row_begin = begin;
+            fa.row_end = ra.row_end = end;
+            const int64_t tiles = (end - begin + kRowsPerTile - 1) / kRowsPerTile * l.n_qb;
+            const unsigned grid = (unsigned)std::min<int64_t>(tiles, h->n_sm);
+            if (ip)
+                flat_ip_filter_kernel<<<grid, kFilterThreads, smem, st>>>(map_x, map_q, fa);
+            else
+                flat_filter_kernel<<<grid, kFilterThreads, smem, st>>>(map_x, map_q, fa);
+            PR_CUDA_CHECK(cudaGetLastError());
+            if ((rc = flat_range_refine_launch(ra, h->metric, n_queries, st)) != PR_OK) return rc;
+            launches += 2;
+            ++h->last_chunks;
+            begin = end;
+            chunk = std::min<int64_t>(chunk * tun.growth, (int64_t)1 << 40);
+        }
+    }
+    h->last_launches = launches;
     return PR_OK;
 }
 

@@ -36,6 +36,8 @@ _FOURCC = {METRIC_L2: FOURCC_FLAT_L2, METRIC_INNER_PRODUCT: FOURCC_FLAT_IP}
 _NAME = {METRIC_L2: "IndexFlatL2", METRIC_INNER_PRODUCT: "IndexFlatIP"}
 _HEADER = struct.Struct("<4siqqqBiQ")     # fourcc, d, ntotal, 2 dummies, is_trained, metric_type, float count
 _COPY_BYTES = 256 << 20                  # host <-> device copies of rows go in pieces of this size
+_RANGE_CAP0 = 1024                       # range_search's first staging size per query ...
+_RANGE_STAGING_BYTES = 1 << 30           # ... and the most its staging buffers take (12 bytes a result)
 
 
 def _check_d(d) -> int:
@@ -82,6 +84,8 @@ class _IndexFlat:
         self._h = None
         self._aux = None
         self._last = None
+        self._range_cap = _RANGE_CAP0   # staging results per query of range_search: the most one query had last time
+        self._range_cap_forced = None   # tests: a fixed staging size (a tiny one takes the second pass)
 
     # ------------------------------------------------------------------ faiss interface
     @property
@@ -131,6 +135,46 @@ class _IndexFlat:
             return D.cpu().numpy(), I.cpu().numpy()
         return D, I
 
+    @torch.no_grad()
+    def range_search(self, x, radius):
+        """(lims, D, I): every row with exact distance D < radius (L2) or score S > radius (IP) for each query row of
+        x [B, d] float32; query q's results are D[lims[q]:lims[q + 1]], I[...], in ascending row id.  The radius is
+        rounded to float32 first; NaN values are never results.  NumPy in -> NumPy out with lims uint64 (faiss's
+        size_t), a CUDA tensor in -> CUDA tensors out with lims int64.  Synchronises the device once (twice when some
+        query has more results than the staging segments hold)."""
+        radius = float(np.float32(radius))
+        as_numpy = isinstance(x, np.ndarray)
+        if not as_numpy:
+            if not isinstance(x, torch.Tensor):
+                raise ValueError(f"queries must be a NumPy array or a CUDA tensor, got {type(x).__name__}")
+            if x.device != self.device:
+                raise ValueError(f"queries are on {x.device}, the index on {self.device}")
+        q = self._as_rows(x, "queries").to(self.device).contiguous()
+        B = q.shape[0]
+        lims = torch.zeros(B + 1, dtype=torch.int64, device=self.device)
+        D = torch.empty(0, dtype=torch.float32, device=self.device)
+        I = torch.empty(0, dtype=torch.int64, device=self.device)
+        if B:
+            cap = self._range_cap_forced or max(1, min(self._range_cap, self.ntotal, _RANGE_STAGING_BYTES // (12 * B)))
+            count = torch.empty(B, dtype=torch.int64, device=self.device)
+            Ds = torch.empty(B * cap, dtype=torch.float32, device=self.device)
+            Is = torch.empty(B * cap, dtype=torch.int64, device=self.device)
+            self._range_call(q, radius, torch.arange(B + 1, device=self.device) * cap, count, Ds, Is)
+            torch.cumsum(count, 0, out=lims[1:])
+            most = int(count.max())
+            if most <= cap:
+                keep = torch.arange(cap, device=self.device)[None, :] < count[:, None]
+                D, I = Ds.view(B, cap)[keep], Is.view(B, cap)[keep]
+            else:                           # the same rows again, written straight to their final places
+                total = int(lims[-1])
+                D = torch.empty(total, dtype=torch.float32, device=self.device)
+                I = torch.empty(total, dtype=torch.int64, device=self.device)
+                self._range_call(q, radius, lims, count, D, I)
+            self._range_cap = max(_RANGE_CAP0, most)
+        if as_numpy:
+            return lims.cpu().numpy().astype(np.uint64), D.cpu().numpy(), I.cpu().numpy()
+        return lims, D, I
+
     # ------------------------------------------------------------------ project extras
     def set_tuning(self, first_chunk_rows: int = 0, growth: int = 0, cand_capacity: int = 0) -> None:
         """Launch plan of the search (0 = default); tests force the one-chunk, many-chunk and overflow paths."""
@@ -144,8 +188,8 @@ class _IndexFlat:
         return {f: getattr(t, f) for f, _ in _lib.FlatTuning._fields_}
 
     def last_stats(self) -> dict:
-        """Launches, chunks, candidates (sum and max per query and chunk) and overflow fallbacks of the last search
-        (synchronises the device)."""
+        """Launches, chunks, candidates (sum and max per query and chunk) and overflow fallbacks of the last search or
+        of the last pass of the last range_search (synchronises the device)."""
         if self._last is None:
             raise ValueError("no search has run on this index")
         _ws, ws_ptr, B, k = self._last
@@ -162,6 +206,20 @@ class _IndexFlat:
     # ------------------------------------------------------------------ internals
     def _as_rows(self, x, what: str) -> torch.Tensor:
         return _as_rows(x, self.d, what)
+
+    def _range_call(self, q, radius: float, lims_in, count, D, I) -> None:
+        """One pr_flat_range_search: hits of query b into D, I at [lims_in[b], lims_in[b + 1]), all counts in count."""
+        L = _lib.lib()
+        h = self._handle()
+        B = q.shape[0]
+        nbytes = int(L.pr_flat_range_workspace_bytes(h, B))
+        ws = torch.empty(nbytes + 1024, dtype=torch.uint8, device=self.device)
+        ws_ptr = (ws.data_ptr() + 1023) // 1024 * 1024
+        with torch.cuda.device(self.device):
+            _lib.check(L.pr_flat_range_search(h, B, q.data_ptr(), radius, lims_in.data_ptr(), count.data_ptr(),
+                                              D.data_ptr(), I.data_ptr(), ws_ptr, nbytes,
+                                              torch.cuda.current_stream(self.device).cuda_stream))
+        self._last = (ws, ws_ptr, B, 1)
 
     def _set_rows(self, rows: torch.Tensor) -> None:
         self._release()
@@ -251,15 +309,19 @@ class _ShardedIndexFlat:
 
     Each row is evaluated on exactly one rank, by the same exact distance or score as the single index, and the merge
     uses the single index's key order, so ties (equal values, even across shard boundaries) rank by global row id.
-    ``local_search(q, k) -> (D, I)`` and ``merge(D [G,B,k], I [G,B,k], bases) -> (D, I)`` can be injected (the host
-    logic is then testable on CPU with an oracle standing in); with them, ``shard`` only needs ``d`` and ``ntotal``.
+    ``local_search(q, k) -> (D, I)``, ``merge(D [G,B,k], I [G,B,k], bases) -> (D, I)`` and
+    ``local_range(q, radius) -> (lims, D, I)`` (tensors) can be injected (the host logic is then testable on CPU with an
+    oracle standing in); with them, ``shard`` only needs ``d`` and ``ntotal``.
+    ``range_search`` gathers every rank's per-query counts and results and concatenates them per query in rank order
+    with global ids: the ranks hold ascending contiguous row ranges, so the result is in ascending global id and equals
+    one index's bit for bit.
     A shard whose ``metric_type`` is the other metric raises ValueError.
     Not supported: appending rows (``add``), writing the sharded index, one process driving several GPUs, multi-node."""
 
     is_trained = True
     metric_type: int
 
-    def __init__(self, shard, row_base: int, group=None, local_search=None, merge=None):
+    def __init__(self, shard, row_base: int, group=None, local_search=None, merge=None, local_range=None):
         from . import sharding
         m = getattr(shard, "metric_type", self.metric_type)
         if m != self.metric_type:
@@ -267,7 +329,7 @@ class _ShardedIndexFlat:
                              f"({_NAME[self.metric_type]}), got a shard of metric {m}")
         self.shard, self.group = shard, group
         self.d = int(shard.d)
-        self._local, self._merge = local_search, merge
+        self._local, self._merge, self._local_range = local_search, merge, local_range
         self._gath = {}
         self.device = getattr(shard, "device", torch.device("cpu"))
         world = sharding._world(group)
@@ -327,6 +389,56 @@ class _ShardedIndexFlat:
         if as_numpy:
             return D.cpu().numpy(), I.cpu().numpy()
         return D, I
+
+    @torch.no_grad()
+    def range_search(self, x, radius):
+        """(lims, D, I) of IndexFlatL2.range_search over ALL ranks' rows (the same batch and radius on every rank),
+        ids global and ascending per query; NumPy in -> NumPy out (lims uint64), a CUDA tensor in -> CUDA tensors
+        out (lims int64)."""
+        from . import sharding
+        as_numpy = isinstance(x, np.ndarray)
+        q = _as_rows(x, self.d, "queries")
+        if self._local_range is not None:
+            lims_l, Dl, Il = self._local_range(q, radius)
+        else:
+            if not as_numpy and q.device != self.device:
+                raise ValueError(f"queries are on {q.device}, the index on {self.device}")
+            lims_l, Dl, Il = self.shard.range_search(q.to(self.device), radius)
+        B, dev = q.shape[0], lims_l.device
+        if B == 0:
+            return (np.zeros(1, np.uint64), Dl.cpu().numpy(), Il.cpu().numpy()) if as_numpy else (lims_l, Dl, Il)
+        world = sharding._world(self.group)
+        counts = (lims_l[1:] - lims_l[:-1]).contiguous()
+        if world > 1:
+            every = torch.empty((world, B), dtype=torch.int64, device=dev)
+            dist.all_gather_into_tensor(every.view(-1), counts, group=self.group)
+        else:
+            every = counts[None]
+        totals = every.sum(1)
+        width = max(1, int(totals.max()))                       # every rank's results, padded to the largest
+        pad_d = torch.zeros(width, dtype=torch.float32, device=dev)
+        pad_i = torch.zeros(width, dtype=torch.int64, device=dev)
+        pad_d[:Dl.numel()], pad_i[:Il.numel()] = Dl, Il
+        gd, gi = sharding.gather_lists(pad_d[None], pad_i[None], self.group)
+        gd, gi = gd.view(world, width), gi.view(world, width)
+        # the results of rank g, query b go to lims[b] + (the results of ranks < g for query b)
+        flat = every.reshape(-1)                                                   # (g, b) rank-major
+        start_gb = torch.cumsum(flat, 0) - flat                                    # their place in the gathered order
+        by_b = every.T.reshape(-1)                                                 # (b, g) query-major
+        out_bg = (torch.cumsum(by_b, 0) - by_b).view(B, world).T.reshape(-1)      # their place in the output, (g, b)
+        seg = torch.repeat_interleave(torch.arange(world * B, device=dev), flat)
+        pos = out_bg[seg] + torch.arange(seg.numel(), device=dev) - start_gb[seg]
+        keep = torch.arange(width, device=dev)[None, :] < totals[:, None]
+        bases = torch.tensor(self.bases, dtype=torch.int64, device=dev)
+        D = torch.empty(seg.numel(), dtype=torch.float32, device=dev)
+        I = torch.empty(seg.numel(), dtype=torch.int64, device=dev)
+        D[pos] = gd[keep]
+        I[pos] = (gi + bases[:, None])[keep]
+        lims = torch.zeros(B + 1, dtype=torch.int64, device=dev)
+        torch.cumsum(every.sum(0), 0, out=lims[1:])
+        if as_numpy:
+            return lims.cpu().numpy().astype(np.uint64), D.cpu().numpy(), I.cpu().numpy()
+        return lims, D, I
 
     # ------------------------------------------------------------------ project extras (this rank's shard)
     def set_tuning(self, first_chunk_rows: int = 0, growth: int = 0, cand_capacity: int = 0) -> None:

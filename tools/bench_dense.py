@@ -16,6 +16,13 @@ parity_checked: 16 queries at full size against the oracle's evaluation order (o
 the same IEEE float64 operations, run on the device over row chunks so the 64 GB matrix is never copied).
 A CPU baseline (the faiss BLAS restatement on a 1M-row slice, numpy on this host) is reported at its own size.
 --metric ip measures IndexFlatIP on the same rows (metric names dense_flat_ip_*); l2, the default, is unchanged.
+
+Range mode, --radius-ranks 10,100 (and/or --radius-values): range_search instead of search, one JSON line per (radius,
+batch).  The radius of rank R is the median over the batch of the exact R-th nearest distance (ip: R-th largest
+score), from the index's own search; --radius-values gives radii directly.  Each line has the time per call (CUDA
+events after warm-up; a call includes its host synchronise), hits and candidates per query, overflow fallbacks, how
+many of the timed calls needed the second pass, and parity_checked: 4 queries of the batch against the fast reference
+(tests/flat_range_fast_oracle.py, bit for bit) when the rows are finite.
 """
 from __future__ import annotations
 
@@ -98,6 +105,8 @@ def main():
     ap.add_argument("--kind", default="clustered", choices=("clustered", "isotropic"))
     ap.add_argument("--cpu-rows", type=int, default=1 << 20)
     ap.add_argument("--out", default=None)
+    ap.add_argument("--radius-ranks", default="")
+    ap.add_argument("--radius-values", default="")
     args = ap.parse_args()
     assert torch.cuda.is_available(), "bench_dense.py measures on a CUDA device"
     torch.cuda.set_device(0)
@@ -119,6 +128,8 @@ def main():
     index.search(synth.dense_queries(index.rows(), 1), 1)       # builds the bf16 copy and the norms
     torch.cuda.synchronize()
     build_s = time.perf_counter() - t0
+    if args.radius_ranks or args.radius_values:
+        return bench_range(args, index, emit, name, power, build_s)
     checked = parity(index, synth.dense_queries(index.rows(), 16, seed=99), 10, ip=ip)
     N, d = args.n, args.d
     for k in [int(s) for s in args.ks.split(",")]:
@@ -168,6 +179,57 @@ def main():
         emit({"metric": f"dense_flat_{args.metric}_cpu_baseline", "impl": "numpy restatement of faiss BLAS flat search",
               "n": Xc.shape[0], "d": d, "k": 10, "batch": B, "ms_per_call": round(s * 1e3, 2),
               "host_threads": torch.get_num_threads(), "note": "slice of the index; not extrapolated to the full size"})
+
+
+def bench_range(args, index, emit, name, power, build_s):
+    sys.path.insert(0, os.path.join(ROOT, "tests"))
+    from flat_range_fast_oracle import range_search_fast
+    ip = args.metric == "ip"
+    for B in [int(s) for s in args.batches.split(",")]:
+        Q = synth.dense_queries(index.rows(), B)
+        radii = []
+        for R in [int(s) for s in args.radius_ranks.split(",") if s]:
+            Dk, _ = index.search(Q, R)
+            radii.append((f"rank {R}", float(torch.median(Dk[:, R - 1]))))
+        radii += [("value", float(s)) for s in args.radius_values.split(",") if s]
+        for how, r in radii:
+            index._range_cap = 1024                          # every setting starts from the default staging size
+            passes = []
+            for _ in range(args.warmup):
+                index.range_search(Q, r)
+            torch.cuda.synchronize()
+            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            e0.record()
+            for _ in range(args.iters):
+                cap = index._range_cap
+                lims, D, I = index.range_search(Q, r)
+                passes.append(int((lims[1:] - lims[:-1]).max()) > min(cap, index.ntotal) if B else False)
+            e1.record()
+            torch.cuda.synchronize()
+            ms = e0.elapsed_time(e1) / args.iters
+            st = index.last_stats()
+            hits = (lims[1:] - lims[:-1]).double()
+            sel = torch.arange(min(4, B), device=Q.device)
+            checked = None                                   # not checked: the reference would copy every hit row
+            if int(lims[len(sel)]) <= 1 << 20:
+                want = range_search_fast(Q[sel], index.rows(), r, args.metric)
+                got = (lims[:len(sel) + 1].cpu().numpy(), D[:int(lims[len(sel)])].cpu().numpy(),
+                       I[:int(lims[len(sel)])].cpu().numpy())
+                checked = bool(np.array_equal(got[0], want[0]) and np.array_equal(got[2], want[2]) and
+                               np.array_equal(got[1].view(np.uint32), want[1].view(np.uint32)))
+            emit({
+                "metric": f"dense_flat_{args.metric}_range_search", "n": args.n, "d": args.d, "batch": B,
+                "data": args.kind, "radius": r, "radius_from": how + (" (median over the batch)" if how != "value" else ""),
+                "ms_per_call": round(ms, 4), "queries_per_s": round(B / (ms * 1e-3), 1),
+                "hits_mean_per_query": round(float(hits.mean()), 1), "hits_max_per_query": int(hits.max()),
+                "candidates_mean_per_query": round(st["candidates"] / B, 1),
+                "candidates_max_query_chunk": st["max_candidates"], "fallback_query_chunks": st["fallback_queries"],
+                "chunks": st["chunks"], "launches": st["launches"],
+                "calls_with_second_pass": sum(passes), "timed_calls": args.iters,
+                "parity_checked": checked, "parity_queries": len(sel), "index_build_s": round(build_s, 1),
+                "gpu": name, "power_limit": power,
+                "timing": f"CUDA events, {args.warmup} warm-up + {args.iters} calls, each ending in a host synchronise",
+            })
 
 
 if __name__ == "__main__":
