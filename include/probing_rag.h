@@ -301,8 +301,14 @@ typedef struct pr_flat_stats {
 int pr_flat_create(pr_flat_t **out, int device, const float *rows_dev, int64_t n, int32_t d);
 int pr_flat_create_metric(pr_flat_t **out, int device, const float *rows_dev, int64_t n, int32_t d, int metric);
 int pr_flat_destroy(pr_flat_t *index);
-/* The bf16 copy of the rows and their norms, built once into caller memory (1024-byte aligned) of
- * pr_flat_aux_bytes() bytes; the handle keeps the pointer.  pr_flat_build_aux synchronises `stream`. */
+/* faiss.IndexScalarQuantizer(d, QT_fp16, metric): a handle over caller-owned IEEE binary16 codes [n][d] (the rows as
+ * stored, e.g. torch's .to(float16) of the f32 rows: round to nearest even, overflow to +-inf), with the checks of
+ * pr_flat_create_metric (codes_dev 16-byte aligned).  Every other pr_flat_* function serves it, with the results an
+ * f32 handle returns over the decoded rows, bit for bit; its aux holds no copy of the rows (12 bytes a row: ||x||^2,
+ * ||x|| and the norm of the row's fp16-subnormal elements), and the filter runs on the codes (DESIGN §4.6). */
+int pr_flat_create_fp16(pr_flat_t **out, int device, const uint16_t *codes_dev, int64_t n, int32_t d, int metric);
+/* The bf16 copy of the rows and their norms (fp16 handle: the norms only), built once into caller memory (1024-byte
+ * aligned) of pr_flat_aux_bytes() bytes; the handle keeps the pointer.  pr_flat_build_aux synchronises `stream`. */
 size_t pr_flat_aux_bytes(const pr_flat_t *index);
 int pr_flat_build_aux(pr_flat_t *index, void *aux_dev, size_t aux_bytes, pr_stream_t stream);
 int pr_flat_set_tuning(pr_flat_t *index, const pr_flat_tuning_t *tuning);

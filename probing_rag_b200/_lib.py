@@ -87,6 +87,7 @@ SIGNATURES = {
                                          c_vp, c_vp, c_vp, c_vp, c_sz, c_vp]),
     "pr_flat_create": (ctypes.c_int, [ctypes.POINTER(c_vp), ctypes.c_int, c_vp, c_i64, c_i32]),
     "pr_flat_create_metric": (ctypes.c_int, [ctypes.POINTER(c_vp), ctypes.c_int, c_vp, c_i64, c_i32, ctypes.c_int]),
+    "pr_flat_create_fp16": (ctypes.c_int, [ctypes.POINTER(c_vp), ctypes.c_int, c_vp, c_i64, c_i32, ctypes.c_int]),
     "pr_flat_destroy": (ctypes.c_int, [c_vp]),
     "pr_flat_aux_bytes": (c_sz, [c_vp]),
     "pr_flat_build_aux": (ctypes.c_int, [c_vp, c_vp, c_sz, c_vp]),

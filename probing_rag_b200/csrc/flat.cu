@@ -27,6 +27,8 @@
 //   range    pr_flat_range_search: the same filter with theta[q] = radius throughout, then the range refine of
 //            flat_range.cu per chunk (each query's candidates in row order, hits appended to the query's segment)
 //   merge    flat_merge_kernel       pr_flat_merge: the lists of row-range shards -> one list in the same order
+//   fp16     pr_flat_create_fp16: rows stored as IEEE binary16 codes; the same host plan launches the fp16 kernels of
+//            flat_fp16.cu (the same GEMM and refines on the codes themselves, no bf16 copy)
 //
 // The rows are cut into chunks of growing size; filter and refine alternate per chunk on the caller's stream, so
 // every chunk filters with the bound the earlier ones established ("bounds raised between launches", as BM25 does).
@@ -38,6 +40,7 @@
 
 #include "common.cuh"
 #include "flat_exact.cuh"
+#include "flat_filter.cuh"
 #include "tcgen05.cuh"
 
 struct pr_flat {
@@ -49,57 +52,20 @@ struct pr_flat {
     const __nv_bfloat16 *rows_bf;   // aux: bf16 copy [n][d]
     const float *norm2, *norm;      // aux: ||x||^2, ||x|| (f32)
     int metric;                     // PR_METRIC_L2 or PR_METRIC_INNER_PRODUCT
+    int32_t fp16;                   // pr_flat_create_fp16 (in what was padding: the offsets of f32 handles are kept)
     pr_flat_tuning_t tun;
     int64_t last_launches, last_chunks;
+    const __half *codes;            // fp16 only (read only when fp16 != 0): the rows [n][d] and the aux ||x_sub||
+    const float *nsub;
 };
 
 namespace {
 
-constexpr int kRowsPerTile = 128;
-constexpr int kMaxNQ = 256;
-constexpr int kMaxStages = 8;
-constexpr int kDocTileBytes = kRowsPerTile * kBK * 2;   // 16 KB
-constexpr int kStageBudget = 192 * 1024;
-constexpr int kFilterThreads = 256;
-constexpr int kRefineThreads = 256;
-constexpr int kRefineKeys = 2048;                       // running list + new exact candidates of one round
-constexpr uint64_t kEmptyKey = ~0ull;
 constexpr int64_t kDefaultFirstChunk = 2048;
 constexpr int32_t kDefaultGrowth = 4;
 constexpr int32_t kDefaultCapacity = 8192;
 
 inline size_t up(size_t x, size_t a) { return (x + a - 1) / a * a; }
-
-// Key of an inner-product score's bits: ascends as the score descends (+inf first, -inf last), with every NaN mapped
-// to 0xFFFFFFFF, above -inf.  ip_bits inverts it (a NaN comes back as the NaN 0xFFFFFFFF).
-__device__ __forceinline__ uint32_t ip_key(uint32_t bits)
-{
-    if ((bits & 0x7FFFFFFFu) > 0x7F800000u) return 0xFFFFFFFFu;
-    return (bits & 0x80000000u) ? bits : bits ^ 0x7FFFFFFFu;
-}
-
-__device__ __forceinline__ uint32_t ip_bits(uint32_t key) { return (key & 0x80000000u) ? key : key ^ 0x7FFFFFFFu; }
-
-// Key of a squared L2 distance's bits: the bits themselves (a distance is +0, positive or +inf), with every NaN, of
-// either sign and any payload, mapped to 0x7FFFFFFF, above +inf.  The key is also the distance returned, so a NaN
-// distance comes back as the NaN 0x7FFFFFFF.
-__device__ __forceinline__ uint32_t l2_key(uint32_t bits)
-{
-    return (bits & 0x7FFFFFFFu) > 0x7F800000u ? 0x7FFFFFFFu : bits;
-}
-
-__device__ __forceinline__ void tmem_ld32_nowait(uint32_t taddr, uint32_t (&r)[32])
-{
-    asm volatile(
-        "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
-        "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, "
-        "%16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31}, [%32];\n"
-        : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-          "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]), "=r"(r[16]),
-          "=r"(r[17]), "=r"(r[18]), "=r"(r[19]), "=r"(r[20]), "=r"(r[21]), "=r"(r[22]), "=r"(r[23]), "=r"(r[24]),
-          "=r"(r[25]), "=r"(r[26]), "=r"(r[27]), "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
-        : "r"(taddr));
-}
 
 // ------------------------------------------------------------------------------------ prep
 // One warp per row: bf16 copy (RNE) and ||x||^2, ||x|| (summed in f64, rounded once to f32).  Rows in [n, n_out)
@@ -139,157 +105,6 @@ __global__ void flat_init_kernel(int n_queries, int k, float theta0, float *__re
     if (i < 4) stats[i] = 0;
 }
 
-// ------------------------------------------------------------------------------------ filter
-struct FilterArgs {
-    int64_t row_begin, row_end;     // the chunk
-    int n_queries, nq, n_qb;        // batch, queries per tile (multiple of 32), query blocks
-    int K;                          // d
-    int n_stages;
-    uint32_t idesc;
-    uint32_t tmem_cols;
-    float c1, c2, c3;               // margin(q, x) = c1 |q| |x| + c2 (|q|^2 + |x|^2) + c3 (1 + |q| + |x|) (IP: c2 = 0)
-    const float *norm2, *norm;      // rows
-    const float *qn2, *qn;          // queries
-    const float *theta;
-    int32_t *count;
-    int32_t *cand;
-    int cap;
-};
-
-// The GEMM and its pipeline are shared; M (PR_METRIC_*) selects only the epilogue's bound and comparison.
-template <int M>
-__device__ __forceinline__ void flat_filter(const CUtensorMap &map_x, const CUtensorMap &map_q, const FilterArgs &g)
-{
-    extern __shared__ unsigned char smem_dyn[];
-    unsigned char *smem = reinterpret_cast<unsigned char *>(((uintptr_t)smem_dyn + 1023) & ~(uintptr_t)1023);
-    const int stage_bytes = kDocTileBytes + g.nq * kBK * 2;
-    uint64_t *full_bar = reinterpret_cast<uint64_t *>(smem + (size_t)g.n_stages * stage_bytes);
-    uint64_t *empty_bar = full_bar + kMaxStages;
-    uint64_t *tfull_bar = empty_bar + kMaxStages;   // [2] accumulator complete
-    uint64_t *tempty_bar = tfull_bar + 2;           // [2] accumulator drained by the epilogue
-    uint32_t *tmem_slot = reinterpret_cast<uint32_t *>(tempty_bar + 2);
-
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int64_t n_row_tiles = (g.row_end - g.row_begin + kRowsPerTile - 1) / kRowsPerTile;
-    const int64_t n_tiles = n_row_tiles * g.n_qb;
-    const int n_kb = g.K / kBK;
-
-    if (warp == 1 && lane == 0) {
-        for (int s = 0; s < g.n_stages; ++s) {
-            mbar_init(&full_bar[s], 1);
-            mbar_init(&empty_bar[s], 1);
-        }
-        for (int a = 0; a < 2; ++a) {
-            mbar_init(&tfull_bar[a], 1);
-            mbar_init(&tempty_bar[a], 4);   // one arrival per epilogue warp
-        }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-    }
-    if (warp == 2) tmem_alloc_1cta(tmem_slot, g.tmem_cols);
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    const uint32_t tmem_base = *tmem_slot;
-
-    if (warp == 0 && lane == 0) {
-        // ===== TMA producer
-        uint32_t kb_total = 0;
-        for (int64_t t = blockIdx.x; t < n_tiles; t += gridDim.x) {
-            const int row0 = (int)(g.row_begin + (t / g.n_qb) * kRowsPerTile);
-            const int q0 = (int)(t % g.n_qb) * g.nq;
-            for (int kb = 0; kb < n_kb; ++kb, ++kb_total) {
-                const int s = (int)(kb_total % (uint32_t)g.n_stages);
-                const uint32_t ph = (kb_total / (uint32_t)g.n_stages) & 1u;
-                mbar_wait(&empty_bar[s], ph ^ 1u);
-                unsigned char *st = smem + (size_t)s * stage_bytes;
-                mbar_expect_tx(&full_bar[s], (uint32_t)stage_bytes);
-                tma_load_2d(st, &map_x, &full_bar[s], kb * kBK, row0);
-                tma_load_2d(st + kDocTileBytes, &map_q, &full_bar[s], kb * kBK, q0);
-            }
-        }
-    } else if (warp == 1 && lane == 0) {
-        // ===== MMA issuer: acc[a][128 rows][nq queries] = X_tile . Q_tile^T
-        uint32_t kb_total = 0, it = 0;
-        for (int64_t t = blockIdx.x; t < n_tiles; t += gridDim.x, ++it) {
-            const uint32_t a = it & 1u;
-            mbar_wait(&tempty_bar[a], ((it >> 1) & 1u) ^ 1u);
-            tc_fence_after();
-            const uint32_t d_tmem = tmem_base + a * (uint32_t)g.nq;
-            for (int kb = 0; kb < n_kb; ++kb, ++kb_total) {
-                const int s = (int)(kb_total % (uint32_t)g.n_stages);
-                const uint32_t ph = (kb_total / (uint32_t)g.n_stages) & 1u;
-                mbar_wait(&full_bar[s], ph);
-                tc_fence_after();
-                const uint32_t st = smem_u32(smem + (size_t)s * stage_bytes);
-                const uint64_t da = umma_desc_sw128(st), db = umma_desc_sw128(st + kDocTileBytes);
-#pragma unroll
-                for (int k = 0; k < kBK / 16; ++k) {
-                    const uint64_t adv = (uint64_t)((k * 16 * 2) >> 4);
-                    umma_bf16_1cta(d_tmem, da + adv, db + adv, g.idesc, (kb | k) ? 1u : 0u);
-                }
-                umma_commit_1cta(&empty_bar[s]);
-            }
-            umma_commit_1cta(&tfull_bar[a]);
-        }
-    } else if (warp >= 4) {
-        // ===== epilogue: thread = one row of the tile (TMEM lane), 32 query columns per tcgen05.ld
-        const int quad = warp & 3;
-        uint32_t it = 0;
-        for (int64_t t = blockIdx.x; t < n_tiles; t += gridDim.x, ++it) {
-            const uint32_t a = it & 1u;
-            const int64_t row = g.row_begin + (t / g.n_qb) * kRowsPerTile + quad * 32 + lane;
-            const int q0 = (int)(t % g.n_qb) * g.nq;
-            const bool live = row < g.row_end;
-            const float nx2 = (M == PR_METRIC_L2 && live) ? __ldg(g.norm2 + row) : 0.f;
-            const float nx = live ? __ldg(g.norm + row) : 0.f;
-            mbar_wait(&tfull_bar[a], (it >> 1) & 1u);
-            tc_fence_after();
-            const uint32_t taddr = tmem_base + a * (uint32_t)g.nq + ((uint32_t)(quad * 32) << 16);
-            for (int c0 = 0; c0 < g.nq && q0 + c0 < g.n_queries; c0 += 32) {
-                uint32_t r[32];
-                tmem_ld32_nowait(taddr + (uint32_t)c0, r);
-                asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-#pragma unroll
-                for (int j = 0; j < 32; ++j) {
-                    const int q = q0 + c0 + j;
-                    if (q >= g.n_queries) continue;   // (warp-uniform)
-                    bool take;
-                    if constexpr (M == PR_METRIC_L2) {
-                        const float qn2 = __ldg(g.qn2 + q), qn = __ldg(g.qn + q), th = __ldg(g.theta + q);
-                        const float s2 = qn2 + nx2;
-                        const float margin = fmaf(g.c1 * qn, nx, fmaf(g.c2, s2, g.c3 * (1.f + qn + nx)));
-                        const float bound = fmaf(-2.f, __uint_as_float(r[j]), s2) - margin;
-                        take = live && !(bound > th);          // (a NaN bound is a candidate)
-                    } else {
-                        const float qn = __ldg(g.qn + q), th = __ldg(g.theta + q);
-                        const float bound = __uint_as_float(r[j]) + fmaf(g.c1 * qn, nx, g.c3 * (1.f + qn + nx));
-                        take = live && !(bound < th);          // (a NaN bound is a candidate)
-                    }
-                    const unsigned m = __ballot_sync(PR_FULL_MASK, take);
-                    if (m) {
-                        int base = 0;
-                        const int leader = __ffs(m) - 1;
-                        if (lane == leader) base = atomicAdd(g.count + q, __popc(m));
-                        base = __shfl_sync(PR_FULL_MASK, base, leader);
-                        const int slot = base + __popc(m & ((1u << lane) - 1u));
-                        if (take && slot < g.cap) g.cand[(size_t)q * g.cap + slot] = (int32_t)row;
-                    }
-                }
-            }
-            tc_fence_before();
-            __syncwarp();
-            if (lane == 0) mbar_arrive(&tempty_bar[a]);
-        }
-    }
-    tc_fence_before();
-    __syncthreads();
-    if (warp == 2) {
-        tc_fence_after();
-        tmem_dealloc_1cta(tmem_base, g.tmem_cols);
-    }
-}
-
 __global__ void __launch_bounds__(kFilterThreads, 1)
 flat_filter_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_constant__ CUtensorMap map_q,
                    const FilterArgs g)
@@ -302,77 +117,6 @@ flat_ip_filter_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_co
                       const FilterArgs g)
 {
     flat_filter<PR_METRIC_INNER_PRODUCT>(map_x, map_q, g);
-}
-
-// ------------------------------------------------------------------------------------ refine
-struct RefineArgs {
-    const float *rows, *queries;
-    int d, k, cap;
-    int64_t row_begin, row_end;
-    int32_t *count;
-    const int32_t *cand;
-    uint64_t *topk;                 // [B][k] keys (l2_key of the distance or ip_key of the score, << 32 | row), ascending
-    float *theta;
-    unsigned long long *stats;      // candidates, max candidates, fallback queries
-};
-
-template <int M>
-__device__ __forceinline__ void flat_refine(const RefineArgs &g)
-{
-    __shared__ uint64_t s_keys[kRefineKeys];
-    __shared__ float s_q[PR_FLAT_MAX_D];
-    __shared__ int s_new;
-    const int q = blockIdx.x, warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int n_warps = blockDim.x >> 5;
-    const int cnt = g.count[q];
-    const bool overflow = cnt > g.cap;
-    const int64_t n_items = overflow ? g.row_end - g.row_begin : cnt;
-    for (int j = threadIdx.x; j < g.d; j += blockDim.x) s_q[j] = g.queries[(size_t)q * g.d + j];
-    for (int i = threadIdx.x; i < g.k; i += blockDim.x) s_keys[i] = g.topk[(size_t)q * g.k + i];
-    if (threadIdx.x == 0) {
-        s_new = 0;
-        if (cnt) {
-            atomicAdd(g.stats + 0, (unsigned long long)cnt);
-            atomicMax(g.stats + 1, (unsigned long long)cnt);
-        }
-        if (overflow) atomicAdd(g.stats + 2, 1ull);
-    }
-    __syncthreads();
-    uint64_t kth = s_keys[g.k - 1];
-    const int round = kRefineKeys - g.k;
-    for (int64_t base = 0; base < n_items; base += round) {
-        const int64_t end = min(n_items, base + round);
-        for (int64_t i = base + warp; i < end; i += n_warps) {
-            const int64_t row = overflow ? g.row_begin + i : (int64_t)g.cand[(size_t)q * g.cap + i];
-            uint32_t hi;
-            if constexpr (M == PR_METRIC_L2)
-                hi = l2_key(__float_as_uint(exact_dist(s_q, g.rows + row * g.d, g.d, lane)));
-            else
-                hi = ip_key(__float_as_uint(exact_ip(s_q, g.rows + row * g.d, g.d, lane)));
-            const uint64_t key = ((uint64_t)hi << 32) | (uint64_t)row;
-            if (lane == 0 && key < kth) s_keys[g.k + atomicAdd(&s_new, 1)] = key;
-        }
-        __syncthreads();
-        const int m = g.k + s_new;
-        if (m > g.k) {
-            int p = 1;
-            while (p < m) p <<= 1;
-            for (int i = m + threadIdx.x; i < p; i += blockDim.x) s_keys[i] = kEmptyKey;
-            block_bitonic_sort(s_keys, p);
-            kth = s_keys[g.k - 1];
-        }
-        __syncthreads();
-        if (threadIdx.x == 0) s_new = 0;
-        __syncthreads();
-    }
-    for (int i = threadIdx.x; i < g.k; i += blockDim.x) g.topk[(size_t)q * g.k + i] = s_keys[i];
-    if (threadIdx.x == 0) {
-        if constexpr (M == PR_METRIC_L2)
-            g.theta[q] = kth == kEmptyKey ? INFINITY : __uint_as_float((uint32_t)(kth >> 32));
-        else
-            g.theta[q] = kth == kEmptyKey ? -INFINITY : __uint_as_float(ip_bits((uint32_t)(kth >> 32)));
-        g.count[q] = 0;
-    }
 }
 
 __global__ void __launch_bounds__(kRefineThreads) flat_refine_kernel(const RefineArgs g) { flat_refine<PR_METRIC_L2>(g); }
@@ -479,11 +223,12 @@ __global__ void __launch_bounds__(kMergeMaxWarps * 32) flat_merge_kernel(const M
 // ------------------------------------------------------------------------------------ host
 struct FlatLayout {
     int nq, n_qb, b_pad;
-    size_t q_bf, qn2, qn, theta, count, cand, topk, stats, total;
+    size_t q_bf, qn2, qn, theta, count, cand, topk, stats, qscale, total;
 };
 
-// queries per tile: as few 32-column groups as cover the batch in equal blocks of at most 256
-FlatLayout flat_layout(int d, int n_queries, int k, int cap)
+// queries per tile: as few 32-column groups as cover the batch in equal blocks of at most 256.  fp16 storage: q_bf holds
+// the fp16 query copy and the per-query scales follow the counters.
+FlatLayout flat_layout(int d, int n_queries, int k, int cap, bool fp16)
 {
     FlatLayout l;
     l.n_qb = (n_queries + kMaxNQ - 1) / kMaxNQ;
@@ -499,12 +244,15 @@ FlatLayout flat_layout(int d, int n_queries, int k, int cap)
     l.cand = o;  o = up(o + (size_t)n_queries * cap * 4, 256);
     l.topk = o;  o = up(o + (size_t)n_queries * k * 8, 256);
     l.stats = o; o = up(o + 4 * 8, 256);
+    l.qscale = o;
+    if (fp16) o = up(o + (size_t)l.b_pad * 4, 256);
     l.total = o;
     return l;
 }
 
-size_t aux_norm2_offset(const pr_flat *h) { return up((size_t)h->n * h->d * 2, 256); }
+size_t aux_norm2_offset(const pr_flat *h) { return h->fp16 ? 0 : up((size_t)h->n * h->d * 2, 256); }
 size_t aux_norm_offset(const pr_flat *h) { return up(aux_norm2_offset(h) + (size_t)h->n * 4, 256); }
+size_t aux_nsub_offset(const pr_flat *h) { return up(aux_norm_offset(h) + (size_t)h->n * 4, 256); }
 
 pr_flat_tuning_t effective_tuning(const pr_flat *h)
 {
@@ -535,6 +283,35 @@ float margin_c1ip(int K)
     const double u = std::ldexp(1.0, -8);
     const double c = ((2.0 * u + u * u) + K * std::ldexp(1.0, -22) * (1.0 + u) * (1.0 + u) +
                       (K + 5) * std::ldexp(1.0, -53) + std::ldexp(1.0, -22)) * (1.0 + std::ldexp(1.0, -10));
+    return std::nextafter((float)c, INFINITY);
+}
+
+// fp16 storage (derivation: DESIGN §4.6, "The fp16 margin").  The rows are exact, only the scaled query is rounded:
+// u = 2^-11 relative where the scaled element is normal, and at most 2^-14 absolute (a subnormal flushed) where it is
+// not, which is sqrt(K) 2^-28 relative to |q||x| since max |q_j| 2^e_q >= 2^14; the assumed fp32 accumulation,
+// K 2^-22 relative to sum |q^_j x_j| <= (1 + 2^-10) |q||x|; then the same factor 2, f64 and f32 terms and head room as
+// the bf16 coefficients above.
+float margin_c1_f16(int K)
+{
+    const double u = std::ldexp(1.0, -11), a = u + std::sqrt((double)K) * std::ldexp(1.0, -28);
+    const double c = 2.0 * (a + K * std::ldexp(1.0, -22) * (1.0 + std::ldexp(1.0, -10))) * (1.0 + std::ldexp(1.0, -10));
+    return std::nextafter((float)c, INFINITY);
+}
+
+float margin_c1ip_f16(int K)
+{
+    const double u = std::ldexp(1.0, -11), a = u + std::sqrt((double)K) * std::ldexp(1.0, -28);
+    const double c = (a + K * std::ldexp(1.0, -22) * (1.0 + std::ldexp(1.0, -10)) + (K + 5) * std::ldexp(1.0, -53) +
+                      std::ldexp(1.0, -22)) * (1.0 + std::ldexp(1.0, -10));
+    return std::nextafter((float)c, INFINITY);
+}
+
+// The coefficient of |q| ||x_sub||: a tensor core that flushes the row's fp16-subnormal elements loses at most
+// |q^| ||x_sub|| <= (1 + 2^-10) |q| ||x_sub|| of the dot product (Cauchy-Schwarz), twice that in the L2 bound; the
+// second 1 + 2^-10 covers the f32 evaluation of the term.
+float margin_csub_f16(int metric)
+{
+    const double c = (metric == PR_METRIC_L2 ? 2.0 : 1.0) * (1.0 + std::ldexp(1.0, -10)) * (1.0 + std::ldexp(1.0, -10));
     return std::nextafter((float)c, INFINITY);
 }
 
@@ -584,6 +361,46 @@ extern "C" int pr_flat_create(pr_flat_t **out, int device, const float *rows_dev
     return pr_flat_create_metric(out, device, rows_dev, n, d, PR_METRIC_L2);
 }
 
+extern "C" int pr_flat_create_fp16(pr_flat_t **out, int device, const uint16_t *codes_dev, int64_t n, int32_t d,
+                                   int metric)
+{
+    if (!out || (n > 0 && !codes_dev) || n < 0) {
+        pr_set_error("pr_flat_create_fp16: bad argument (null pointer or negative row count)");
+        return PR_EINVAL;
+    }
+    *out = nullptr;
+    if (metric != PR_METRIC_L2 && metric != PR_METRIC_INNER_PRODUCT) {
+        pr_set_error("pr_flat_create_fp16: metric %d unsupported (PR_METRIC_INNER_PRODUCT = 0 or PR_METRIC_L2 = 1)",
+                     metric);
+        return PR_EUNSUPPORTED;
+    }
+    if (d < 64 || d > PR_FLAT_MAX_D || d % 64 != 0) {
+        pr_set_error("pr_flat_create_fp16: d = %d unsupported (a multiple of 64 in [64, %d])", d, PR_FLAT_MAX_D);
+        return PR_EUNSUPPORTED;
+    }
+    if (n > INT32_MAX) {
+        pr_set_error("pr_flat_create_fp16: %lld rows, at most 2^31 - 1 per index", (long long)n);
+        return PR_EUNSUPPORTED;
+    }
+    if ((uintptr_t)codes_dev & 15) {
+        pr_set_error("pr_flat_create_fp16: codes_dev must be 16-byte aligned");
+        return PR_EINVAL;
+    }
+    PR_CUDA_CHECK(cudaSetDevice(device));
+    int n_sm = 0;
+    PR_CUDA_CHECK(cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, device));
+    pr_flat *h = new pr_flat();
+    h->device = device;
+    h->n_sm = n_sm;
+    h->n = n;
+    h->d = d;
+    h->metric = metric;
+    h->fp16 = 1;
+    h->codes = (const __half *)codes_dev;
+    *out = h;
+    return PR_OK;
+}
+
 extern "C" int pr_flat_destroy(pr_flat_t *h)
 {
     delete h;
@@ -593,7 +410,7 @@ extern "C" int pr_flat_destroy(pr_flat_t *h)
 extern "C" size_t pr_flat_aux_bytes(const pr_flat_t *h)
 {
     if (!h) return 0;
-    return up(aux_norm_offset(h) + (size_t)h->n * 4, 256);
+    return up((h->fp16 ? aux_nsub_offset(h) : aux_norm_offset(h)) + (size_t)h->n * 4, 256);
 }
 
 extern "C" int pr_flat_build_aux(pr_flat_t *h, void *aux_dev, size_t aux_bytes, pr_stream_t stream)
@@ -611,12 +428,21 @@ extern "C" int pr_flat_build_aux(pr_flat_t *h, void *aux_dev, size_t aux_bytes, 
         return PR_EINVAL;
     }
     unsigned char *a = (unsigned char *)aux_dev;
-    h->rows_bf = (const __nv_bfloat16 *)a;
+    h->rows_bf = h->fp16 ? nullptr : (const __nv_bfloat16 *)a;
     h->norm2 = (const float *)(a + aux_norm2_offset(h));
     h->norm = (const float *)(a + aux_norm_offset(h));
+    if (h->fp16) h->nsub = (const float *)(a + aux_nsub_offset(h));
     if (h->n == 0) return PR_OK;
     PR_CUDA_CHECK(cudaSetDevice(h->device));
     cudaStream_t st = (cudaStream_t)stream;
+    if (h->fp16) {
+        int rc;
+        if ((rc = flat_fp16_prep_rows(h->codes, h->n, h->d, (float *)h->norm2, (float *)h->norm, (float *)h->nsub,
+                                      st)) != PR_OK)
+            return rc;
+        PR_CUDA_CHECK(cudaStreamSynchronize(st));
+        return PR_OK;
+    }
     const int64_t blocks = (h->n + 7) / 8;
     flat_prep_kernel<<<(unsigned)blocks, 256, 0, st>>>(h->rows, h->n, h->n, h->d, (__nv_bfloat16 *)h->rows_bf,
                                                        (float *)h->norm2, (float *)h->norm);
@@ -648,7 +474,7 @@ extern "C" int pr_flat_get_tuning(const pr_flat_t *h, pr_flat_tuning_t *t)
 extern "C" size_t pr_flat_workspace_bytes(const pr_flat_t *h, int32_t n_queries, int32_t k)
 {
     if (!h || n_queries < 1 || k < 1 || k > PR_MAX_K) return 0;
-    return flat_layout(h->d, n_queries, k, effective_tuning(h).cand_capacity).total;
+    return flat_layout(h->d, n_queries, k, effective_tuning(h).cand_capacity, h->fp16).total;
 }
 
 extern "C" int pr_flat_search(pr_flat_t *h, int32_t n_queries, const float *queries_dev, int32_t k, float *out_dist_dev,
@@ -662,7 +488,7 @@ extern "C" int pr_flat_search(pr_flat_t *h, int32_t n_queries, const float *quer
         pr_set_error("pr_flat_search: k must be in [1, %d], got %d", PR_MAX_K, k);
         return PR_EINVAL;
     }
-    if (h->n > 0 && !h->rows_bf) {
+    if (h->n > 0 && !h->norm2) {
         pr_set_error("pr_flat_search: pr_flat_build_aux has not been called on this handle");
         return PR_EINVAL;
     }
@@ -674,7 +500,7 @@ extern "C" int pr_flat_search(pr_flat_t *h, int32_t n_queries, const float *quer
     h->last_chunks = 0;
     if (n_queries == 0) return PR_OK;
     const pr_flat_tuning_t tun = effective_tuning(h);
-    const FlatLayout l = flat_layout(h->d, n_queries, k, tun.cand_capacity);
+    const FlatLayout l = flat_layout(h->d, n_queries, k, tun.cand_capacity, h->fp16);
     if (workspace_bytes < l.total) {
         pr_set_error("pr_flat_search: workspace of %zu bytes, need %zu", workspace_bytes, l.total);
         return PR_EWORKSPACE;
@@ -694,12 +520,21 @@ extern "C" int pr_flat_search(pr_flat_t *h, int32_t n_queries, const float *quer
                                                                      count, topk, stats);
     int64_t launches = 1;
     if (h->n > 0) {
-        flat_prep_kernel<<<(unsigned)((l.b_pad + 7) / 8), 256, 0, st>>>(queries_dev, n_queries, l.b_pad, h->d, q_bf, qn2, qn);
+        float *qscale = (float *)(ws + l.qscale);
+        int rc;
+        if (h->fp16) {
+            if ((rc = flat_fp16_prep_queries(queries_dev, n_queries, l.b_pad, h->d, (__half *)q_bf, qn2, qn, qscale,
+                                             st)) != PR_OK)
+                return rc;
+        } else {
+            flat_prep_kernel<<<(unsigned)((l.b_pad + 7) / 8), 256, 0, st>>>(queries_dev, n_queries, l.b_pad, h->d, q_bf, qn2, qn);
+        }
         ++launches;
         CUtensorMap map_x, map_q;
-        int rc;
-        if ((rc = make_map(&map_x, h->rows_bf, (uint64_t)h->n, (uint64_t)h->d, kRowsPerTile)) != PR_OK) return rc;
-        if ((rc = make_map(&map_q, q_bf, (uint64_t)l.b_pad, (uint64_t)h->d, (uint32_t)l.nq)) != PR_OK) return rc;
+        const CUtensorMapDataType dtype = h->fp16 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
+        const void *x_ops = h->fp16 ? (const void *)h->codes : (const void *)h->rows_bf;
+        if ((rc = make_map(&map_x, x_ops, (uint64_t)h->n, (uint64_t)h->d, kRowsPerTile, dtype)) != PR_OK) return rc;
+        if ((rc = make_map(&map_q, q_bf, (uint64_t)l.b_pad, (uint64_t)h->d, (uint32_t)l.nq, dtype)) != PR_OK) return rc;
         const int stage_bytes = kDocTileBytes + l.nq * kBK * 2;
         FilterArgs fa;
         fa.n_queries = n_queries;
@@ -707,12 +542,18 @@ extern "C" int pr_flat_search(pr_flat_t *h, int32_t n_queries, const float *quer
         fa.n_qb = l.n_qb;
         fa.K = h->d;
         fa.n_stages = std::min(kMaxStages, kStageBudget / stage_bytes);
-        fa.idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(l.nq >> 3) << 17) | ((uint32_t)(kRowsPerTile >> 4) << 24);
+        // D f32; A and B BF16 (format 1) or, for fp16 storage, F16 (format 0); N = nq; M = 128
+        fa.idesc = (1u << 4) | (h->fp16 ? 0u : (1u << 7) | (1u << 10)) | ((uint32_t)(l.nq >> 3) << 17) |
+                   ((uint32_t)(kRowsPerTile >> 4) << 24);
         fa.tmem_cols = 32;
         while (fa.tmem_cols < (uint32_t)(2 * l.nq)) fa.tmem_cols <<= 1;
-        fa.c1 = ip ? margin_c1ip(h->d) : margin_c1(h->d);
+        if (h->fp16)
+            fa.c1 = ip ? margin_c1ip_f16(h->d) : margin_c1_f16(h->d);
+        else
+            fa.c1 = ip ? margin_c1ip(h->d) : margin_c1(h->d);
         fa.c2 = ip ? 0.f : std::ldexp(1.f, -17);
         fa.c3 = std::ldexp(1.f, -100);
+        const FilterF16Args fh = {qscale, h->fp16 ? h->nsub : nullptr, h->fp16 ? margin_csub_f16(h->metric) : 0.f};
         fa.norm2 = h->norm2;
         fa.norm = h->norm;
         fa.qn2 = qn2;
@@ -729,6 +570,7 @@ extern "C" int pr_flat_search(pr_flat_t *h, int32_t n_queries, const float *quer
                                            1024 + kStageBudget + (2 * kMaxStages + 4) * 8 + 16));
         RefineArgs ra;
         ra.rows = h->rows;
+        ra.rows_h = h->fp16 ? h->codes : nullptr;
         ra.queries = queries_dev;
         ra.d = h->d;
         ra.k = k;
@@ -745,7 +587,10 @@ extern "C" int pr_flat_search(pr_flat_t *h, int32_t n_queries, const float *quer
             fa.row_end = ra.row_end = end;
             const int64_t tiles = (end - begin + kRowsPerTile - 1) / kRowsPerTile * l.n_qb;
             const unsigned grid = (unsigned)std::min<int64_t>(tiles, h->n_sm);
-            if (ip) {
+            if (h->fp16) {
+                if ((rc = flat_fp16_filter_launch(h->metric, grid, smem, map_x, map_q, fa, fh, st)) != PR_OK) return rc;
+                if ((rc = flat_fp16_refine_launch(h->metric, n_queries, ra, st)) != PR_OK) return rc;
+            } else if (ip) {
                 flat_ip_filter_kernel<<<grid, kFilterThreads, smem, st>>>(map_x, map_q, fa);
                 flat_ip_refine_kernel<<<n_queries, kRefineThreads, 0, st>>>(ra);
             } else {
@@ -773,7 +618,7 @@ extern "C" int pr_flat_last_stats(const pr_flat_t *h, const void *workspace_dev,
         pr_set_error("pr_flat_last_stats: bad argument");
         return PR_EINVAL;
     }
-    const FlatLayout l = flat_layout(h->d, n_queries, k, effective_tuning(h).cand_capacity);
+    const FlatLayout l = flat_layout(h->d, n_queries, k, effective_tuning(h).cand_capacity, h->fp16);
     unsigned long long s[4];
     PR_CUDA_CHECK(cudaSetDevice(h->device));
     PR_CUDA_CHECK(cudaMemcpyAsync(s, (const unsigned char *)workspace_dev + l.stats, sizeof(s), cudaMemcpyDeviceToHost,
@@ -791,7 +636,7 @@ extern "C" int pr_flat_last_stats(const pr_flat_t *h, const void *workspace_dev,
 extern "C" size_t pr_flat_range_workspace_bytes(const pr_flat_t *h, int32_t n_queries)
 {
     if (!h || n_queries < 1) return 0;
-    return flat_layout(h->d, n_queries, 1, effective_tuning(h).cand_capacity).total;
+    return flat_layout(h->d, n_queries, 1, effective_tuning(h).cand_capacity, h->fp16).total;
 }
 
 extern "C" int pr_flat_range_search(pr_flat_t *h, int32_t n_queries, const float *queries_dev, float radius,
@@ -803,7 +648,7 @@ extern "C" int pr_flat_range_search(pr_flat_t *h, int32_t n_queries, const float
         pr_set_error("pr_flat_range_search: bad argument (null pointer or negative batch)");
         return PR_EINVAL;
     }
-    if (h->n > 0 && !h->rows_bf) {
+    if (h->n > 0 && !h->norm2) {
         pr_set_error("pr_flat_range_search: pr_flat_build_aux has not been called on this handle");
         return PR_EINVAL;
     }
@@ -817,7 +662,7 @@ extern "C" int pr_flat_range_search(pr_flat_t *h, int32_t n_queries, const float
     h->last_chunks = 0;
     if (n_queries == 0) return PR_OK;
     const pr_flat_tuning_t tun = effective_tuning(h);
-    const FlatLayout l = flat_layout(h->d, n_queries, 1, tun.cand_capacity);
+    const FlatLayout l = flat_layout(h->d, n_queries, 1, tun.cand_capacity, h->fp16);
     if (workspace_bytes < l.total) {
         pr_set_error("pr_flat_range_search: workspace of %zu bytes, need %zu", workspace_bytes, l.total);
         return PR_EWORKSPACE;
@@ -841,12 +686,21 @@ extern "C" int pr_flat_range_search(pr_flat_t *h, int32_t n_queries, const float
     PR_CUDA_CHECK(cudaGetLastError());
     int64_t launches = 1;
     if (h->n > 0) {
-        flat_prep_kernel<<<(unsigned)((l.b_pad + 7) / 8), 256, 0, st>>>(queries_dev, n_queries, l.b_pad, h->d, q_bf, qn2, qn);
+        float *qscale = (float *)(ws + l.qscale);
+        int rc;
+        if (h->fp16) {
+            if ((rc = flat_fp16_prep_queries(queries_dev, n_queries, l.b_pad, h->d, (__half *)q_bf, qn2, qn, qscale,
+                                             st)) != PR_OK)
+                return rc;
+        } else {
+            flat_prep_kernel<<<(unsigned)((l.b_pad + 7) / 8), 256, 0, st>>>(queries_dev, n_queries, l.b_pad, h->d, q_bf, qn2, qn);
+        }
         ++launches;
         CUtensorMap map_x, map_q;
-        int rc;
-        if ((rc = make_map(&map_x, h->rows_bf, (uint64_t)h->n, (uint64_t)h->d, kRowsPerTile)) != PR_OK) return rc;
-        if ((rc = make_map(&map_q, q_bf, (uint64_t)l.b_pad, (uint64_t)h->d, (uint32_t)l.nq)) != PR_OK) return rc;
+        const CUtensorMapDataType dtype = h->fp16 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
+        const void *x_ops = h->fp16 ? (const void *)h->codes : (const void *)h->rows_bf;
+        if ((rc = make_map(&map_x, x_ops, (uint64_t)h->n, (uint64_t)h->d, kRowsPerTile, dtype)) != PR_OK) return rc;
+        if ((rc = make_map(&map_q, q_bf, (uint64_t)l.b_pad, (uint64_t)h->d, (uint32_t)l.nq, dtype)) != PR_OK) return rc;
         const int cap = std::min<int>(tun.cand_capacity, kFlatRangeMaxCap);
         const int stage_bytes = kDocTileBytes + l.nq * kBK * 2;
         FilterArgs fa;
@@ -855,12 +709,18 @@ extern "C" int pr_flat_range_search(pr_flat_t *h, int32_t n_queries, const float
         fa.n_qb = l.n_qb;
         fa.K = h->d;
         fa.n_stages = std::min(kMaxStages, kStageBudget / stage_bytes);
-        fa.idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(l.nq >> 3) << 17) | ((uint32_t)(kRowsPerTile >> 4) << 24);
+        // D f32; A and B BF16 (format 1) or, for fp16 storage, F16 (format 0); N = nq; M = 128
+        fa.idesc = (1u << 4) | (h->fp16 ? 0u : (1u << 7) | (1u << 10)) | ((uint32_t)(l.nq >> 3) << 17) |
+                   ((uint32_t)(kRowsPerTile >> 4) << 24);
         fa.tmem_cols = 32;
         while (fa.tmem_cols < (uint32_t)(2 * l.nq)) fa.tmem_cols <<= 1;
-        fa.c1 = ip ? margin_c1ip(h->d) : margin_c1(h->d);
+        if (h->fp16)
+            fa.c1 = ip ? margin_c1ip_f16(h->d) : margin_c1_f16(h->d);
+        else
+            fa.c1 = ip ? margin_c1ip(h->d) : margin_c1(h->d);
         fa.c2 = ip ? 0.f : std::ldexp(1.f, -17);
         fa.c3 = std::ldexp(1.f, -100);
+        const FilterF16Args fh = {qscale, h->fp16 ? h->nsub : nullptr, h->fp16 ? margin_csub_f16(h->metric) : 0.f};
         fa.norm2 = h->norm2;
         fa.norm = h->norm;
         fa.qn2 = qn2;
@@ -875,6 +735,7 @@ extern "C" int pr_flat_range_search(pr_flat_t *h, int32_t n_queries, const float
                                            1024 + kStageBudget + (2 * kMaxStages + 4) * 8 + 16));
         FlatRangeArgs ra;
         ra.rows = h->rows;
+        ra.rows_h = h->fp16 ? h->codes : nullptr;
         ra.queries = queries_dev;
         ra.d = h->d;
         ra.cap = cap;
@@ -893,12 +754,17 @@ extern "C" int pr_flat_range_search(pr_flat_t *h, int32_t n_queries, const float
             fa.row_end = ra.row_end = end;
             const int64_t tiles = (end - begin + kRowsPerTile - 1) / kRowsPerTile * l.n_qb;
             const unsigned grid = (unsigned)std::min<int64_t>(tiles, h->n_sm);
-            if (ip)
-                flat_ip_filter_kernel<<<grid, kFilterThreads, smem, st>>>(map_x, map_q, fa);
-            else
-                flat_filter_kernel<<<grid, kFilterThreads, smem, st>>>(map_x, map_q, fa);
-            PR_CUDA_CHECK(cudaGetLastError());
-            if ((rc = flat_range_refine_launch(ra, h->metric, n_queries, st)) != PR_OK) return rc;
+            if (h->fp16) {
+                if ((rc = flat_fp16_filter_launch(h->metric, grid, smem, map_x, map_q, fa, fh, st)) != PR_OK) return rc;
+                if ((rc = flat_fp16_range_refine_launch(h->metric, n_queries, ra, st)) != PR_OK) return rc;
+            } else {
+                if (ip)
+                    flat_ip_filter_kernel<<<grid, kFilterThreads, smem, st>>>(map_x, map_q, fa);
+                else
+                    flat_filter_kernel<<<grid, kFilterThreads, smem, st>>>(map_x, map_q, fa);
+                PR_CUDA_CHECK(cudaGetLastError());
+                if ((rc = flat_range_refine_launch(ra, h->metric, n_queries, st)) != PR_OK) return rc;
+            }
             launches += 2;
             ++h->last_chunks;
             begin = end;

@@ -217,8 +217,10 @@ encode_tiled_t get_encode_tiled()
     return fn;
 }
 
-// bf16 matrix [rows][cols] row-major -> tiles of box_rows x 64 columns, 128-byte swizzle
-int make_map(CUtensorMap *map, const void *base, uint64_t rows, uint64_t cols, uint32_t box_rows)
+// bf16 (or, with dtype = CU_TENSOR_MAP_DATA_TYPE_FLOAT16, fp16) matrix [rows][cols] row-major -> tiles of box_rows x
+// 64 columns, 128-byte swizzle
+int make_map(CUtensorMap *map, const void *base, uint64_t rows, uint64_t cols, uint32_t box_rows,
+             CUtensorMapDataType dtype = CU_TENSOR_MAP_DATA_TYPE_BFLOAT16)
 {
     encode_tiled_t enc = get_encode_tiled();
     if (!enc) {
@@ -229,7 +231,7 @@ int make_map(CUtensorMap *map, const void *base, uint64_t rows, uint64_t cols, u
     const cuuint64_t strides[1] = {cols * 2};
     const cuuint32_t box[2] = {(cuuint32_t)kBK, box_rows};
     const cuuint32_t estr[2] = {1, 1};
-    const CUresult r = enc(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void *>(base), dims, strides, box, estr,
+    const CUresult r = enc(map, dtype, 2, const_cast<void *>(base), dims, strides, box, estr,
                            CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                            CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     if (r != CUDA_SUCCESS) {

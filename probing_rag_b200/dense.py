@@ -14,7 +14,9 @@ of the file and returns a ``ShardedIndexFlatL2``; its ``search`` returns, on eve
 ``D`` holds float32 squared L2 distances, ascending, ties broken by row id; ``I`` int64 row ids; rows short of k are
 (FLT_MAX, -1).  ``IndexFlatIP`` (Contriever's and DPR's own indexes, fourcc 'IxFI') returns inner products q.x instead,
 descending, ties by row id, NaN after -inf, rows short of k padded (-FLT_MAX, -1); ``read_index`` returns whichever class
-the file holds.  The distances are exact (float64 evaluation in a fixed order, DESIGN §3), so they can differ from
+the file holds.  ``IndexScalarQuantizer(d, ScalarQuantizer.QT_fp16, metric)`` (fourcc 'IxSQ') stores the rows as fp16
+codes, a third of an IndexFlat's device memory, and returns bit for bit what IndexFlatL2 / IndexFlatIP returns over the
+fp16-decoded rows.  The distances are exact (float64 evaluation in a fixed order, DESIGN §3), so they can differ from
 faiss's own fp32 BLAS results in the last bits and near-ties may rank differently.  A CUDA tensor batch returns CUDA
 tensors without a host copy.  There is no CPU path: search runs the sm_100a kernels of libprobingrag.so.
 """
@@ -31,10 +33,13 @@ import torch.distributed as dist
 from . import _lib
 
 METRIC_INNER_PRODUCT, METRIC_L2 = _lib.PR_METRIC_INNER_PRODUCT, _lib.PR_METRIC_L2     # faiss's numbering
-FOURCC_FLAT_L2, FOURCC_FLAT_IP = b"IxF2", b"IxFI"
+FOURCC_FLAT_L2, FOURCC_FLAT_IP, FOURCC_SQ = b"IxF2", b"IxFI", b"IxSQ"
 _FOURCC = {METRIC_L2: FOURCC_FLAT_L2, METRIC_INNER_PRODUCT: FOURCC_FLAT_IP}
 _NAME = {METRIC_L2: "IndexFlatL2", METRIC_INNER_PRODUCT: "IndexFlatIP"}
 _HEADER = struct.Struct("<4siqqqBiQ")     # fourcc, d, ntotal, 2 dummies, is_trained, metric_type, float count
+_SQ_HEADER = struct.Struct("<4siqqqBiiifQQQ")   # IxSQ: the index header without the float count, then the
+#                                                 ScalarQuantizer: qtype, rangestat, rangestat_arg, d, code_size,
+#                                                 trained count (its floats follow, then the codes' byte count)
 _COPY_BYTES = 256 << 20                  # host <-> device copies of rows go in pieces of this size
 _RANGE_CAP0 = 1024                       # range_search's first staging size per query ...
 _RANGE_STAGING_BYTES = 1 << 30           # ... and the most its staging buffers take (12 bytes a result)
@@ -235,8 +240,7 @@ class _IndexFlat:
             L = _lib.lib()
             h = ctypes.c_void_p()
             n = self.ntotal
-            _lib.check(L.pr_flat_create_metric(ctypes.byref(h), self.device.index,
-                                               self._rows.data_ptr() if n else None, n, self.d, self.metric_type))
+            _lib.check(self._create(L, h, n))
             try:
                 _lib.check(L.pr_flat_set_tuning(h, ctypes.byref(self._tuning)))
                 nbytes = int(L.pr_flat_aux_bytes(h))
@@ -250,6 +254,10 @@ class _IndexFlat:
                 raise
             self._h, self._aux = h, aux
         return self._h
+
+    def _create(self, L, h, n: int) -> int:
+        return L.pr_flat_create_metric(ctypes.byref(h), self.device.index, self._rows.data_ptr() if n else None, n,
+                                       self.d, self.metric_type)
 
     def __del__(self):
         try:
@@ -271,6 +279,68 @@ class IndexFlatIP(_IndexFlat):
     descending, ties by row id, NaN after -inf; rows short of k are (-FLT_MAX, -1)."""
 
     metric_type = METRIC_INNER_PRODUCT
+
+
+class ScalarQuantizer:
+    """faiss.ScalarQuantizer's qtype numbering.  Only QT_fp16 is built; IndexScalarQuantizer raises for the others."""
+    QT_8bit, QT_4bit, QT_8bit_uniform, QT_4bit_uniform, QT_fp16, QT_8bit_direct, QT_6bit, QT_bf16, \
+        QT_8bit_direct_signed = range(9)
+
+
+class IndexScalarQuantizer(_IndexFlat):
+    """faiss.IndexScalarQuantizer(d, ScalarQuantizer.QT_fp16, metric) on one GPU: ``d``, ``ntotal``, ``is_trained``,
+    ``metric_type``, ``code_size`` (2 d), ``train`` (nothing to learn for fp16), ``add``, ``reset``, ``search``,
+    ``range_search``.  ``add`` encodes float32 rows to IEEE binary16 (round to nearest even, overflow to +-inf, as
+    numpy's astype(float16) and faiss's F16C encoder); only the codes (2 d bytes a row) and 12 bytes of norms a row
+    stay on the device.  Results are bit for bit those of IndexFlatL2 / IndexFlatIP over the decoded rows
+    ``codes().float()``; the tensor-core filter reads the codes themselves."""
+
+    def __init__(self, d: int, qtype: int, metric: int = METRIC_L2, device="cuda"):
+        if qtype != ScalarQuantizer.QT_fp16:
+            raise ValueError(f"qtype {qtype!r} unsupported: only ScalarQuantizer.QT_fp16 = {ScalarQuantizer.QT_fp16}")
+        if metric not in _FOURCC:
+            raise ValueError(f"metric {metric!r} unsupported (METRIC_L2 = 1 or METRIC_INNER_PRODUCT = 0)")
+        self.metric_type = int(metric)
+        self.qtype = int(qtype)
+        super().__init__(d, device)
+        self._rows = torch.empty((0, self.d), dtype=torch.float16, device=self.device)
+
+    @property
+    def code_size(self) -> int:
+        return 2 * self.d
+
+    def train(self, x) -> None:
+        """fp16 has no trained parameters: checks x as faiss would accept it and does nothing."""
+        self._as_rows(x, "x")
+
+    def add(self, x) -> None:
+        """Append float32 rows [n, d] (NumPy array or tensor), encoded to fp16 on the device in pieces, so that no
+        float32 copy of the whole input is made there."""
+        x = self._as_rows(x, "x")
+        n = x.shape[0]
+        if self.ntotal + n > 2 ** 31 - 1:
+            raise ValueError("an IndexScalarQuantizer holds at most 2^31 - 1 rows")
+        codes = torch.empty((self.ntotal + n, self.d), dtype=torch.float16, device=self.device)
+        codes[:self.ntotal].copy_(self._rows)
+        step = max(1, _COPY_BYTES // (4 * self.d))
+        for a in range(0, n, step):
+            codes[self.ntotal + a:self.ntotal + a + step].copy_(x[a:a + step].to(self.device).to(torch.float16))
+        self._set_rows(codes)
+
+    def reset(self) -> None:
+        self._set_rows(torch.empty((0, self.d), dtype=torch.float16, device=self.device))
+
+    def codes(self) -> torch.Tensor:
+        """The fp16 codes [ntotal, d] on the device (not a copy)."""
+        return self._rows
+
+    def rows(self) -> torch.Tensor:
+        """The decoded rows [ntotal, d] as a new float32 tensor on the device (4 d bytes a row)."""
+        return self._rows.float()
+
+    def _create(self, L, h, n: int) -> int:
+        return L.pr_flat_create_fp16(ctypes.byref(h), self.device.index, self._rows.data_ptr() if n else None, n,
+                                     self.d, self.metric_type)
 
 
 # ---------------------------------------------------------------------- row-range shards over the GPUs of one box
@@ -474,8 +544,48 @@ def _metric_of(path: str) -> int:
     for metric, fourcc in _FOURCC.items():
         if head == fourcc:
             return metric
-    raise ValueError(f"{path}: index type {head!r} is not supported (only IndexFlatL2, fourcc 'IxF2', and "
-                     f"IndexFlatIP, fourcc 'IxFI')")
+    raise ValueError(f"{path}: index type {head!r} is not supported (only IndexFlatL2, fourcc 'IxF2', "
+                     f"IndexFlatIP, fourcc 'IxFI', and IndexScalarQuantizer with QT_fp16, fourcc 'IxSQ')")
+
+
+def _read_sq_header(path: str):
+    """(d, ntotal, metric, codes offset) of an IndexScalarQuantizer file (faiss index_write.cpp: the index header, the
+    ScalarQuantizer, the codes); ValueError unless it holds QT_fp16 codes of a supported d and metric."""
+    size = os.path.getsize(path)
+    with open(path, "rb") as f:
+        head = f.read(_SQ_HEADER.size)
+        if len(head) < _SQ_HEADER.size:
+            raise ValueError(f"{path}: truncated header")
+        fourcc, d, ntotal, _, _, _, metric, qtype, _, _, sq_d, code_size, n_trained = _SQ_HEADER.unpack(head)
+        if fourcc != FOURCC_SQ:
+            raise ValueError(f"{path}: index type {fourcc!r} is not an IndexScalarQuantizer (fourcc 'IxSQ')")
+        if qtype != ScalarQuantizer.QT_fp16:
+            raise ValueError(f"{path}: qtype {qtype} is not supported (only QT_fp16 = {ScalarQuantizer.QT_fp16})")
+        if metric not in _FOURCC:
+            raise ValueError(f"{path}: metric_type {metric} is not supported (METRIC_L2 = 1 or METRIC_INNER_PRODUCT = 0)")
+        _check_d(d)
+        if sq_d != d or code_size != 2 * d or ntotal < 0:
+            raise ValueError(f"{path}: ScalarQuantizer d = {sq_d}, code_size = {code_size} for an index of d = {d}")
+        off = _SQ_HEADER.size + 4 * n_trained
+        f.seek(off)
+        raw = f.read(8)
+        if len(raw) < 8:
+            raise ValueError(f"{path}: truncated header")
+        (nbytes,) = struct.unpack("<Q", raw)
+    if nbytes != ntotal * code_size:
+        raise ValueError(f"{path}: {nbytes} code bytes stored for ntotal = {ntotal}, code_size = {code_size}")
+    if size < off + 8 + nbytes:
+        raise ValueError(f"{path}: truncated payload")
+    return d, ntotal, metric, off + 8
+
+
+def read_codes(path: str) -> tuple[np.ndarray, int]:
+    """(codes, metric) of an IndexScalarQuantizer(QT_fp16) file: the codes as a read-only float16 memory map
+    [ntotal, d] (nothing is read yet)."""
+    d, ntotal, metric, off = _read_sq_header(path)
+    if ntotal == 0:
+        return np.zeros((0, d), dtype=np.float16), metric
+    return np.memmap(path, dtype="<f2", mode="r", offset=off, shape=(ntotal, d)), metric
 
 
 def _read_header(path: str, metric: int = METRIC_L2):
@@ -519,11 +629,14 @@ def read_shard_rows(path: str, group=None, metric: int = METRIC_L2):
 
 
 def read_index(path: str, device="cuda", sharded: bool = False, group=None):
-    """faiss.read_index for IndexFlatL2 and IndexFlatIP files (the fourcc picks the class): the payload is
+    """faiss.read_index for IndexFlatL2, IndexFlatIP and IndexScalarQuantizer(QT_fp16) files (the fourcc picks the
+    class; the sharded classes take IndexScalarQuantizer shards of their metric): the payload is
     memory-mapped and copied to the device in pieces, so a 64 GB index is never held in host RAM (not even once).
     sharded=True (one process per GPU, torch.distributed initialised, every rank of `group` calling): each rank copies
     only its row range (read_shard_rows) and gets a ShardedIndexFlatL2 / ShardedIndexFlatIP whose search covers the
     whole file."""
+    if _fourcc(path) == FOURCC_SQ:
+        return _read_sq_index(path, device, sharded, group)
     metric = _metric_of(path)
     if sharded:
         row_base, rows_mm = read_shard_rows(path, group, metric)
@@ -538,6 +651,48 @@ def read_index(path: str, device="cuda", sharded: bool = False, group=None):
         rows[a:a + step].copy_(torch.from_numpy(np.array(rows_mm[a:a + step], dtype=np.float32)))
     index._set_rows(rows)
     return sharded_cls(index, row_base, group) if sharded else index
+
+
+def _read_sq_index(path: str, device, sharded: bool, group):
+    """read_index for an 'IxSQ' file: the codes are memory-mapped and copied to the device in pieces; sharded=True
+    copies this rank's row range only and returns a ShardedIndexFlatL2 / ShardedIndexFlatIP over it."""
+    from . import sharding
+    codes_mm, metric = read_codes(path)
+    row_base = 0
+    if sharded:
+        rank = dist.get_rank(group) if sharding._world(group) > 1 else 0
+        row_base, hi = sharding.shard_range(codes_mm.shape[0], rank, sharding._world(group))
+        codes_mm = codes_mm[row_base:hi]
+    n, d = codes_mm.shape
+    index = IndexScalarQuantizer(d, ScalarQuantizer.QT_fp16, metric, device)
+    codes = torch.empty((n, d), dtype=torch.float16, device=index.device)
+    step = max(1, _COPY_BYTES // (2 * d))
+    for a in range(0, n, step):
+        codes[a:a + step].copy_(torch.from_numpy(np.array(codes_mm[a:a + step], dtype=np.float16)))
+    index._set_rows(codes)
+    if not sharded:
+        return index
+    return (ShardedIndexFlatL2 if metric == METRIC_L2 else ShardedIndexFlatIP)(index, row_base, group)
+
+
+def write_codes(path: str, codes, d: int, metric: int = METRIC_L2) -> None:
+    """Write fp16 codes [n, d] (a float16 NumPy array, or a tensor copied to the host piece by piece) as an
+    IndexScalarQuantizer(d, QT_fp16, metric) file readable by faiss.read_index."""
+    if metric not in _FOURCC:
+        raise ValueError(f"metric {metric!r} unsupported (METRIC_L2 = 1 or METRIC_INNER_PRODUCT = 0)")
+    n = int(codes.shape[0])
+    with open(path, "wb") as f:
+        f.write(_SQ_HEADER.pack(FOURCC_SQ, d, n, 1 << 20, 1 << 20, 1, metric, ScalarQuantizer.QT_fp16, 0, 0.0, d,
+                                2 * d, 0))
+        f.write(struct.pack("<Q", n * 2 * d))
+        step = max(1, _COPY_BYTES // (2 * d))
+        for a in range(0, n, step):
+            piece = codes[a:a + step]
+            if isinstance(piece, torch.Tensor):
+                piece = piece.cpu().numpy()
+            if piece.dtype != np.float16:
+                raise ValueError(f"codes must be float16, got {piece.dtype}")
+            f.write(np.ascontiguousarray(piece, dtype="<f2").tobytes())
 
 
 def write_rows(path: str, rows, d: int, metric: int = METRIC_L2) -> None:
@@ -557,7 +712,11 @@ def write_rows(path: str, rows, d: int, metric: int = METRIC_L2) -> None:
 
 
 def write_index(index, path: str) -> None:
-    """faiss.write_index for an IndexFlatL2 or an IndexFlatIP."""
+    """faiss.write_index for an IndexFlatL2, an IndexFlatIP or an IndexScalarQuantizer (QT_fp16)."""
+    if isinstance(index, IndexScalarQuantizer):
+        write_codes(path, index.codes(), index.d, index.metric_type)
+        return
     if not isinstance(index, _IndexFlat):
-        raise ValueError(f"write_index writes IndexFlatL2 and IndexFlatIP only, got {type(index).__name__}")
+        raise ValueError(f"write_index writes IndexFlatL2, IndexFlatIP and IndexScalarQuantizer only, "
+                         f"got {type(index).__name__}")
     write_rows(path, index.rows(), index.d, index.metric_type)

@@ -23,6 +23,13 @@ score), from the index's own search; --radius-values gives radii directly.  Each
 events after warm-up; a call includes its host synchronise), hits and candidates per query, overflow fallbacks, how
 many of the timed calls needed the second pass, and parity_checked: 4 queries of the batch against the fast reference
 (tests/flat_range_fast_oracle.py, bit for bit) when the rows are finite.
+
+--storage fp16: IndexScalarQuantizer(QT_fp16) beside the IndexFlat of --metric over the same rows (the IndexFlat
+holds the generated rows without a copy, so both fit at once).  Three rounds alternate the two over every (k, batch),
+one JSON line per index, round, k and batch: time per call, candidates per query, fallbacks, the index's bytes on the
+device and parity_checked (16 queries of the fp16 index bit for bit against the oracle's evaluation order over the
+fp16-decoded rows, decoded chunk by chunk; the IndexFlat as in the default mode).  --storage f32, the default, keeps the
+output above.
 """
 from __future__ import annotations
 
@@ -41,7 +48,7 @@ import torch  # noqa: E402
 
 from oracle import flat_oracle as fo  # noqa: E402
 from oracle import flat_ip_oracle as fio  # noqa: E402
-from probing_rag_b200 import IndexFlatIP, IndexFlatL2, synth  # noqa: E402
+from probing_rag_b200 import IndexFlatIP, IndexFlatL2, IndexScalarQuantizer, ScalarQuantizer, synth  # noqa: E402
 
 DATASHEET_HBM_GBS = 7700.0
 DATASHEET_BF16_TFLOPS = 2250.0
@@ -72,18 +79,20 @@ def peaks():
 
 def parity(index, Q, k, chunk=1 << 21, ip=False):
     """Bit-exact check of (D, I) against the oracle's evaluation order, the rows streamed in chunks (ip: the inner
-    products, ranked by their key, compared as keys so that a NaN equals itself)."""
+    products, ranked by their key, compared as keys so that a NaN equals itself).  An IndexScalarQuantizer is checked
+    against its decoded rows, decoded one chunk at a time."""
     D, I = index.search(Q, k)
-    X = index.rows()
+    X = index.codes() if isinstance(index, IndexScalarQuantizer) else index.rows()
     ok = True
     for b in range(Q.shape[0]):
         best_d = torch.empty(0, dtype=torch.int64 if ip else torch.float32, device=X.device)
         best_i = torch.empty(0, dtype=torch.int64, device=X.device)
         for a in range(0, X.shape[0], chunk):
+            Xc = X[a:a + chunk].float()
             if ip:
-                dist = fio.ip_key_torch(fio.exact_inner_products_torch(Q[b], X[a:a + chunk]))
+                dist = fio.ip_key_torch(fio.exact_inner_products_torch(Q[b], Xc))
             else:
-                dist = fo.exact_distances_torch(Q[b], X[a:a + chunk])
+                dist = fo.exact_distances_torch(Q[b], Xc)
             cd = torch.cat([best_d, dist])
             ci = torch.cat([best_i, torch.arange(a, a + dist.numel(), device=X.device)])
             s, o = torch.sort(cd, stable=True)      # ci ascending within equal distances: canonical order
@@ -107,6 +116,8 @@ def main():
     ap.add_argument("--out", default=None)
     ap.add_argument("--radius-ranks", default="")
     ap.add_argument("--radius-values", default="")
+    ap.add_argument("--storage", default="f32", choices=("f32", "fp16"))
+    ap.add_argument("--rounds", type=int, default=3)
     args = ap.parse_args()
     assert torch.cuda.is_available(), "bench_dense.py measures on a CUDA device"
     torch.cuda.set_device(0)
@@ -121,6 +132,8 @@ def main():
             out.write(line + "\n")
             out.flush()
 
+    if args.storage == "fp16":
+        return bench_fp16(args, emit, name, power)
     t0 = time.perf_counter()
     ip = args.metric == "ip"
     index = (IndexFlatIP if ip else IndexFlatL2)(args.d)
@@ -179,6 +192,59 @@ def main():
         emit({"metric": f"dense_flat_{args.metric}_cpu_baseline", "impl": "numpy restatement of faiss BLAS flat search",
               "n": Xc.shape[0], "d": d, "k": 10, "batch": B, "ms_per_call": round(s * 1e3, 2),
               "host_threads": torch.get_num_threads(), "note": "slice of the index; not extrapolated to the full size"})
+
+
+def time_search(index, Q, k, warmup, iters):
+    for _ in range(warmup):
+        index.search(Q, k)
+    torch.cuda.synchronize()
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    e0.record()
+    for _ in range(iters):
+        index.search(Q, k)
+    e1.record()
+    torch.cuda.synchronize()
+    return e0.elapsed_time(e1) / iters
+
+
+def bench_fp16(args, emit, name, power):
+    ip = args.metric == "ip"
+    t0 = time.perf_counter()
+    rows = synth.dense_rows(args.n, args.d, kind=args.kind)
+    sq = IndexScalarQuantizer(args.d, ScalarQuantizer.QT_fp16, 0 if ip else 1)
+    sq.add(rows)
+    flat = (IndexFlatIP if ip else IndexFlatL2)(args.d)
+    flat._set_rows(rows)                                        # the generated rows themselves, no second copy
+    del rows
+    Q1 = synth.dense_queries(flat.rows(), 1)
+    for index in (flat, sq):
+        index.search(Q1, 1)                                     # builds the aux (bf16 copy and norms / norms only)
+    torch.cuda.synchronize()
+    build_s = time.perf_counter() - t0
+    Qp = synth.dense_queries(flat.rows(), 16, seed=99)
+    checked = {"f32": parity(flat, Qp, 10, ip=ip), "fp16": parity(sq, Qp, 10, ip=ip)}
+    dev_bytes = {"f32": flat.rows().numel() * 4 + flat._aux.numel(), "fp16": sq.codes().numel() * 2 + sq._aux.numel()}
+    for rnd in range(args.rounds):
+        for k in [int(s) for s in args.ks.split(",")]:
+            for B in [int(s) for s in args.batches.split(",")]:
+                Q = synth.dense_queries(flat.rows(), B)
+                for storage, index in (("f32", flat), ("fp16", sq)):
+                    ms = time_search(index, Q, k, args.warmup, args.iters)
+                    st = index.last_stats()
+                    emit({
+                        "metric": f"dense_{'sq_fp16' if storage == 'fp16' else 'flat'}_{args.metric}_search",
+                        "storage": storage, "round": rnd, "n": args.n, "d": args.d, "k": k, "batch": B,
+                        "data": args.kind, "ms_per_call": round(ms, 4), "queries_per_s": round(B / (ms * 1e-3), 1),
+                        "candidates_mean_per_query": round(st["candidates"] / B, 1),
+                        "candidates_max_query_chunk": st["max_candidates"],
+                        "fallback_query_chunks": st["fallback_queries"], "chunks": st["chunks"],
+                        "index_device_bytes": dev_bytes[storage], "parity_checked": checked[storage],
+                        "parity_queries": 16, "parity_reference": "oracle evaluation order over the "
+                        + ("fp16-decoded rows" if storage == "fp16" else "f32 rows"),
+                        "index_build_s": round(build_s, 1), "gpu": name, "power_limit": power,
+                        "timing": f"CUDA events, {args.warmup} warm-up + {args.iters} calls; f32 and fp16 alternate "
+                                  f"per (k, batch) in each of {args.rounds} rounds",
+                    })
 
 
 def bench_range(args, index, emit, name, power, build_s):
