@@ -30,8 +30,13 @@
 //   fp16     pr_flat_create_fp16: rows stored as IEEE binary16 codes; the same host plan launches the fp16 kernels of
 //            flat_fp16.cu (the same GEMM and refines on the codes themselves, no bf16 copy)
 //
-// The rows are cut into chunks of growing size; filter and refine alternate per chunk on the caller's stream, so
-// every chunk filters with the bound the earlier ones established ("bounds raised between launches", as BM25 does).
+// One host plan (flat_plan) serves both searches and both storage types: init (theta[q] = +-inf for top-k search, the
+// radius for range search), query prep, the two tensor maps and the filter's arguments, then the rows cut into chunks
+// of growing size, filter and refine alternating per chunk on the caller's stream, so that every chunk filters with
+// the bound the earlier ones established ("bounds raised between launches", as BM25 does).  The caller chooses the
+// refine: the top-k refine, then the output kernel (pr_flat_search), or the range refine (pr_flat_range_search).  Each
+// stage's kernel is picked by the storage type at one call site and by the metric in the launcher of its translation
+// unit.
 #include <algorithm>
 #include <cfloat>
 #include <cmath>
@@ -52,7 +57,8 @@ struct pr_flat {
     const __nv_bfloat16 *rows_bf;   // aux: bf16 copy [n][d]
     const float *norm2, *norm;      // aux: ||x||^2, ||x|| (f32)
     int metric;                     // PR_METRIC_L2 or PR_METRIC_INNER_PRODUCT
-    int32_t fp16;                   // pr_flat_create_fp16 (in what was padding: the offsets of f32 handles are kept)
+    int32_t fp16;                   // pr_flat_create_fp16; in the padding before `tun`, so that the fields up to
+                                    // last_chunks keep the offsets tests/test_flat_range_oracle.py mirrors (_FakeFlat)
     pr_flat_tuning_t tun;
     int64_t last_launches, last_chunks;
     const __half *codes;            // fp16 only (read only when fp16 != 0): the rows [n][d] and the aux ||x_sub||
@@ -250,6 +256,24 @@ FlatLayout flat_layout(int d, int n_queries, int k, int cap, bool fp16)
     return l;
 }
 
+// The workspace of one call, carved by its layout.  q_ops: the queries' bf16 copy, or their scaled fp16 copy.
+struct FlatWs {
+    void *q_ops;
+    float *qn2, *qn, *theta;
+    int32_t *count, *cand;
+    uint64_t *topk;
+    unsigned long long *stats;
+    float *qscale;                  // fp16 storage only
+};
+
+FlatWs flat_ws(const FlatLayout &l, void *base)
+{
+    unsigned char *ws = (unsigned char *)base;
+    return {ws + l.q_bf, (float *)(ws + l.qn2), (float *)(ws + l.qn), (float *)(ws + l.theta),
+            (int32_t *)(ws + l.count), (int32_t *)(ws + l.cand), (uint64_t *)(ws + l.topk),
+            (unsigned long long *)(ws + l.stats), (float *)(ws + l.qscale)};
+}
+
 size_t aux_norm2_offset(const pr_flat *h) { return h->fp16 ? 0 : up((size_t)h->n * h->d * 2, 256); }
 size_t aux_norm_offset(const pr_flat *h) { return up(aux_norm2_offset(h) + (size_t)h->n * 4, 256); }
 size_t aux_nsub_offset(const pr_flat *h) { return up(aux_norm_offset(h) + (size_t)h->n * 4, 256); }
@@ -315,13 +339,12 @@ float margin_csub_f16(int metric)
     return std::nextafter((float)c, INFINITY);
 }
 
-}  // namespace
-
-extern "C" int pr_flat_create_metric(pr_flat_t **out, int device, const float *rows_dev, int64_t n, int32_t d,
-                                     int metric)
+// The checks and the construction of every pr_flat_create*: fn is the name the messages start with, arg the name of
+// the rows argument; fp16 handles hold `rows` as codes.
+int flat_create(pr_flat_t **out, const char *fn, const char *arg, int device, const void *rows, int64_t n, int32_t d,
+                int metric, bool fp16)
 {
-    const char *fn = metric == PR_METRIC_L2 ? "pr_flat_create" : "pr_flat_create_metric";
-    if (!out || (n > 0 && !rows_dev) || n < 0) {
+    if (!out || (n > 0 && !rows) || n < 0) {
         pr_set_error("%s: bad argument (null pointer or negative row count)", fn);
         return PR_EINVAL;
     }
@@ -338,8 +361,8 @@ extern "C" int pr_flat_create_metric(pr_flat_t **out, int device, const float *r
         pr_set_error("%s: %lld rows, at most 2^31 - 1 per index", fn, (long long)n);
         return PR_EUNSUPPORTED;
     }
-    if ((uintptr_t)rows_dev & 15) {
-        pr_set_error("%s: rows_dev must be 16-byte aligned", fn);
+    if ((uintptr_t)rows & 15) {
+        pr_set_error("%s: %s must be 16-byte aligned", fn, arg);
         return PR_EINVAL;
     }
     PR_CUDA_CHECK(cudaSetDevice(device));
@@ -350,55 +373,140 @@ extern "C" int pr_flat_create_metric(pr_flat_t **out, int device, const float *r
     h->n_sm = n_sm;
     h->n = n;
     h->d = d;
-    h->rows = rows_dev;
     h->metric = metric;
+    h->fp16 = fp16;
+    if (fp16)
+        h->codes = (const __half *)rows;
+    else
+        h->rows = (const float *)rows;
     *out = h;
     return PR_OK;
 }
 
+// The launches of flat.cu's f32 kernels, in the argument order of flat_fp16.cu's: the metric picks the kernel.  A function
+// attribute holds for the current device only: it is set on every launch (host-only and cheap), so that an index on a
+// second GPU of the process launches as the first one did.
+int flat_filter_launch(int metric, unsigned grid, size_t smem, const CUtensorMap &map_x, const CUtensorMap &map_q,
+                       const FilterArgs &fa, cudaStream_t st)
+{
+    const bool ip = metric == PR_METRIC_INNER_PRODUCT;
+    const void *filter = ip ? (const void *)flat_ip_filter_kernel : (const void *)flat_filter_kernel;
+    PR_CUDA_CHECK(cudaFuncSetAttribute(filter, cudaFuncAttributeMaxDynamicSharedMemorySize, kFilterSmemMax));
+    if (ip)
+        flat_ip_filter_kernel<<<grid, kFilterThreads, smem, st>>>(map_x, map_q, fa);
+    else
+        flat_filter_kernel<<<grid, kFilterThreads, smem, st>>>(map_x, map_q, fa);
+    PR_CUDA_CHECK(cudaGetLastError());
+    return PR_OK;
+}
+
+int flat_refine_launch(int metric, int n_queries, const RefineArgs &ra, cudaStream_t st)
+{
+    if (metric == PR_METRIC_INNER_PRODUCT)
+        flat_ip_refine_kernel<<<n_queries, kRefineThreads, 0, st>>>(ra);
+    else
+        flat_refine_kernel<<<n_queries, kRefineThreads, 0, st>>>(ra);
+    PR_CUDA_CHECK(cudaGetLastError());
+    return PR_OK;
+}
+
+// The launch plan of both searches (stated at the top of this file) on the workspace `w` of layout `l`: theta0 is
+// every query's starting bound, cap the candidates per (query, chunk) the filter stores, and refine(begin, end)
+// launches the caller's refine of the chunk [begin, end) (PR_OK or an error code).  Records the launches and chunks
+// in the handle.
+template <typename Refine>
+int flat_plan(pr_flat *h, int n_queries, const float *queries, int k, const FlatLayout &l, const FlatWs &w,
+              float theta0, int cap, cudaStream_t st, Refine refine)
+{
+    flat_init_kernel<<<(unsigned)(((int64_t)n_queries * k + 255) / 256), 256, 0, st>>>(n_queries, k, theta0, w.theta,
+                                                                                     w.count, w.topk, w.stats);
+    PR_CUDA_CHECK(cudaGetLastError());
+    int64_t launches = 1;
+    if (h->n == 0) {
+        h->last_launches = launches;
+        return PR_OK;
+    }
+    int rc;
+    if (h->fp16) {
+        if ((rc = flat_fp16_prep_queries(queries, n_queries, l.b_pad, h->d, (__half *)w.q_ops, w.qn2, w.qn,
+                                         w.qscale, st)) != PR_OK)
+            return rc;
+    } else {
+        flat_prep_kernel<<<(unsigned)((l.b_pad + 7) / 8), 256, 0, st>>>(queries, n_queries, l.b_pad, h->d,
+                                                                        (__nv_bfloat16 *)w.q_ops, w.qn2, w.qn);
+        PR_CUDA_CHECK(cudaGetLastError());
+    }
+    ++launches;
+    CUtensorMap map_x, map_q;
+    const CUtensorMapDataType dtype = h->fp16 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
+    const void *x_ops = h->fp16 ? (const void *)h->codes : (const void *)h->rows_bf;
+    if ((rc = make_map(&map_x, x_ops, (uint64_t)h->n, (uint64_t)h->d, kRowsPerTile, dtype)) != PR_OK) return rc;
+    if ((rc = make_map(&map_q, w.q_ops, (uint64_t)l.b_pad, (uint64_t)h->d, (uint32_t)l.nq, dtype)) != PR_OK) return rc;
+    const bool ip = h->metric == PR_METRIC_INNER_PRODUCT;
+    const int stage_bytes = kDocTileBytes + l.nq * kBK * 2;
+    FilterArgs fa;
+    fa.n_queries = n_queries;
+    fa.nq = l.nq;
+    fa.n_qb = l.n_qb;
+    fa.K = h->d;
+    fa.n_stages = std::min(kMaxStages, kStageBudget / stage_bytes);
+    // D f32; A and B BF16 (format 1) or, for fp16 storage, F16 (format 0); N = nq; M = 128
+    fa.idesc = (1u << 4) | (h->fp16 ? 0u : (1u << 7) | (1u << 10)) | ((uint32_t)(l.nq >> 3) << 17) |
+               ((uint32_t)(kRowsPerTile >> 4) << 24);
+    fa.tmem_cols = 32;
+    while (fa.tmem_cols < (uint32_t)(2 * l.nq)) fa.tmem_cols <<= 1;
+    fa.c1 = h->fp16 ? (ip ? margin_c1ip_f16(h->d) : margin_c1_f16(h->d)) : (ip ? margin_c1ip(h->d) : margin_c1(h->d));
+    fa.c2 = ip ? 0.f : std::ldexp(1.f, -17);
+    fa.c3 = std::ldexp(1.f, -100);
+    fa.norm2 = h->norm2;
+    fa.norm = h->norm;
+    fa.qn2 = w.qn2;
+    fa.qn = w.qn;
+    fa.theta = w.theta;
+    fa.count = w.count;
+    fa.cand = w.cand;
+    fa.cap = cap;
+    const FilterF16Args fh = {w.qscale, h->nsub, margin_csub_f16(h->metric)};   // (read by the fp16 filters only)
+    const size_t smem = kFilterSmemFixed + (size_t)fa.n_stages * stage_bytes;
+    const pr_flat_tuning_t tun = effective_tuning(h);
+    int64_t chunk = (tun.first_chunk_rows + kRowsPerTile - 1) / kRowsPerTile * kRowsPerTile;
+    for (int64_t begin = 0; begin < h->n;) {
+        const int64_t end = std::min(h->n, begin + chunk);
+        fa.row_begin = begin;
+        fa.row_end = end;
+        const int64_t tiles = (end - begin + kRowsPerTile - 1) / kRowsPerTile * l.n_qb;
+        const unsigned grid = (unsigned)std::min<int64_t>(tiles, h->n_sm);
+        rc = h->fp16 ? flat_fp16_filter_launch(h->metric, grid, smem, map_x, map_q, fa, fh, st)
+                     : flat_filter_launch(h->metric, grid, smem, map_x, map_q, fa, st);
+        if (rc != PR_OK) return rc;
+        if ((rc = refine(begin, end)) != PR_OK) return rc;
+        launches += 2;
+        ++h->last_chunks;
+        begin = end;
+        chunk = std::min<int64_t>(chunk * tun.growth, (int64_t)1 << 40);
+    }
+    h->last_launches = launches;
+    return PR_OK;
+}
+
+}  // namespace
+
+extern "C" int pr_flat_create_metric(pr_flat_t **out, int device, const float *rows_dev, int64_t n, int32_t d,
+                                     int metric)
+{
+    return flat_create(out, metric == PR_METRIC_L2 ? "pr_flat_create" : "pr_flat_create_metric", "rows_dev", device,
+                       rows_dev, n, d, metric, false);
+}
+
 extern "C" int pr_flat_create(pr_flat_t **out, int device, const float *rows_dev, int64_t n, int32_t d)
 {
-    return pr_flat_create_metric(out, device, rows_dev, n, d, PR_METRIC_L2);
+    return flat_create(out, "pr_flat_create", "rows_dev", device, rows_dev, n, d, PR_METRIC_L2, false);
 }
 
 extern "C" int pr_flat_create_fp16(pr_flat_t **out, int device, const uint16_t *codes_dev, int64_t n, int32_t d,
                                    int metric)
 {
-    if (!out || (n > 0 && !codes_dev) || n < 0) {
-        pr_set_error("pr_flat_create_fp16: bad argument (null pointer or negative row count)");
-        return PR_EINVAL;
-    }
-    *out = nullptr;
-    if (metric != PR_METRIC_L2 && metric != PR_METRIC_INNER_PRODUCT) {
-        pr_set_error("pr_flat_create_fp16: metric %d unsupported (PR_METRIC_INNER_PRODUCT = 0 or PR_METRIC_L2 = 1)",
-                     metric);
-        return PR_EUNSUPPORTED;
-    }
-    if (d < 64 || d > PR_FLAT_MAX_D || d % 64 != 0) {
-        pr_set_error("pr_flat_create_fp16: d = %d unsupported (a multiple of 64 in [64, %d])", d, PR_FLAT_MAX_D);
-        return PR_EUNSUPPORTED;
-    }
-    if (n > INT32_MAX) {
-        pr_set_error("pr_flat_create_fp16: %lld rows, at most 2^31 - 1 per index", (long long)n);
-        return PR_EUNSUPPORTED;
-    }
-    if ((uintptr_t)codes_dev & 15) {
-        pr_set_error("pr_flat_create_fp16: codes_dev must be 16-byte aligned");
-        return PR_EINVAL;
-    }
-    PR_CUDA_CHECK(cudaSetDevice(device));
-    int n_sm = 0;
-    PR_CUDA_CHECK(cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, device));
-    pr_flat *h = new pr_flat();
-    h->device = device;
-    h->n_sm = n_sm;
-    h->n = n;
-    h->d = d;
-    h->metric = metric;
-    h->fp16 = 1;
-    h->codes = (const __half *)codes_dev;
-    *out = h;
-    return PR_OK;
+    return flat_create(out, "pr_flat_create_fp16", "codes_dev", device, codes_dev, n, d, metric, true);
 }
 
 extern "C" int pr_flat_destroy(pr_flat_t *h)
@@ -440,13 +548,12 @@ extern "C" int pr_flat_build_aux(pr_flat_t *h, void *aux_dev, size_t aux_bytes, 
         if ((rc = flat_fp16_prep_rows(h->codes, h->n, h->d, (float *)h->norm2, (float *)h->norm, (float *)h->nsub,
                                       st)) != PR_OK)
             return rc;
-        PR_CUDA_CHECK(cudaStreamSynchronize(st));
-        return PR_OK;
+    } else {
+        flat_prep_kernel<<<(unsigned)((h->n + 7) / 8), 256, 0, st>>>(h->rows, h->n, h->n, h->d,
+                                                                     (__nv_bfloat16 *)h->rows_bf, (float *)h->norm2,
+                                                                     (float *)h->norm);
+        PR_CUDA_CHECK(cudaGetLastError());
     }
-    const int64_t blocks = (h->n + 7) / 8;
-    flat_prep_kernel<<<(unsigned)blocks, 256, 0, st>>>(h->rows, h->n, h->n, h->d, (__nv_bfloat16 *)h->rows_bf,
-                                                       (float *)h->norm2, (float *)h->norm);
-    PR_CUDA_CHECK(cudaGetLastError());
     PR_CUDA_CHECK(cudaStreamSynchronize(st));
     return PR_OK;
 }
@@ -499,115 +606,40 @@ extern "C" int pr_flat_search(pr_flat_t *h, int32_t n_queries, const float *quer
     h->last_launches = 0;
     h->last_chunks = 0;
     if (n_queries == 0) return PR_OK;
-    const pr_flat_tuning_t tun = effective_tuning(h);
-    const FlatLayout l = flat_layout(h->d, n_queries, k, tun.cand_capacity, h->fp16);
+    const int cap = effective_tuning(h).cand_capacity;
+    const FlatLayout l = flat_layout(h->d, n_queries, k, cap, h->fp16);
     if (workspace_bytes < l.total) {
         pr_set_error("pr_flat_search: workspace of %zu bytes, need %zu", workspace_bytes, l.total);
         return PR_EWORKSPACE;
     }
     PR_CUDA_CHECK(cudaSetDevice(h->device));
     cudaStream_t st = (cudaStream_t)stream;
-    unsigned char *ws = (unsigned char *)workspace_dev;
-    __nv_bfloat16 *q_bf = (__nv_bfloat16 *)(ws + l.q_bf);
-    float *qn2 = (float *)(ws + l.qn2), *qn = (float *)(ws + l.qn), *theta = (float *)(ws + l.theta);
-    int32_t *count = (int32_t *)(ws + l.count), *cand = (int32_t *)(ws + l.cand);
-    uint64_t *topk = (uint64_t *)(ws + l.topk);
-    unsigned long long *stats = (unsigned long long *)(ws + l.stats);
+    const FlatWs w = flat_ws(l, workspace_dev);
+    RefineArgs ra;
+    ra.rows = h->rows;
+    ra.rows_h = h->codes;
+    ra.queries = queries_dev;
+    ra.d = h->d;
+    ra.k = k;
+    ra.cap = cap;
+    ra.count = w.count;
+    ra.cand = w.cand;
+    ra.topk = w.topk;
+    ra.theta = w.theta;
+    ra.stats = w.stats;
+    const float theta0 = h->metric == PR_METRIC_INNER_PRODUCT ? -INFINITY : INFINITY;
+    const int rc = flat_plan(h, n_queries, queries_dev, k, l, w, theta0, cap, st, [&](int64_t begin, int64_t end) {
+        ra.row_begin = begin;
+        ra.row_end = end;
+        return h->fp16 ? flat_fp16_refine_launch(h->metric, n_queries, ra, st)
+                       : flat_refine_launch(h->metric, n_queries, ra, st);
+    });
+    if (rc != PR_OK) return rc;
     const int64_t total = (int64_t)n_queries * k;
-
-    const bool ip = h->metric == PR_METRIC_INNER_PRODUCT;
-    flat_init_kernel<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(n_queries, k, ip ? -INFINITY : INFINITY, theta,
-                                                                     count, topk, stats);
-    int64_t launches = 1;
-    if (h->n > 0) {
-        float *qscale = (float *)(ws + l.qscale);
-        int rc;
-        if (h->fp16) {
-            if ((rc = flat_fp16_prep_queries(queries_dev, n_queries, l.b_pad, h->d, (__half *)q_bf, qn2, qn, qscale,
-                                             st)) != PR_OK)
-                return rc;
-        } else {
-            flat_prep_kernel<<<(unsigned)((l.b_pad + 7) / 8), 256, 0, st>>>(queries_dev, n_queries, l.b_pad, h->d, q_bf, qn2, qn);
-        }
-        ++launches;
-        CUtensorMap map_x, map_q;
-        const CUtensorMapDataType dtype = h->fp16 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
-        const void *x_ops = h->fp16 ? (const void *)h->codes : (const void *)h->rows_bf;
-        if ((rc = make_map(&map_x, x_ops, (uint64_t)h->n, (uint64_t)h->d, kRowsPerTile, dtype)) != PR_OK) return rc;
-        if ((rc = make_map(&map_q, q_bf, (uint64_t)l.b_pad, (uint64_t)h->d, (uint32_t)l.nq, dtype)) != PR_OK) return rc;
-        const int stage_bytes = kDocTileBytes + l.nq * kBK * 2;
-        FilterArgs fa;
-        fa.n_queries = n_queries;
-        fa.nq = l.nq;
-        fa.n_qb = l.n_qb;
-        fa.K = h->d;
-        fa.n_stages = std::min(kMaxStages, kStageBudget / stage_bytes);
-        // D f32; A and B BF16 (format 1) or, for fp16 storage, F16 (format 0); N = nq; M = 128
-        fa.idesc = (1u << 4) | (h->fp16 ? 0u : (1u << 7) | (1u << 10)) | ((uint32_t)(l.nq >> 3) << 17) |
-                   ((uint32_t)(kRowsPerTile >> 4) << 24);
-        fa.tmem_cols = 32;
-        while (fa.tmem_cols < (uint32_t)(2 * l.nq)) fa.tmem_cols <<= 1;
-        if (h->fp16)
-            fa.c1 = ip ? margin_c1ip_f16(h->d) : margin_c1_f16(h->d);
-        else
-            fa.c1 = ip ? margin_c1ip(h->d) : margin_c1(h->d);
-        fa.c2 = ip ? 0.f : std::ldexp(1.f, -17);
-        fa.c3 = std::ldexp(1.f, -100);
-        const FilterF16Args fh = {qscale, h->fp16 ? h->nsub : nullptr, h->fp16 ? margin_csub_f16(h->metric) : 0.f};
-        fa.norm2 = h->norm2;
-        fa.norm = h->norm;
-        fa.qn2 = qn2;
-        fa.qn = qn;
-        fa.theta = theta;
-        fa.count = count;
-        fa.cand = cand;
-        fa.cap = tun.cand_capacity;
-        const size_t smem = 1024 + (size_t)fa.n_stages * stage_bytes + (2 * kMaxStages + 4) * 8 + 16;
-        const void *filter = ip ? (const void *)flat_ip_filter_kernel : (const void *)flat_filter_kernel;
-        // A function attribute holds for the current device only: set it on every call (host-only and cheap), so that
-        // an index on a second GPU of the process launches as the first one did.
-        PR_CUDA_CHECK(cudaFuncSetAttribute(filter, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                           1024 + kStageBudget + (2 * kMaxStages + 4) * 8 + 16));
-        RefineArgs ra;
-        ra.rows = h->rows;
-        ra.rows_h = h->fp16 ? h->codes : nullptr;
-        ra.queries = queries_dev;
-        ra.d = h->d;
-        ra.k = k;
-        ra.cap = tun.cand_capacity;
-        ra.count = count;
-        ra.cand = cand;
-        ra.topk = topk;
-        ra.theta = theta;
-        ra.stats = stats;
-        int64_t chunk = (tun.first_chunk_rows + kRowsPerTile - 1) / kRowsPerTile * kRowsPerTile;
-        for (int64_t begin = 0; begin < h->n;) {
-            const int64_t end = std::min(h->n, begin + chunk);
-            fa.row_begin = ra.row_begin = begin;
-            fa.row_end = ra.row_end = end;
-            const int64_t tiles = (end - begin + kRowsPerTile - 1) / kRowsPerTile * l.n_qb;
-            const unsigned grid = (unsigned)std::min<int64_t>(tiles, h->n_sm);
-            if (h->fp16) {
-                if ((rc = flat_fp16_filter_launch(h->metric, grid, smem, map_x, map_q, fa, fh, st)) != PR_OK) return rc;
-                if ((rc = flat_fp16_refine_launch(h->metric, n_queries, ra, st)) != PR_OK) return rc;
-            } else if (ip) {
-                flat_ip_filter_kernel<<<grid, kFilterThreads, smem, st>>>(map_x, map_q, fa);
-                flat_ip_refine_kernel<<<n_queries, kRefineThreads, 0, st>>>(ra);
-            } else {
-                flat_filter_kernel<<<grid, kFilterThreads, smem, st>>>(map_x, map_q, fa);
-                flat_refine_kernel<<<n_queries, kRefineThreads, 0, st>>>(ra);
-            }
-            PR_CUDA_CHECK(cudaGetLastError());
-            launches += 2;
-            ++h->last_chunks;
-            begin = end;
-            chunk = std::min<int64_t>(chunk * tun.growth, (int64_t)1 << 40);
-        }
-    }
-    flat_output_kernel<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(total, topk, out_dist_dev, out_ids_dev,
+    flat_output_kernel<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(total, w.topk, out_dist_dev, out_ids_dev,
                                                                        h->metric);
     PR_CUDA_CHECK(cudaGetLastError());
-    h->last_launches = launches + 1;
+    ++h->last_launches;
     return PR_OK;
 }
 
@@ -621,8 +653,8 @@ extern "C" int pr_flat_last_stats(const pr_flat_t *h, const void *workspace_dev,
     const FlatLayout l = flat_layout(h->d, n_queries, k, effective_tuning(h).cand_capacity, h->fp16);
     unsigned long long s[4];
     PR_CUDA_CHECK(cudaSetDevice(h->device));
-    PR_CUDA_CHECK(cudaMemcpyAsync(s, (const unsigned char *)workspace_dev + l.stats, sizeof(s), cudaMemcpyDeviceToHost,
-                                  (cudaStream_t)stream));
+    PR_CUDA_CHECK(cudaMemcpyAsync(s, flat_ws(l, const_cast<void *>(workspace_dev)).stats, sizeof(s),
+                                  cudaMemcpyDeviceToHost, (cudaStream_t)stream));
     PR_CUDA_CHECK(cudaStreamSynchronize((cudaStream_t)stream));
     out->launches = h->last_launches;
     out->chunks = h->last_chunks;
@@ -669,110 +701,32 @@ extern "C" int pr_flat_range_search(pr_flat_t *h, int32_t n_queries, const float
     }
     PR_CUDA_CHECK(cudaSetDevice(h->device));
     cudaStream_t st = (cudaStream_t)stream;
-    unsigned char *ws = (unsigned char *)workspace_dev;
+    const FlatWs w = flat_ws(l, workspace_dev);
     PR_CUDA_CHECK(cudaMemsetAsync(count_dev, 0, (size_t)n_queries * sizeof(int64_t), st));
     if (std::isnan(radius)) {                  // no results; the counters read zero
-        PR_CUDA_CHECK(cudaMemsetAsync(ws + l.stats, 0, 4 * 8, st));
+        PR_CUDA_CHECK(cudaMemsetAsync(w.stats, 0, 4 * 8, st));
         return PR_OK;
     }
-    __nv_bfloat16 *q_bf = (__nv_bfloat16 *)(ws + l.q_bf);
-    float *qn2 = (float *)(ws + l.qn2), *qn = (float *)(ws + l.qn), *theta = (float *)(ws + l.theta);
-    int32_t *count = (int32_t *)(ws + l.count), *cand = (int32_t *)(ws + l.cand);
-    unsigned long long *stats = (unsigned long long *)(ws + l.stats);
-
-    const bool ip = h->metric == PR_METRIC_INNER_PRODUCT;
-    flat_init_kernel<<<(unsigned)((n_queries + 255) / 256), 256, 0, st>>>(n_queries, 1, radius, theta, count,
-                                                                         (uint64_t *)(ws + l.topk), stats);
-    PR_CUDA_CHECK(cudaGetLastError());
-    int64_t launches = 1;
-    if (h->n > 0) {
-        float *qscale = (float *)(ws + l.qscale);
-        int rc;
-        if (h->fp16) {
-            if ((rc = flat_fp16_prep_queries(queries_dev, n_queries, l.b_pad, h->d, (__half *)q_bf, qn2, qn, qscale,
-                                             st)) != PR_OK)
-                return rc;
-        } else {
-            flat_prep_kernel<<<(unsigned)((l.b_pad + 7) / 8), 256, 0, st>>>(queries_dev, n_queries, l.b_pad, h->d, q_bf, qn2, qn);
-        }
-        ++launches;
-        CUtensorMap map_x, map_q;
-        const CUtensorMapDataType dtype = h->fp16 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
-        const void *x_ops = h->fp16 ? (const void *)h->codes : (const void *)h->rows_bf;
-        if ((rc = make_map(&map_x, x_ops, (uint64_t)h->n, (uint64_t)h->d, kRowsPerTile, dtype)) != PR_OK) return rc;
-        if ((rc = make_map(&map_q, q_bf, (uint64_t)l.b_pad, (uint64_t)h->d, (uint32_t)l.nq, dtype)) != PR_OK) return rc;
-        const int cap = std::min<int>(tun.cand_capacity, kFlatRangeMaxCap);
-        const int stage_bytes = kDocTileBytes + l.nq * kBK * 2;
-        FilterArgs fa;
-        fa.n_queries = n_queries;
-        fa.nq = l.nq;
-        fa.n_qb = l.n_qb;
-        fa.K = h->d;
-        fa.n_stages = std::min(kMaxStages, kStageBudget / stage_bytes);
-        // D f32; A and B BF16 (format 1) or, for fp16 storage, F16 (format 0); N = nq; M = 128
-        fa.idesc = (1u << 4) | (h->fp16 ? 0u : (1u << 7) | (1u << 10)) | ((uint32_t)(l.nq >> 3) << 17) |
-                   ((uint32_t)(kRowsPerTile >> 4) << 24);
-        fa.tmem_cols = 32;
-        while (fa.tmem_cols < (uint32_t)(2 * l.nq)) fa.tmem_cols <<= 1;
-        if (h->fp16)
-            fa.c1 = ip ? margin_c1ip_f16(h->d) : margin_c1_f16(h->d);
-        else
-            fa.c1 = ip ? margin_c1ip(h->d) : margin_c1(h->d);
-        fa.c2 = ip ? 0.f : std::ldexp(1.f, -17);
-        fa.c3 = std::ldexp(1.f, -100);
-        const FilterF16Args fh = {qscale, h->fp16 ? h->nsub : nullptr, h->fp16 ? margin_csub_f16(h->metric) : 0.f};
-        fa.norm2 = h->norm2;
-        fa.norm = h->norm;
-        fa.qn2 = qn2;
-        fa.qn = qn;
-        fa.theta = theta;
-        fa.count = count;
-        fa.cand = cand;
-        fa.cap = cap;
-        const size_t smem = 1024 + (size_t)fa.n_stages * stage_bytes + (2 * kMaxStages + 4) * 8 + 16;
-        const void *filter = ip ? (const void *)flat_ip_filter_kernel : (const void *)flat_filter_kernel;
-        PR_CUDA_CHECK(cudaFuncSetAttribute(filter, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                           1024 + kStageBudget + (2 * kMaxStages + 4) * 8 + 16));
-        FlatRangeArgs ra;
-        ra.rows = h->rows;
-        ra.rows_h = h->fp16 ? h->codes : nullptr;
-        ra.queries = queries_dev;
-        ra.d = h->d;
-        ra.cap = cap;
-        ra.radius = radius;
-        ra.count = count;
-        ra.cand = cand;
-        ra.lims = lims_in_dev;
-        ra.hits = count_dev;
-        ra.dist = dist_dev;
-        ra.ids = ids_dev;
-        ra.stats = stats;
-        int64_t chunk = (tun.first_chunk_rows + kRowsPerTile - 1) / kRowsPerTile * kRowsPerTile;
-        for (int64_t begin = 0; begin < h->n;) {
-            const int64_t end = std::min(h->n, begin + chunk);
-            fa.row_begin = ra.row_begin = begin;
-            fa.row_end = ra.row_end = end;
-            const int64_t tiles = (end - begin + kRowsPerTile - 1) / kRowsPerTile * l.n_qb;
-            const unsigned grid = (unsigned)std::min<int64_t>(tiles, h->n_sm);
-            if (h->fp16) {
-                if ((rc = flat_fp16_filter_launch(h->metric, grid, smem, map_x, map_q, fa, fh, st)) != PR_OK) return rc;
-                if ((rc = flat_fp16_range_refine_launch(h->metric, n_queries, ra, st)) != PR_OK) return rc;
-            } else {
-                if (ip)
-                    flat_ip_filter_kernel<<<grid, kFilterThreads, smem, st>>>(map_x, map_q, fa);
-                else
-                    flat_filter_kernel<<<grid, kFilterThreads, smem, st>>>(map_x, map_q, fa);
-                PR_CUDA_CHECK(cudaGetLastError());
-                if ((rc = flat_range_refine_launch(ra, h->metric, n_queries, st)) != PR_OK) return rc;
-            }
-            launches += 2;
-            ++h->last_chunks;
-            begin = end;
-            chunk = std::min<int64_t>(chunk * tun.growth, (int64_t)1 << 40);
-        }
-    }
-    h->last_launches = launches;
-    return PR_OK;
+    FlatRangeArgs ra;
+    ra.rows = h->rows;
+    ra.rows_h = h->codes;
+    ra.queries = queries_dev;
+    ra.d = h->d;
+    ra.cap = std::min<int>(tun.cand_capacity, kFlatRangeMaxCap);
+    ra.radius = radius;
+    ra.count = w.count;
+    ra.cand = w.cand;
+    ra.lims = lims_in_dev;
+    ra.hits = count_dev;
+    ra.dist = dist_dev;
+    ra.ids = ids_dev;
+    ra.stats = w.stats;
+    return flat_plan(h, n_queries, queries_dev, 1, l, w, radius, ra.cap, st, [&](int64_t begin, int64_t end) {
+        ra.row_begin = begin;
+        ra.row_end = end;
+        return h->fp16 ? flat_fp16_range_refine_launch(h->metric, n_queries, ra, st)
+                       : flat_range_refine_launch(h->metric, n_queries, ra, st);
+    });
 }
 
 extern "C" int pr_flat_merge_metric(int32_t n_queries, int32_t k, int32_t n_lists, const float *dist_dev,

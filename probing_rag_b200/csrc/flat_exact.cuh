@@ -100,7 +100,7 @@ struct FlatRangeArgs {
 };
 
 // Enqueues the range refine of one chunk for n_queries queries on `stream`; PR_OK or PR_ECUDA.
-int flat_range_refine_launch(const FlatRangeArgs &g, int metric, int n_queries, cudaStream_t stream);
+int flat_range_refine_launch(int metric, int n_queries, const FlatRangeArgs &g, cudaStream_t stream);
 
 namespace {
 

@@ -17,6 +17,8 @@ constexpr int kMaxNQ = 256;
 constexpr int kMaxStages = 8;
 constexpr int kDocTileBytes = kRowsPerTile * kBK * 2;   // 16 KB
 constexpr int kStageBudget = 192 * 1024;
+constexpr int kFilterSmemFixed = 1024 + (2 * kMaxStages + 4) * 8 + 16;   // alignment slack, barriers, TMEM slot
+constexpr int kFilterSmemMax = kFilterSmemFixed + kStageBudget;          // the filters' dynamic shared memory limit
 constexpr int kFilterThreads = 256;
 constexpr int kRefineThreads = 256;
 constexpr int kRefineKeys = 2048;                       // running list + new exact candidates of one round
@@ -310,7 +312,8 @@ __device__ __forceinline__ void flat_refine(const RefineArgs &g)
 }  // namespace
 
 // ------------------------------------------------------------------------------------ fp16 storage (flat_fp16.cu)
-// The launches of the fp16-row kernels, for the host code of flat.cu; each returns PR_OK or PR_ECUDA.
+// The launches of the fp16-row kernels, for the host code of flat.cu; each returns PR_OK or PR_ECUDA.  The launchers
+// take (metric, grid, ..., arguments, stream) as those of flat.cu and flat_range.cu do, and the metric picks the kernel.
 // Aux of one index: ||x||^2, ||x|| (f64 sums of the decoded row, rounded once to f32) and ||x_sub|| rounded up.
 int flat_fp16_prep_rows(const __half *codes, int64_t n, int d, float *norm2, float *norm, float *nsub, cudaStream_t st);
 // Per call: rows [n, n_out) of q_h, qn2, qn, qscale of the zero-padded batch; q_h = fp16(q 2^e_q), qscale = 2^-e_q.

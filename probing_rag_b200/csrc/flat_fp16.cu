@@ -155,9 +155,8 @@ int flat_fp16_filter_launch(int metric, unsigned grid, size_t smem, const CUtens
 {
     const bool ip = metric == PR_METRIC_INNER_PRODUCT;
     const void *filter = ip ? (const void *)flat_fp16_ip_filter_kernel : (const void *)flat_fp16_filter_kernel;
-    // per device, as in flat.cu: set on every call
-    PR_CUDA_CHECK(cudaFuncSetAttribute(filter, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                       1024 + kStageBudget + (2 * kMaxStages + 4) * 8 + 16));
+    // per device, as in flat.cu: set on every launch
+    PR_CUDA_CHECK(cudaFuncSetAttribute(filter, cudaFuncAttributeMaxDynamicSharedMemorySize, kFilterSmemMax));
     if (ip)
         flat_fp16_ip_filter_kernel<<<grid, kFilterThreads, smem, st>>>(map_x, map_q, fa, fh);
     else

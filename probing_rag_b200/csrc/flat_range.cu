@@ -22,7 +22,7 @@ __global__ void __launch_bounds__(kRangeThreads) flat_ip_range_refine_kernel(con
 
 }  // namespace
 
-int flat_range_refine_launch(const FlatRangeArgs &g, int metric, int n_queries, cudaStream_t stream)
+int flat_range_refine_launch(int metric, int n_queries, const FlatRangeArgs &g, cudaStream_t stream)
 {
     if (metric == PR_METRIC_INNER_PRODUCT)
         flat_ip_range_refine_kernel<<<n_queries, kRangeThreads, 0, stream>>>(g);

@@ -71,6 +71,29 @@ def _as_rows(x, d: int, what: str) -> torch.Tensor:
     return x
 
 
+def _queries(x, d: int, device=None) -> torch.Tensor:
+    """The query rows [B, d] float32 of x, a NumPy array or a tensor; a tensor must be on `device` (None: anywhere)."""
+    if isinstance(x, torch.Tensor) and device is not None and x.device != device:
+        raise ValueError(f"queries are on {x.device}, the index on {device}")
+    return _as_rows(x, d, "queries")
+
+
+def _like_queries(x, *res):
+    """Results as the queries x came: tensors for a tensor; NumPy arrays for a NumPy array, with a range search's
+    lims (the first of three) as uint64, faiss's size_t."""
+    if not isinstance(x, np.ndarray):
+        return res
+    res = tuple(r.cpu().numpy() for r in res)
+    return (res[0].astype(np.uint64),) + res[1:] if len(res) == 3 else res
+
+
+def _aligned(nbytes: int, device) -> tuple[torch.Tensor, int]:
+    """(buffer, pointer): nbytes of device memory from a 1024-byte-aligned pointer, as the C ABI takes workspaces and
+    aux buffers."""
+    buf = torch.empty(nbytes + 1024, dtype=torch.uint8, device=device)
+    return buf, (buf.data_ptr() + 1023) // 1024 * 1024
+
+
 class _IndexFlat:
     """A flat index of one metric (the subclass's ``metric_type``) on one GPU."""
 
@@ -116,13 +139,7 @@ class _IndexFlat:
         """(D, I) of the k nearest rows (L2) or the k largest inner products (IP) of every query row of x [B, d]
         float32."""
         k = _check_k(k)
-        as_numpy = isinstance(x, np.ndarray)
-        if not as_numpy:
-            if not isinstance(x, torch.Tensor):
-                raise ValueError(f"queries must be a NumPy array or a CUDA tensor, got {type(x).__name__}")
-            if x.device != self.device:
-                raise ValueError(f"queries are on {x.device}, the index on {self.device}")
-        q = self._as_rows(x, "queries").to(self.device).contiguous()
+        q = _queries(x, self.d, self.device).to(self.device).contiguous()
         B = q.shape[0]
         D = torch.empty((B, k), dtype=torch.float32, device=self.device)
         I = torch.empty((B, k), dtype=torch.int64, device=self.device)
@@ -130,15 +147,12 @@ class _IndexFlat:
             L = _lib.lib()
             h = self._handle()
             nbytes = int(L.pr_flat_workspace_bytes(h, B, k))
-            ws = torch.empty(nbytes + 1024, dtype=torch.uint8, device=self.device)
-            ws_ptr = (ws.data_ptr() + 1023) // 1024 * 1024
+            ws, ws_ptr = _aligned(nbytes, self.device)
             with torch.cuda.device(self.device):
                 _lib.check(L.pr_flat_search(h, B, q.data_ptr(), k, D.data_ptr(), I.data_ptr(), ws_ptr,
                                             nbytes, torch.cuda.current_stream(self.device).cuda_stream))
             self._last = (ws, ws_ptr, B, k)
-        if as_numpy:
-            return D.cpu().numpy(), I.cpu().numpy()
-        return D, I
+        return _like_queries(x, D, I)
 
     @torch.no_grad()
     def range_search(self, x, radius):
@@ -148,13 +162,7 @@ class _IndexFlat:
         size_t), a CUDA tensor in -> CUDA tensors out with lims int64.  Synchronises the device once (twice when some
         query has more results than the staging segments hold)."""
         radius = float(np.float32(radius))
-        as_numpy = isinstance(x, np.ndarray)
-        if not as_numpy:
-            if not isinstance(x, torch.Tensor):
-                raise ValueError(f"queries must be a NumPy array or a CUDA tensor, got {type(x).__name__}")
-            if x.device != self.device:
-                raise ValueError(f"queries are on {x.device}, the index on {self.device}")
-        q = self._as_rows(x, "queries").to(self.device).contiguous()
+        q = _queries(x, self.d, self.device).to(self.device).contiguous()
         B = q.shape[0]
         lims = torch.zeros(B + 1, dtype=torch.int64, device=self.device)
         D = torch.empty(0, dtype=torch.float32, device=self.device)
@@ -176,9 +184,7 @@ class _IndexFlat:
                 I = torch.empty(total, dtype=torch.int64, device=self.device)
                 self._range_call(q, radius, lims, count, D, I)
             self._range_cap = max(_RANGE_CAP0, most)
-        if as_numpy:
-            return lims.cpu().numpy().astype(np.uint64), D.cpu().numpy(), I.cpu().numpy()
-        return lims, D, I
+        return _like_queries(x, lims, D, I)
 
     # ------------------------------------------------------------------ project extras
     def set_tuning(self, first_chunk_rows: int = 0, growth: int = 0, cand_capacity: int = 0) -> None:
@@ -218,8 +224,7 @@ class _IndexFlat:
         h = self._handle()
         B = q.shape[0]
         nbytes = int(L.pr_flat_range_workspace_bytes(h, B))
-        ws = torch.empty(nbytes + 1024, dtype=torch.uint8, device=self.device)
-        ws_ptr = (ws.data_ptr() + 1023) // 1024 * 1024
+        ws, ws_ptr = _aligned(nbytes, self.device)
         with torch.cuda.device(self.device):
             _lib.check(L.pr_flat_range_search(h, B, q.data_ptr(), radius, lims_in.data_ptr(), count.data_ptr(),
                                               D.data_ptr(), I.data_ptr(), ws_ptr, nbytes,
@@ -244,8 +249,7 @@ class _IndexFlat:
             try:
                 _lib.check(L.pr_flat_set_tuning(h, ctypes.byref(self._tuning)))
                 nbytes = int(L.pr_flat_aux_bytes(h))
-                aux = torch.empty(nbytes + 1024, dtype=torch.uint8, device=self.device)
-                aux_ptr = (aux.data_ptr() + 1023) // 1024 * 1024
+                aux, aux_ptr = _aligned(nbytes, self.device)
                 with torch.cuda.device(self.device):
                     _lib.check(L.pr_flat_build_aux(h, aux_ptr, nbytes,
                                                    torch.cuda.current_stream(self.device).cuda_stream))
@@ -438,14 +442,8 @@ class _ShardedIndexFlat:
         every rank); NumPy in -> NumPy out, a CUDA tensor in -> CUDA tensors out."""
         from . import sharding
         k = _check_k(k)
-        as_numpy = isinstance(x, np.ndarray)
-        q = _as_rows(x, self.d, "queries")
-        if self._local is not None:
-            Dl, Il = self._local(q, k)
-        else:
-            if not as_numpy and q.device != self.device:
-                raise ValueError(f"queries are on {q.device}, the index on {self.device}")
-            Dl, Il = self.shard.search(q.to(self.device), k)
+        q = _queries(x, self.d, self.device if self._local is None else None)
+        Dl, Il = self.shard.search(q.to(self.device), k) if self._local is None else self._local(q, k)
         B = q.shape[0]
         if B:
             key = (B, k)
@@ -456,9 +454,7 @@ class _ShardedIndexFlat:
                 merge_lists(gd, gi, self.bases, self.metric_type)
         else:
             D, I = Dl, Il
-        if as_numpy:
-            return D.cpu().numpy(), I.cpu().numpy()
-        return D, I
+        return _like_queries(x, D, I)
 
     @torch.no_grad()
     def range_search(self, x, radius):
@@ -466,17 +462,12 @@ class _ShardedIndexFlat:
         ids global and ascending per query; NumPy in -> NumPy out (lims uint64), a CUDA tensor in -> CUDA tensors
         out (lims int64)."""
         from . import sharding
-        as_numpy = isinstance(x, np.ndarray)
-        q = _as_rows(x, self.d, "queries")
-        if self._local_range is not None:
-            lims_l, Dl, Il = self._local_range(q, radius)
-        else:
-            if not as_numpy and q.device != self.device:
-                raise ValueError(f"queries are on {q.device}, the index on {self.device}")
-            lims_l, Dl, Il = self.shard.range_search(q.to(self.device), radius)
+        q = _queries(x, self.d, self.device if self._local_range is None else None)
+        lims_l, Dl, Il = self.shard.range_search(q.to(self.device), radius) if self._local_range is None else \
+            self._local_range(q, radius)
         B, dev = q.shape[0], lims_l.device
         if B == 0:
-            return (np.zeros(1, np.uint64), Dl.cpu().numpy(), Il.cpu().numpy()) if as_numpy else (lims_l, Dl, Il)
+            return _like_queries(x, lims_l, Dl, Il)
         world = sharding._world(self.group)
         counts = (lims_l[1:] - lims_l[:-1]).contiguous()
         if world > 1:
@@ -506,9 +497,7 @@ class _ShardedIndexFlat:
         I[pos] = (gi + bases[:, None])[keep]
         lims = torch.zeros(B + 1, dtype=torch.int64, device=dev)
         torch.cumsum(every.sum(0), 0, out=lims[1:])
-        if as_numpy:
-            return lims.cpu().numpy().astype(np.uint64), D.cpu().numpy(), I.cpu().numpy()
-        return lims, D, I
+        return _like_queries(x, lims, D, I)
 
     # ------------------------------------------------------------------ project extras (this rank's shard)
     def set_tuning(self, first_chunk_rows: int = 0, growth: int = 0, cand_capacity: int = 0) -> None:
@@ -618,14 +607,31 @@ def read_rows(path: str, metric: int = METRIC_L2) -> np.ndarray:
     return np.memmap(path, dtype="<f4", mode="r", offset=off, shape=(ntotal, d))
 
 
+def _my_rows(n: int, group) -> tuple[int, int]:
+    """This rank's row range [lo, hi) of n rows: sharding.shard_range(n, rank, world)."""
+    from . import sharding
+    world = sharding._world(group)
+    return sharding.shard_range(n, dist.get_rank(group) if world > 1 else 0, world)
+
+
 def read_shard_rows(path: str, group=None, metric: int = METRIC_L2):
     """(row_base, rows): this rank's row range sharding.shard_range(ntotal, rank, world) of a flat index file of
     `metric`, as a read-only memory map (nothing is read yet)."""
-    from . import sharding
     rows_mm = read_rows(path, metric)
-    rank = dist.get_rank(group) if sharding._world(group) > 1 else 0
-    lo, hi = sharding.shard_range(rows_mm.shape[0], rank, sharding._world(group))
+    lo, hi = _my_rows(rows_mm.shape[0], group)
     return lo, rows_mm[lo:hi]
+
+
+def _to_device(mm: np.ndarray, device) -> torch.Tensor:
+    """A new tensor on `device` holding mm [n, d] (a memory map of float32 rows or fp16 codes), copied in pieces of
+    _COPY_BYTES so that the file is never held in host RAM."""
+    n, d = mm.shape
+    native = mm.dtype.newbyteorder("=")
+    out = torch.empty((n, d), dtype=torch.from_numpy(np.empty(0, native)).dtype, device=device)
+    step = max(1, _COPY_BYTES // (native.itemsize * d))
+    for a in range(0, n, step):
+        out[a:a + step].copy_(torch.from_numpy(np.array(mm[a:a + step], dtype=native)))
+    return out
 
 
 def read_index(path: str, device="cuda", sharded: bool = False, group=None):
@@ -635,44 +641,35 @@ def read_index(path: str, device="cuda", sharded: bool = False, group=None):
     sharded=True (one process per GPU, torch.distributed initialised, every rank of `group` calling): each rank copies
     only its row range (read_shard_rows) and gets a ShardedIndexFlatL2 / ShardedIndexFlatIP whose search covers the
     whole file."""
-    if _fourcc(path) == FOURCC_SQ:
-        return _read_sq_index(path, device, sharded, group)
-    metric = _metric_of(path)
-    if sharded:
-        row_base, rows_mm = read_shard_rows(path, group, metric)
+    sq = _fourcc(path) == FOURCC_SQ
+    if sq:
+        mm, metric = read_codes(path)
     else:
-        row_base, rows_mm = 0, read_rows(path, metric)
-    cls, sharded_cls = (IndexFlatL2, ShardedIndexFlatL2) if metric == METRIC_L2 else (IndexFlatIP, ShardedIndexFlatIP)
-    index = cls(rows_mm.shape[1], device)
-    n, d = rows_mm.shape
-    rows = torch.empty((n, d), dtype=torch.float32, device=index.device)
-    step = max(1, _COPY_BYTES // (4 * d))
-    for a in range(0, n, step):
-        rows[a:a + step].copy_(torch.from_numpy(np.array(rows_mm[a:a + step], dtype=np.float32)))
-    index._set_rows(rows)
-    return sharded_cls(index, row_base, group) if sharded else index
-
-
-def _read_sq_index(path: str, device, sharded: bool, group):
-    """read_index for an 'IxSQ' file: the codes are memory-mapped and copied to the device in pieces; sharded=True
-    copies this rank's row range only and returns a ShardedIndexFlatL2 / ShardedIndexFlatIP over it."""
-    from . import sharding
-    codes_mm, metric = read_codes(path)
-    row_base = 0
-    if sharded:
-        rank = dist.get_rank(group) if sharding._world(group) > 1 else 0
-        row_base, hi = sharding.shard_range(codes_mm.shape[0], rank, sharding._world(group))
-        codes_mm = codes_mm[row_base:hi]
-    n, d = codes_mm.shape
-    index = IndexScalarQuantizer(d, ScalarQuantizer.QT_fp16, metric, device)
-    codes = torch.empty((n, d), dtype=torch.float16, device=index.device)
-    step = max(1, _COPY_BYTES // (2 * d))
-    for a in range(0, n, step):
-        codes[a:a + step].copy_(torch.from_numpy(np.array(codes_mm[a:a + step], dtype=np.float16)))
-    index._set_rows(codes)
+        metric = _metric_of(path)
+        mm = read_rows(path, metric)
+    row_base, hi = _my_rows(mm.shape[0], group) if sharded else (0, mm.shape[0])
+    mm = mm[row_base:hi]
+    if sq:
+        index = IndexScalarQuantizer(mm.shape[1], ScalarQuantizer.QT_fp16, metric, device)
+    else:
+        index = (IndexFlatL2 if metric == METRIC_L2 else IndexFlatIP)(mm.shape[1], device)
+    index._set_rows(_to_device(mm, index.device))
     if not sharded:
         return index
     return (ShardedIndexFlatL2 if metric == METRIC_L2 else ShardedIndexFlatIP)(index, row_base, group)
+
+
+def _write_pieces(f, a, dtype: str, d: int) -> None:
+    """Append a [n, d] (a NumPy array, or a tensor copied to the host piece by piece) to f as `dtype`, '<f4' or '<f2',
+    in pieces of _COPY_BYTES; '<f2' takes float16 input only."""
+    step = max(1, _COPY_BYTES // (np.dtype(dtype).itemsize * d))
+    for i in range(0, int(a.shape[0]), step):
+        piece = a[i:i + step]
+        if isinstance(piece, torch.Tensor):
+            piece = piece.cpu().numpy()
+        if dtype == "<f2" and piece.dtype != np.float16:
+            raise ValueError(f"codes must be float16, got {piece.dtype}")
+        f.write(np.ascontiguousarray(piece, dtype=dtype).tobytes())
 
 
 def write_codes(path: str, codes, d: int, metric: int = METRIC_L2) -> None:
@@ -685,14 +682,7 @@ def write_codes(path: str, codes, d: int, metric: int = METRIC_L2) -> None:
         f.write(_SQ_HEADER.pack(FOURCC_SQ, d, n, 1 << 20, 1 << 20, 1, metric, ScalarQuantizer.QT_fp16, 0, 0.0, d,
                                 2 * d, 0))
         f.write(struct.pack("<Q", n * 2 * d))
-        step = max(1, _COPY_BYTES // (2 * d))
-        for a in range(0, n, step):
-            piece = codes[a:a + step]
-            if isinstance(piece, torch.Tensor):
-                piece = piece.cpu().numpy()
-            if piece.dtype != np.float16:
-                raise ValueError(f"codes must be float16, got {piece.dtype}")
-            f.write(np.ascontiguousarray(piece, dtype="<f2").tobytes())
+        _write_pieces(f, codes, "<f2", d)
 
 
 def write_rows(path: str, rows, d: int, metric: int = METRIC_L2) -> None:
@@ -703,12 +693,7 @@ def write_rows(path: str, rows, d: int, metric: int = METRIC_L2) -> None:
     n = int(rows.shape[0])
     with open(path, "wb") as f:
         f.write(_HEADER.pack(_FOURCC[metric], d, n, 1 << 20, 1 << 20, 1, metric, n * d))
-        step = max(1, _COPY_BYTES // (4 * d))
-        for a in range(0, n, step):
-            piece = rows[a:a + step]
-            if isinstance(piece, torch.Tensor):
-                piece = piece.cpu().numpy()
-            f.write(np.ascontiguousarray(piece, dtype="<f4").tobytes())
+        _write_pieces(f, rows, "<f4", d)
 
 
 def write_index(index, path: str) -> None:

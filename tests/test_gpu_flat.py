@@ -62,6 +62,9 @@ def test_duplicates_ties_zero_rows_and_padding():
     empty = IndexFlatL2(128)
     D, I = empty.search(Q, 4)
     assert torch.all(I == -1) and torch.all(D == torch.finfo(torch.float32).max)
+    assert empty.last_stats()["launches"] == 2                    # init and output
+    lims, D, I = empty.range_search(Q, 1.0)
+    assert torch.all(lims == 0) and D.numel() == 0 and empty.last_stats()["launches"] == 1    # init
 
 
 def test_near_tie_shells():

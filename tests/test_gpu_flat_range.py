@@ -156,6 +156,7 @@ def test_launch_plans_and_staging_sizes_give_identical_output(metric):
             ix = _index(rows, metric, **plan)
             assert _same(ix.range_search(Q, r), ref), plan
             st = ix.last_stats()
+            assert st["launches"] == 2 * st["chunks"] + 2, plan
             if plan.get("first_chunk_rows") == 1 << 30:
                 assert st["chunks"] == 1
             if plan.get("cand_capacity") == 1:

@@ -94,6 +94,7 @@ def test_launch_plans_and_overflow_fallback(plan, metric):
     ix = _sq(rows, metric, **plan)
     _check(ix, synth.dense_queries(rows, 257), 100, metric)
     st = ix.last_stats()
+    assert st["launches"] == 2 * st["chunks"] + 3
     if plan.get("first_chunk_rows") == 1 << 30:
         assert st["chunks"] == 1
     if "cand_capacity" in plan:
@@ -116,6 +117,8 @@ def test_range_search_plans_and_second_pass(metric):
     for plan in (dict(first_chunk_rows=1 << 30), dict(first_chunk_rows=128, growth=2, cand_capacity=4)):
         ix.set_tuning(**plan)
         _check_range(ix, Q, radius, metric)
+        st = ix.last_stats()
+        assert st["launches"] == 2 * st["chunks"] + 2, plan
 
 
 # ---------------------------------------------------------------------------------------------- hazards
